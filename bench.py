@@ -11,6 +11,7 @@ all ranks' bases divided by the max-over-ranks device time.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]         # the CUDA path (libblu_b200.so)
     python bench.py --impl reference ...                         # the CPU restatement of rwl/blu
+    python bench.py ... --dump-outputs DIR                       # also write the last timed step's outputs (dump_outputs)
 
 The reference is a Rust crate and this image has no Rust toolchain, so `--impl reference` and the
 `cpu_baseline` leg time oracle/ (the C restatement, kind "port"), one instance per host core.
@@ -31,6 +32,8 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 METRIC = "factorize+solve matrices/sec (batched)"
 UNIT = "matrices/s"
 M, NSLACK, PMEAN = 2000, 700, 5.0
+DUMP_BYTES = 48 * 10**6      # --dump-outputs: solutions beyond this are sampled, so that a dump stays under 64 MB
+DUMP_INFO = ["rank", "l_nz", "u_nz", "min_pivot", "max_pivot", "condest_l", "condest_u", "onenorm", "infnorm", "residual_test"]
 
 
 def host_cores():
@@ -124,6 +127,22 @@ def kernel_source_hash():
     return h.hexdigest()[:16]
 
 
+def dump_outputs(out_dir, x, status, info=None):
+    """What the last timed step returned, as float64 .npy files, so that two builds can be compared output for output
+    on the same seeded inputs.  x.npy holds the solutions [bases, m] of every basis, or of a fixed seeded sample of
+    them when all of them would exceed DUMP_BYTES; bases.npy gives their indices in the batch.  status.npy and
+    factor_info.npy (the per-basis getters DUMP_INFO, one column each) cover every basis."""
+    n, m = x.shape
+    keep = max(1, DUMP_BYTES // (8 * m))
+    idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    out = {"x": x[idx], "bases": idx, "status": status}
+    if info is not None:
+        out["factor_info"] = info
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -149,6 +168,8 @@ def run_reference(args, rank, world):
         assert (st == 0).all()
         if it >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x, st)
     T = sum(times)
     value = nsample * len(times) / T
     sample = f"{nsample} of the {args.nmat} bases per step (seeds 2000..), factorize+solve_dense each, {nt} threads, file_diff asserts on (setup_bump.rs:228-251)"
@@ -177,7 +198,10 @@ def main():
     ap.add_argument("--threads-per-basis", type=int, default=0)
     ap.add_argument("--ref-per-core", type=int, default=16, help="bases per host core in one reference step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     # stdout carries exactly ONE line, the JSON record: everything else that libraries print there
     # (NCCL prints its version banner on stdout) is sent to stderr
@@ -204,7 +228,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 
     from blu_b200 import BLUBatch, gen
-    from blu_b200.shard import shard_range
+    from blu_b200.shard import gather_rows, shard_range
 
     if args.scaling == "strong":
         lo, hi = shard_range(args.nmat, rank, world)      # rank's contiguous range of the ONE batch
@@ -276,6 +300,11 @@ def main():
     nbad = int((status != 0).sum())
     assert nbad == 0, f"{nbad} bases did not solve"
     nrealloc_after = int(b.info(0, "nrealloc"))
+    if args.dump_outputs:
+        info = np.array([[b.info(k, n) for n in DUMP_INFO] for k in range(nmat)])
+        x_all, status_all, info_all = (gather_rows(a, total) for a in (x, status, info))
+        if rank == 0:
+            dump_outputs(args.dump_outputs, x_all, status_all, info_all)
 
     # ---------------- end to end through the C ABI with host buffers ----------------
     import ctypes
