@@ -81,6 +81,8 @@ def load_library(path=None):
     L.blu_batch_solve_dense.argtypes = [vp, f64p, f64p, ctypes.c_char, i32p]
     L.blu_batch_solve_for_update.argtypes = [vp, i64p, i64p, f64p, ctypes.c_int, i64p, i64p, f64p, i32p, ctypes.c_char]
     L.blu_batch_update.argtypes = [vp, f64p, i32p]
+    L.blu_batch_maxvolume.argtypes = [vp, ctypes.c_int64, i64p, i64p, i64p, f64p, ctypes.c_int64, i64p, i64p,
+                                      ctypes.c_double, i64p, i32p]
     L.blu_batch_get_info.argtypes = [vp, ctypes.c_int64, ctypes.c_int]; L.blu_batch_get_info.restype = ctypes.c_double
     L.blu_batch_get_factors.argtypes = [vp, ctypes.c_int64, i64p, i64p, i64p, i64p, f64p, i64p, i64p, f64p]
     L.blu_batch_upload.argtypes = [vp, i64p, i64p, i64p, f64p, ctypes.c_int64, f64p]
@@ -342,6 +344,21 @@ class BLUBatch(_Base):
         stat = np.zeros(self.nmat, dtype=np.int32)
         st = self._L.blu_batch_update(self._h, _pf(x), stat.ctypes.data_as(i32p))
         return st, stat
+
+    def maxvolume(self, ncol, a_begin, a_end, a_i, a_x, basis, isbasic, volumetol):
+        """maxvolume (maxvolume.rs:64-224) on every basis at once.  Basis k's pool column j is
+        a_i/a_x[a_begin[k*ncol+j] : a_end[k*ncol+j]]; basis (nmat*m) and isbasic (nmat*ncol) are updated in place,
+        like maxvolume().  Returns (status, per-basis status, per-basis nupdate)."""
+        ab, ae, ai, ax = _i64(a_begin), _i64(a_end), _i64(a_i), _f64(a_x)
+        bas = _i64(basis).reshape(-1).copy()
+        isb = _i64(isbasic).reshape(-1).copy()
+        stat = np.zeros(self.nmat, dtype=np.int32)
+        nup = np.zeros(self.nmat, dtype=np.int64)
+        st = self._L.blu_batch_maxvolume(self._h, int(ncol), _pi(ab), _pi(ae), _pi(ai), _pf(ax), len(ai), _pi(bas), _pi(isb),
+                                         float(volumetol), _pi(nup), stat.ctypes.data_as(i32p))
+        basis[...] = bas.reshape(np.shape(basis))
+        isbasic[...] = isb.reshape(np.shape(isbasic))
+        return st, stat, nup
 
     def get_factors(self, k):
         m = self.m

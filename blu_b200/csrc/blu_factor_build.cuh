@@ -310,6 +310,7 @@ template <int NT> __global__ void __launch_bounds__(NT, FACT_MINB(NT)) k_factori
         const bool fresh = mode == BLU_MODE_WHOLE || mode == BLU_MODE_HEAD;
         if (!fresh && D.info[s].status != (mode == BLU_MODE_TAIL ? BLU_SUSPENDED_TAIL : BLU_SUSPENDED_BUILD)) continue;
         if (fresh && rerun && D.info[s].status != BLU_REALLOCATE) continue;      /* only the bases that asked for more memory run again */
+        if (fresh && D.run && !D.run[s]) continue;                               /* a subset of the batch (blu_batch_maxvolume) */
         if (tid == 0) {
             mat_view(S.M, D, s);
             shm_carve(S, dyn, cap, NT / 32, D.m);

@@ -11,6 +11,7 @@
 #include "blu_fact_launch.h"
 #include "blu_solve.cuh"
 #include "blu_sparse.cuh"
+#include "blu_maxvolume.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -1484,6 +1485,272 @@ extern "C" int blu_batch_update(blu_batch_t *o, const double *xtbl, int *status)
     }
     o->info_dirty = 1;
     return worst;
+}
+
+/* ------------------------------------------------------------------ */
+/* batch: maxvolume on every basis at once (maxvolume.rs:64-224)       */
+/* ------------------------------------------------------------------ */
+
+/* device buffers and pinned words of one blu_batch_maxvolume call; released on every way out, and the run mask
+ * is taken off the batch again so that later launches run every slot */
+struct MvCall {
+    blu_b200 *o;
+    std::vector<void *> mem;
+    unsigned long long *h_cnt = nullptr;
+    int *h_st = nullptr;
+    explicit MvCall(blu_b200 *b) : o(b) {}
+    template <typename T> int alloc(T **p, size_t n) {
+        int st = dalloc(o, p, n);
+        if (st == BLU_OK) mem.push_back(*p);
+        return st;
+    }
+    ~MvCall() {
+        cudaStreamSynchronize(o->stream);
+        o->d.run = nullptr;
+        for (void *p : mem) dfree(o, p);
+        if (h_cnt) cudaFreeHost(h_cnt);
+        if (h_st) cudaFreeHost(h_st);
+    }
+};
+
+/* room for B's of up to maxnz entries in the row-wise copy, which only lives during a factorization: a larger one
+ * replaces it, content dropped */
+static int mv_ensure_bt_cap(blu_b200 *o, int64_t maxnz) {
+    BluDev &d = o->d;
+    if (maxnz <= d.bnz_cap) return BLU_OK;
+    CK(cudaStreamSynchronize(o->stream));
+    dfree(o, d.bt_idx); dfree(o, d.bt_val); d.bt_idx = nullptr; d.bt_val = nullptr;
+    int st = dalloc(o, &d.bt_idx, (size_t)d.nmat * (size_t)maxnz);
+    if (st == BLU_OK) st = dalloc(o, &d.bt_val, (size_t)d.nmat * (size_t)maxnz);
+    if (st != BLU_OK) return st;
+    d.bnz_cap = maxnz;
+    return BLU_OK;
+}
+
+/* the bases with run = 1 are factorized (B as written by k_mv_decide), Reallocate handled as blu.rs:95-118
+ * (grow the bases that asked, run them again), then condest/residual_test; every basis whose factorization is
+ * not OK stops.  maxnz: the most entries of one of those B. */
+static int mv_factorize(blu_b200 *o, MvCall &c, const MvDev &V, int64_t maxnz) {
+    BluDev &d = o->d;
+    const int n = d.nmat, g = (n + 127) / 128;
+    { int st = mv_ensure_bt_cap(o, maxnz); if (st != BLU_OK) return st; }
+    for (int attempt = 0;; attempt++) {
+        if (attempt == 40) return BLU_ERROR_INTERNAL;
+        int st = launch_factorize(o, o->stream, 0, n, attempt > 0);
+        if (st != BLU_OK) return st;
+        CK(cudaMemsetAsync(V.cnt + MV_CNT_REALLOC, 0, sizeof(unsigned long long), o->stream));
+        BLU_LAUNCH(k_mv_factor_status, g, 128, 0, o->stream, V, d, 0);
+        o->launches++;
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(c.h_cnt, V.cnt, MV_CNT_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, o->stream));
+        CK(cudaStreamSynchronize(o->stream));
+        if (c.h_cnt[MV_CNT_REALLOC] == 0) break;
+        if ((st = fetch_info(o)) != BLU_OK) return st;
+        if ((st = grow_hungry_slots(o)) != BLU_OK) return st;
+    }
+    if (o->norms) {
+        BLU_LAUNCH(k_factor_norms, n, 128, 0, o->stream, d);
+        o->launches++;
+        CK(cudaGetLastError());
+    }
+    BLU_LAUNCH(k_mv_factor_status, g, 128, 0, o->stream, V, d, 1);
+    o->launches++;
+    CK(cudaGetLastError());
+    return BLU_OK;
+}
+
+/* statuses of the last masked launch (stride words apart) and the counters: does a basis ask for more memory?
+ * (a masked-out slot keeps the word of an earlier launch, which is never Reallocate once that launch is done) */
+static int mv_any_realloc(blu_b200 *o, MvCall &c, const MvDev &V, const int *d_st, int stride, bool *any) {
+    const size_t n = (size_t)o->d.nmat;
+    CK(cudaMemcpyAsync(c.h_st, d_st, n * stride * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
+    CK(cudaMemcpyAsync(c.h_cnt, V.cnt, MV_CNT_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, o->stream));
+    CK(cudaStreamSynchronize(o->stream));
+    *any = false;
+    for (size_t k = 0; k < n; k++) *any = *any || c.h_st[k * stride] == BLU_REALLOCATE;
+    return BLU_OK;
+}
+
+/* maxvolume (maxvolume.rs:64-224) on every basis of the batch, the bases in lockstep over their pool columns.
+ * The pool, basis and isbasic are uploaded once; per column the host queues set-up, the masked 'N' solve,
+ * leaving-row selection, the masked 'T' solve, the masked update and the refactorization decision, and reads
+ * back only status words and counts (three synchronisations, two more when some basis refactorizes). */
+extern "C" int blu_batch_maxvolume(blu_batch_t *o, int64_t ncol, const int64_t *a_begin, const int64_t *a_end,
+                                   const int64_t *a_i, const double *a_x, int64_t anz_total,
+                                   int64_t *basis, int64_t *isbasic, double volumetol, int64_t *nupdate, int *status) {
+    if (!o || o->single) return BLU_ERROR_INVALID_ARGUMENT;
+    if (ncol < 0 || anz_total < 0 || !basis || (ncol > 0 && (!a_begin || !a_end || !isbasic)) || (anz_total > 0 && (!a_i || !a_x)))
+        return BLU_ERROR_INVALID_ARGUMENT;
+    const int n = o->d.nmat, m = o->d.m;
+    const size_t N = (size_t)n, M = (size_t)m, C = (size_t)ncol;
+    auto reject = [&]() {
+        for (size_t k = 0; k < N; k++) { if (nupdate) nupdate[k] = 0; if (status) status[k] = BLU_ERROR_INVALID_ARGUMENT; }
+        return BLU_ERROR_INVALID_ARGUMENT;
+    };
+    if (volumetol < 1.0) return reject();      /* maxvolume.rs:83-90: nothing runs */
+    /* the reference indexes out of bounds (a panic) here: one answer for the whole call instead */
+    for (size_t q = 0; q < N * M; q++) if (basis[q] < 0 || basis[q] >= ncol) return reject();
+    for (size_t q = 0; q < N * C; q++)
+        if (a_begin[q] < 0 || a_begin[q] > anz_total || a_end[q] < 0 || a_end[q] > anz_total) return reject();
+    CK(cudaSetDevice(o->device));
+    BluDev &d = o->d;
+    MvCall c(o);
+    int st = ensure_b_cap(o, std::max<int64_t>(anz_total, 1));      /* the pool lives where B does; never a null pointer */
+    if (st == BLU_OK) st = ensure_batch_sparse(o, 0);
+    MvDev V;
+    memset(&V, 0, sizeof V);
+    V.nmat = n; V.m = m; V.ncol = ncol;
+    blu_i64 *abeg = nullptr, *aend = nullptr, *iota = nullptr; int *ust = nullptr;
+    if (st == BLU_OK) st = c.alloc(&abeg, N * C);
+    if (st == BLU_OK) st = c.alloc(&aend, N * C);
+    if (st == BLU_OK) st = c.alloc(&V.isbasic, N * C);
+    if (st == BLU_OK) st = c.alloc(&V.basis, N * M);
+    if (st == BLU_OK) st = c.alloc(&V.nupdate, N);
+    if (st == BLU_OK) st = c.alloc(&V.mvst, N);
+    if (st == BLU_OK) st = c.alloc(&V.run, N);
+    if (st == BLU_OK) st = c.alloc(&V.rhs_begin, N);
+    if (st == BLU_OK) st = c.alloc(&V.rhs_end, N);
+    if (st == BLU_OK) st = c.alloc(&V.leave, N);
+    if (st == BLU_OK) st = c.alloc(&iota, N + 1);
+    if (st == BLU_OK) st = c.alloc(&ust, N);
+    if (st == BLU_OK) st = c.alloc(&V.cnt, (size_t)MV_CNT_N);
+    if (st != BLU_OK) return st;
+    if (cudaMallocHost((void **)&c.h_cnt, MV_CNT_N * sizeof(unsigned long long)) != cudaSuccess ||
+        cudaMallocHost((void **)&c.h_st, 2 * N * sizeof(int)) != cudaSuccess) return BLU_ERROR_OUT_OF_MEMORY;
+    V.a_begin = abeg; V.a_end = aend;
+    V.b_begin = (blu_i64 *)o->db_begin; V.b_end = (blu_i64 *)o->db_end;
+    V.xtbl = o->sm_dbls;
+    std::vector<blu_i64> hiota(N + 1);
+    for (size_t k = 0; k <= N; k++) hiota[k] = (blu_i64)k;
+    std::vector<int> ones(N, 1);
+    const cudaStream_t s = o->stream;
+    if (ncol > 0) {
+        CK(cudaMemcpyAsync(abeg, a_begin, N * C * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(aend, a_end, N * C * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(V.isbasic, isbasic, N * C * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    }
+    CK(cudaMemcpyAsync(V.basis, basis, N * M * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    if (anz_total > 0) {
+        CK(cudaMemcpyAsync(o->db_i, a_i, (size_t)anz_total * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(o->db_x, a_x, (size_t)anz_total * sizeof(double), cudaMemcpyHostToDevice, s));
+    }
+    CK(cudaMemcpyAsync(iota, hiota.data(), (N + 1) * sizeof(blu_i64), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(V.run, ones.data(), N * sizeof(int), cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(o->sm_scal, 0, 2 * N * sizeof(int), s));      /* no status word of an earlier call says Reallocate */
+    /* B is the basis' columns of the pool from now on (the resident B of the batch after the call) */
+    d.b_begin = (const blu_i64 *)o->db_begin; d.b_end = (const blu_i64 *)o->db_end;
+    d.b_i = (const blu_i64 *)o->db_i; d.b_x = o->db_x; d.b_total = anz_total;
+    o->have_b = 1; o->b_external = 0;
+    d.run = V.run;
+    o->info_dirty = 1;
+    const int g = (n + 127) / 128;
+    auto read_cnt = [&]() -> int {
+        CK(cudaMemcpyAsync(c.h_cnt, V.cnt, MV_CNT_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        return BLU_OK;
+    };
+    /* decide + next (+ their counters); ust = null: the first factorization */
+    auto decide_next = [&](const int *u, int64_t j0) -> int {
+        CK(cudaMemsetAsync(V.cnt, 0, MV_CNT_N * sizeof(unsigned long long), s));
+        CK(cudaMemsetAsync(V.cnt + MV_CNT_NEXT, 0xff, sizeof(unsigned long long), s));
+        BLU_LAUNCH(k_mv_decide, n, 32, 0, s, V, d, u);
+        BLU_LAUNCH(k_mv_next, n, 32, 0, s, V, (blu_i64)j0);
+        o->launches += 2;
+        CK(cudaGetLastError());
+        return BLU_OK;
+    };
+    auto next_after_factorize = [&](int64_t j0) -> int {
+        CK(cudaMemsetAsync(V.cnt + MV_CNT_NEXT, 0xff, sizeof(unsigned long long), s));
+        BLU_LAUNCH(k_mv_next, n, 32, 0, s, V, (blu_i64)j0);
+        o->launches++;
+        CK(cudaGetLastError());
+        return read_cnt();
+    };
+
+    /* the next column: ~0 from k_mv_next means that no basis is running any more */
+    auto next_col = [&]() { return (int64_t)std::min<unsigned long long>(c.h_cnt[MV_CNT_NEXT], (unsigned long long)ncol); };
+    auto pass = [&]() -> int {
+        /* the first factorization, maxvolume.rs:92-95 */
+        if ((st = decide_next(nullptr, 0)) != BLU_OK || (st = read_cnt()) != BLU_OK) return st;
+        if ((st = mv_factorize(o, c, V, (int64_t)c.h_cnt[MV_CNT_MAXNZ])) != BLU_OK) return st;
+        if ((st = next_after_factorize(0)) != BLU_OK) return st;
+        for (int64_t j = next_col(); j < ncol; j = next_col()) {
+            bool again = false;
+            /* B^{-1} a_j straight from the pool, maxvolume.rs:100-118 */
+            BLU_LAUNCH(k_mv_setup, g, 128, 0, s, V, (blu_i64)j);
+            o->launches++;
+            for (int attempt = 0;; attempt++) {
+                SpMulti W{n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)V.rhs_begin, (const i64 *)V.rhs_end};
+                BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, d, 0, (const i64 *)o->db_i, (const double *)o->db_x, 'N', 1, 1,
+                           o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
+                o->launches++;
+                CK(cudaGetLastError());
+                if ((st = mv_any_realloc(o, c, V, o->sm_scal, 2, &again)) != BLU_OK) return st;
+                if (!again) break;
+                if (attempt == 39) return BLU_ERROR_OUT_OF_MEMORY;
+                if ((st = grow_batch_stores(o)) != BLU_OK) return st;      /* blu.rs:268-291 */
+            }
+            BLU_LAUNCH(k_mv_select, n, 32, 0, s, V, (blu_i64)j, (const int *)o->sm_scal, (const blu_i64 *)o->sm_ilhs, (const double *)o->sm_xout, volumetol);
+            o->launches++;
+            /* the leaving row, maxvolume.rs:143-150 */
+            for (int attempt = 0;; attempt++) {
+                SpMulti W{n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)iota, nullptr};
+                BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, d, 0, (const i64 *)V.leave, (const double *)nullptr, 'T', 1, 0,
+                           o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
+                BLU_LAUNCH(k_mv_absorb, g, 128, 0, s, V, (const int *)o->sm_scal, 2);
+                o->launches += 2;
+                CK(cudaGetLastError());
+                if ((st = mv_any_realloc(o, c, V, o->sm_scal, 2, &again)) != BLU_OK) return st;
+                if (!again) break;
+                if (attempt == 39) return BLU_ERROR_OUT_OF_MEMORY;
+                if ((st = grow_batch_stores(o)) != BLU_OK) return st;
+            }
+            /* update and the refactorization policy, maxvolume.rs:151-170 */
+            for (int attempt = 0;; attempt++) {
+                BLU_LAUNCH(k_update, n, 32, 0, s, d, 0.0, ust, (const double *)V.xtbl, attempt > 0 ? 1 : 0);
+                o->launches++;
+                if ((st = decide_next(ust, j + 1)) != BLU_OK) return st;
+                if ((st = mv_any_realloc(o, c, V, ust, 1, &again)) != BLU_OK) return st;
+                if (!again) break;
+                if (attempt == 39) return BLU_ERROR_OUT_OF_MEMORY;
+                if ((st = grow_batch_stores(o)) != BLU_OK) return st;      /* blu.rs:319-334 */
+            }
+            if (c.h_cnt[MV_CNT_REFACTOR] > 0) {
+                if ((st = mv_factorize(o, c, V, (int64_t)c.h_cnt[MV_CNT_MAXNZ])) != BLU_OK) return st;
+                if ((st = next_after_factorize(j + 1)) != BLU_OK) return st;
+            }
+        }
+        return BLU_OK;
+    };
+    const int failed = pass();
+    if (failed == BLU_ERROR_CUDA) return failed;
+
+    /* the resident B of the batch: every basis' final columns of the pool (k_mv_decide without an update status
+     * writes the view of every basis whose run flag is set) */
+    CK(cudaMemcpyAsync(V.run, ones.data(), N * sizeof(int), cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(V.cnt, 0, MV_CNT_N * sizeof(unsigned long long), s));
+    BLU_LAUNCH(k_mv_decide, n, 32, 0, s, V, d, (const int *)nullptr);
+    o->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(c.h_cnt, V.cnt, MV_CNT_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    /* what the device holds, also when a store could not grow partway through the pass */
+    std::vector<int> hst(N);
+    std::vector<int64_t> hnup(N);
+    CK(cudaMemcpyAsync(basis, V.basis, N * M * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    if (ncol > 0) CK(cudaMemcpyAsync(isbasic, V.isbasic, N * C * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(hnup.data(), V.nupdate, N * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(hst.data(), V.mvst, N * sizeof(int), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    /* a later factorization of the resident B needs a row-wise copy that holds it */
+    if ((st = mv_ensure_bt_cap(o, (int64_t)c.h_cnt[MV_CNT_MAXNZ])) != BLU_OK) return st;
+    int worst = BLU_OK;
+    for (size_t k = 0; k < N; k++) {
+        if (failed != BLU_OK && hst[k] == BLU_OK) hst[k] = failed;      /* the bases the failure stopped mid-pass */
+        if (nupdate) nupdate[k] = hnup[k];
+        if (status) status[k] = hst[k];
+        if (hst[k] != BLU_OK && worst == BLU_OK) worst = hst[k];
+    }
+    return failed != BLU_OK ? failed : worst;
 }
 
 /* ------------------------------------------------------------------ */

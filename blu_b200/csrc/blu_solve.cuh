@@ -745,6 +745,7 @@ __global__ void __launch_bounds__(128, NORMS_MINB) k_factor_norms(BluDev D) {
     __shared__ double sres[8];
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     for (int s = D.slot0 + blockIdx.x; s < D.slot0 + D.nslot; s += gridDim.x) {
+        if (D.run && !D.run[s]) continue;      /* not refactorized by this (masked) factorization */
         __syncthreads();
         if (tid == 0) mat_view(M, D, s);
         __syncthreads();

@@ -461,6 +461,7 @@ struct SpMulti {
     double *dbls;             /* nunits * 2m : work | xlhs  (all-zero between calls) */
     int *markers;             /* nunits */
     const i64 *rhs_begin;     /* nunits + 1 offsets into irhs64 / xrhs */
+    const i64 *rhs_end;       /* null, or nunits end offsets: unit u's right-hand side is [rhs_begin[u], rhs_end[u]) (columns of a resident pool) */
 };
 __device__ __forceinline__ void sp_ctx_init_unit(SpCtx &C, const BluDev &D, const SpMulti &W, int u) {
     mat_view(C.M, D, 0);
@@ -499,7 +500,8 @@ __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i
     if (units) {
         /* unit = blockIdx.x: its slice of the right-hand sides and of the outputs */
         const int u = blockIdx.x;
-        const i64 b = W.rhs_begin[u], e = W.rhs_begin[u + 1];
+        if (W.per_slot && D.run && !D.run[u]) return;      /* masked out: neither its state nor its status word is touched */
+        const i64 b = W.rhs_begin[u], e = W.rhs_end ? W.rhs_end[u] : W.rhs_begin[u + 1];
         irhs64 += b; if (xrhs) xrhs += b;
         nrhs = (e - b < 0 || e - b > 0x7fffffff) ? -1 : (int)(e - b);
         scal += 2 * u; ilhs_out += (size_t)u * D.m; xout += (size_t)u * D.m;
@@ -833,6 +835,7 @@ __global__ void __launch_bounds__(32) k_update(BluDev D, double xtbl, int *scal,
     const int lane = threadIdx.x & 31;
     /* object API: one block, slot 0.  Batch: block u updates basis u with its own xtbl and status word. */
     const int slot = xtbl_per_slot ? (int)blockIdx.x : 0;
+    if (xtbl_per_slot && D.run && !D.run[slot]) return;      /* masked out: state and status word untouched */
     if (xtbl_per_slot) { xtbl = xtbl_per_slot[slot]; scal += slot; }
     if (rerun && scal[0] != BLU_REALLOCATE) return;      /* batch re-run after a store was grown: only the bases that asked */
     if (lane == 0) sp_ctx_init(C, D, slot);

@@ -85,6 +85,7 @@ struct BluDev {
     blu_i64 l_mem, u_mem, w_mem, bnz_cap;
     blu_i64 b_total;            /* entries of b_i / b_x: every column pointer must lie in [0, b_total] */
     const BluSlotStore *slot_store; /* nmat overrides (null pointers inside = uniform store), or null */
+    const int *run;             /* nmat per-slot run flags of a batch launch (0: the slot is left untouched, status word included), or null: every slot runs */
     BluParams prm;
     /* input B */
     const blu_i64 *b_begin, *b_end, *b_i; /* b_begin/b_end: nmat*m; positions into b_i/b_x */

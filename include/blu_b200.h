@@ -161,6 +161,19 @@ int blu_batch_solve_for_update(blu_batch_t *b, const int64_t *rhs_begin, const i
                                int want_solution, int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans);
 int blu_batch_update(blu_batch_t *b, const double *xtbl, int *status);
 
+/* maxvolume (maxvolume.rs:64-224) on every basis of the batch, all bases in lockstep over the pool columns.
+ * Basis k has its own pool of ncol columns: column j is a_i/a_x[a_begin[k*ncol+j] .. a_end[k*ncol+j]) (anz_total
+ * entries in all, the same convention as blu_batch_factorize).  basis[k*m .. +m) and isbasic[k*ncol .. +ncol) are
+ * updated in place; nupdate[k] and status[k] (either may be NULL) receive what maxvolume returns for basis k: a
+ * basis stops at its first non-OK status, the others carry on.  The return value is the first non-OK status.
+ * volumetol < 1, a basis entry outside [0, ncol) or a pool offset outside [0, anz_total]:
+ * BLU_ERROR_INVALID_ARGUMENT, nothing runs.  Reallocate never escapes.  Afterwards every basis is in the state
+ * maxvolume leaves it in (getters, solves and updates continue from there), and the resident B of the batch is
+ * the basis' columns of the pool. */
+int blu_batch_maxvolume(blu_batch_t *b, int64_t ncol, const int64_t *a_begin, const int64_t *a_end,
+                        const int64_t *a_i, const double *a_x, int64_t anz_total,
+                        int64_t *basis, int64_t *isbasic, double volumetol, int64_t *nupdate, int *status);
+
 /* Device-resident variants for throughput measurement: upload once, then time kernels only. */
 int blu_batch_upload(blu_batch_t *b, const int64_t *b_begin, const int64_t *b_end,
                      const int64_t *b_i, const double *b_x, int64_t bnz_total, const double *rhs);
