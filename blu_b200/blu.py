@@ -81,6 +81,8 @@ def load_library(path=None):
     L.blu_batch_solve_dense.argtypes = [vp, f64p, f64p, ctypes.c_char, i32p]
     L.blu_batch_solve_for_update.argtypes = [vp, i64p, i64p, f64p, ctypes.c_int, i64p, i64p, f64p, i32p, ctypes.c_char]
     L.blu_batch_update.argtypes = [vp, f64p, i32p]
+    L.blu_batch_solve_sparse.argtypes = [vp, i64p, i64p, i64p, f64p, i64p, i64p, f64p, i32p, ctypes.c_char]
+    L.blu_batch_solve_dense_multi.argtypes = [vp, ctypes.c_int64, f64p, f64p, ctypes.c_char, i32p]
     L.blu_batch_maxvolume.argtypes = [vp, ctypes.c_int64, i64p, i64p, i64p, f64p, ctypes.c_int64, i64p, i64p,
                                       ctypes.c_double, i64p, i32p]
     L.blu_batch_get_info.argtypes = [vp, ctypes.c_int64, ctypes.c_int]; L.blu_batch_get_info.restype = ctypes.c_double
@@ -344,6 +346,46 @@ class BLUBatch(_Base):
         stat = np.zeros(self.nmat, dtype=np.int32)
         st = self._L.blu_batch_update(self._h, _pf(x), stat.ctypes.data_as(i32p))
         return st, stat
+
+    def solve_sparse(self, rhs_lists, trans="N"):
+        """rhs_lists[k] = [(irhs, xrhs), ...] for basis k -> (status, [[(ilhs, values), ...] per basis],
+        [unit status per basis]): solve_sparse for every right-hand side of every basis, one warp each, as
+        BLU.solve_sparse_multi does for one basis.  A rejected right-hand side gives empty arrays."""
+        if len(rhs_lists) != self.nmat:
+            raise IndexError("rhs_lists needs one list per basis")
+        counts = np.array([len(r) for r in rhs_lists], dtype=np.int64)
+        unit_begin = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+        units = [pair for r in rhs_lists for pair in r]
+        n = len(units)
+        rhs_begin = np.concatenate([[0], np.cumsum([len(ii) for ii, _ in units])]).astype(np.int64)
+        irhs = _i64(np.concatenate([np.asarray(ii, dtype=np.int64).reshape(-1) for ii, _ in units])) if n else np.zeros(0, np.int64)
+        xrhs = _f64(np.concatenate([np.asarray(xx, dtype=np.float64).reshape(-1) for _, xx in units])) if n else np.zeros(0)
+        nz = np.zeros(n, dtype=np.int64)
+        il = np.zeros(max(n, 1) * self.m, dtype=np.int64)
+        xl = np.zeros(max(n, 1) * self.m)
+        stat = np.zeros(max(n, 1), dtype=np.int32)
+        st = self._L.blu_batch_solve_sparse(self._h, _pi(unit_begin), _pi(rhs_begin), _pi(irhs), _pf(xrhs), _pi(nz), _pi(il),
+                                            _pf(xl), stat.ctypes.data_as(i32p), _ch(trans))
+        out, ustat = [], []
+        for k in range(self.nmat):
+            res = []
+            for u in range(unit_begin[k], unit_begin[k + 1]):
+                c = max(int(nz[u]), 0)
+                res.append((il[u * self.m:u * self.m + c].copy(), xl[u * self.m:u * self.m + c].copy()))
+            out.append(res)
+            ustat.append(stat[unit_begin[k]:unit_begin[k + 1]].copy())
+        return st, out, ustat
+
+    def solve_dense_multi(self, rhs, trans="N"):
+        """rhs[nmat, nrhs, m] -> (status, x[nmat, nrhs, m], status[nmat, nrhs]): solve_dense for every right-hand
+        side of every basis, one warp each."""
+        r = _f64(rhs)
+        nrhs = r.size // (self.nmat * self.m)
+        r = r.reshape(self.nmat, nrhs, self.m)
+        x = np.zeros_like(r)
+        stat = np.zeros((self.nmat, nrhs), dtype=np.int32)
+        st = self._L.blu_batch_solve_dense_multi(self._h, nrhs, _pf(r), _pf(x), _ch(trans), stat.ctypes.data_as(i32p))
+        return st, x, stat
 
     def maxvolume(self, ncol, a_begin, a_end, a_i, a_x, basis, isbasic, volumetol):
         """maxvolume (maxvolume.rs:64-224) on every basis at once.  Basis k's pool column j is

@@ -25,6 +25,20 @@
 
 #define PADDING 160 /* slack entries after the L/U/W stores: warp-wide terminator scans read up to 96 entries ahead */
 
+/* Scratch of the batch solves with many right-hand sides per basis (blu_batch_solve_sparse,
+ * blu_batch_solve_dense_multi).  One unit = one right-hand side of one basis; the units of a call go through
+ * the pool in chunks of at most blu_b200::solve_units, one launch per chunk.  Allocated on first use. */
+struct UnitPool {
+    int64_t cap = 0;            /* units the sparse scratch holds */
+    int *ints = nullptr, *markers = nullptr, *scal = nullptr; double *dbls = nullptr;   /* SpMulti layout; dbls all-zero between calls */
+    int64_t *ilhs = nullptr, *off = nullptr; double *xout = nullptr; blu_u64 *fill = nullptr;   /* the solutions of a chunk, packed */
+    int64_t dcap = 0;           /* units the dense scratch holds */
+    double *rhs = nullptr, *lhs = nullptr, *work = nullptr; int *dstatus = nullptr;
+    int64_t ucap = 0; int *slot = nullptr; int64_t *begin = nullptr;      /* per unit of a call: its basis, its right-hand side */
+    int64_t rcap = 0; int64_t *irhs = nullptr; double *xrhs = nullptr;
+    int64_t hcap = 0; int64_t *h_ilhs = nullptr; double *h_xout = nullptr;    /* pinned landing place of the packed solutions */
+};
+
 struct blu_b200 {
     int device;
     int single;                 /* created by blu_create (object API) */
@@ -57,6 +71,8 @@ struct blu_b200 {
     double *dm_rhs, *dm_lhs, *dm_work; int *dm_status; int64_t multi_cap;   /* blu_solve_dense_multi staging */
     int *sm_ints, *sm_markers, *sm_scal; double *sm_dbls, *sm_xout; int64_t *sm_ilhs, *sm_begin; int64_t smulti_cap;   /* blu_solve_sparse_multi */
     int64_t *sm_irhs; double *sm_xrhs; int64_t smulti_rhs_cap;
+    int solve_units;            /* largest chunk of units of a batch multi-RHS solve (BLU_B200_SOLVE_UNITS) */
+    UnitPool up;
     int info_dirty;             /* device info block is newer than hinfo */
     int norms;                  /* run condest/residual_test after every factorization (factorize.rs:121-147) */
     cudaStream_t copy_stream, chunk_stream[4]; cudaEvent_t ev_up[16], ev_ch[4]; int have_pipe;   /* pipelined upload (blu_batch_factorize) */
@@ -219,6 +235,8 @@ static int create_common(blu_b200 **out, int64_t nmat, int64_t m, int64_t bnz_ca
     o->dm_rhs = o->dm_lhs = o->dm_work = nullptr; o->dm_status = nullptr; o->multi_cap = 0;
     o->sm_ints = o->sm_markers = o->sm_scal = nullptr; o->sm_dbls = o->sm_xout = nullptr; o->sm_ilhs = o->sm_begin = nullptr; o->smulti_cap = 0;
     o->sm_irhs = nullptr; o->sm_xrhs = nullptr; o->smulti_rhs_cap = 0;
+    o->solve_units = 8192;      /* configs[1], 16,384 units (DESIGN.md §5): beyond this the kernels gain ~10 %, the call nothing */
+    if (const char *e = getenv("BLU_B200_SOLVE_UNITS")) { long v = atol(e); if (v >= 1 && v <= (1L << 24)) o->solve_units = (int)v; }   /* tuning / test knob */
     o->h_scal = nullptr; o->h_ilhs = nullptr; o->h_xout = nullptr;
     o->time_factorize = o->time_solve = o->time_update = 0.0;
     BluDev &d = o->d;
@@ -309,6 +327,8 @@ static void destroy_common(blu_b200 *o) {
     if (o->h_scal) cudaFreeHost(o->h_scal);
     if (o->h_ilhs) cudaFreeHost(o->h_ilhs);
     if (o->h_xout) cudaFreeHost(o->h_xout);
+    if (o->up.h_ilhs) cudaFreeHost(o->up.h_ilhs);
+    if (o->up.h_xout) cudaFreeHost(o->up.h_xout);
 #ifndef BLU_EMU
     cudaEventDestroy(o->ev0); cudaEventDestroy(o->ev1);
     for (int q = 0; q < 4; q++) cudaEventDestroy(o->ev_k[q]);
@@ -581,7 +601,7 @@ extern "C" int blu_batch_factorize_resident(blu_batch_t *o) {
 static int solve_dense_resident(blu_b200 *o, char trans) {
     CK(cudaSetDevice(o->device));
     timer_start(o);
-    BLU_LAUNCH(k_solve_dense, o->d.nmat, 32, 0, o->stream, o->d, (const double *)o->d_rhs, o->d_lhs, trans, o->d_status, (double *)nullptr, 0);
+    BLU_LAUNCH(k_solve_dense, o->d.nmat, 32, 0, o->stream, o->d, (const double *)o->d_rhs, o->d_lhs, trans, o->d_status, (double *)nullptr, 0, (const int *)nullptr);
     o->launches++;
     CK(cudaGetLastError());
     timer_stop(o, 1);
@@ -607,7 +627,7 @@ extern "C" int blu_batch_solve_dense_dev(blu_batch_t *o, const double *d_rhs, do
     if (!o || !d_rhs || !d_lhs) return BLU_ERROR_INVALID_ARGUMENT;
     CK(cudaSetDevice(o->device));
     timer_start(o);
-    BLU_LAUNCH(k_solve_dense, o->d.nmat, 32, 0, o->stream, o->d, d_rhs, d_lhs, trans, d_status ? d_status : o->d_status, (double *)nullptr, 0);
+    BLU_LAUNCH(k_solve_dense, o->d.nmat, 32, 0, o->stream, o->d, d_rhs, d_lhs, trans, d_status ? d_status : o->d_status, (double *)nullptr, 0, (const int *)nullptr);
     o->launches++;
     CK(cudaGetLastError());
     timer_stop(o, 1);
@@ -630,7 +650,7 @@ extern "C" int blu_batch_graph_capture(blu_batch_t *o, char trans) {
     CK(cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal));
     int st = launch_factorize(o, cap, 0, d.nmat);
     if (st == BLU_OK && o->norms) { BLU_LAUNCH(k_factor_norms, d.nmat, 128, 0, cap, d); o->launches++; }
-    if (st == BLU_OK) { BLU_LAUNCH(k_solve_dense, d.nmat, 32, 0, cap, d, (const double *)o->d_rhs, o->d_lhs, trans, o->d_status, (double *)nullptr, 0); o->launches++; }
+    if (st == BLU_OK) { BLU_LAUNCH(k_solve_dense, d.nmat, 32, 0, cap, d, (const double *)o->d_rhs, o->d_lhs, trans, o->d_status, (double *)nullptr, 0, (const int *)nullptr); o->launches++; }
     cudaError_t e = cudaStreamEndCapture(cap, &o->graph);
     cudaStreamDestroy(cap);
     if (st != BLU_OK) return st;
@@ -1265,7 +1285,7 @@ extern "C" int blu_solve_dense_multi(blu_t *o, int64_t nrhs, const double *rhs, 
     BLU_LAUNCH(k_garbage_perm, 1, 32, 0, o->stream, o->d);
     timer_start(o);
     BLU_LAUNCH(k_solve_dense, (int)std::min<size_t>(n, 1u << 20), 32, 0, o->stream, o->d, (const double *)o->dm_rhs, o->dm_lhs, trans,
-               o->dm_status, o->dm_work, (int)nrhs);
+               o->dm_status, o->dm_work, (int)nrhs, (const int *)nullptr);
     o->launches += 2;
     CK(cudaGetLastError());
     timer_stop(o, 1);
@@ -1484,6 +1504,209 @@ extern "C" int blu_batch_update(blu_batch_t *o, const double *xtbl, int *status)
         if (s != BLU_OK && worst == BLU_OK) worst = s;
     }
     o->info_dirty = 1;
+    return worst;
+}
+
+/* ------------------------------------------------------------------ */
+/* batch: many right-hand sides on every basis (one warp per unit)     */
+/* ------------------------------------------------------------------ */
+
+/* the per-unit tables of a call (basis of each unit, offsets of its right-hand side) */
+static int up_ensure_units(blu_b200 *o, int64_t nunits) {
+    UnitPool &U = o->up;
+    if (nunits <= U.ucap) return BLU_OK;
+    dfree(o, U.slot); dfree(o, U.begin); U.slot = nullptr; U.begin = nullptr; U.ucap = 0;
+    int st = dalloc(o, &U.slot, (size_t)nunits);
+    if (st == BLU_OK) st = dalloc(o, &U.begin, (size_t)nunits + 1);
+    if (st == BLU_OK) U.ucap = nunits;
+    return st;
+}
+/* SpMulti scratch for P units (dbls starts all-zero and k_solve_sparse leaves it so) and tot right-hand side entries */
+static int up_ensure_sparse(blu_b200 *o, int64_t P, int64_t tot) {
+    UnitPool &U = o->up;
+    const size_t m = (size_t)o->d.m, n = (size_t)P;
+    int st = BLU_OK;
+    if (P > U.cap) {
+        dfree(o, U.ints); dfree(o, U.dbls); dfree(o, U.markers); dfree(o, U.scal); dfree(o, U.ilhs); dfree(o, U.xout); dfree(o, U.off); dfree(o, U.fill);
+        U.ints = U.markers = U.scal = nullptr; U.dbls = U.xout = nullptr; U.ilhs = U.off = nullptr; U.fill = nullptr; U.cap = 0;
+        st = dalloc(o, &U.ints, n * 7 * m);
+        if (st == BLU_OK) st = dalloc(o, &U.dbls, n * 2 * m);
+        if (st == BLU_OK) st = dalloc(o, &U.markers, n);
+        if (st == BLU_OK) st = dalloc(o, &U.scal, 2 * n);
+        if (st == BLU_OK) st = dalloc(o, &U.ilhs, n * m);
+        if (st == BLU_OK) st = dalloc(o, &U.xout, n * m);
+        if (st == BLU_OK) st = dalloc(o, &U.off, n);
+        if (st == BLU_OK) st = dalloc(o, &U.fill, 1);
+        if (st != BLU_OK) return st;
+        U.cap = P;
+    }
+    if (tot > U.rcap) {
+        dfree(o, U.irhs); dfree(o, U.xrhs); U.irhs = nullptr; U.xrhs = nullptr; U.rcap = 0;
+        st = dalloc(o, &U.irhs, (size_t)tot);
+        if (st == BLU_OK) st = dalloc(o, &U.xrhs, (size_t)tot);
+        if (st != BLU_OK) return st;
+        U.rcap = tot;
+    }
+    return BLU_OK;
+}
+static int up_ensure_dense(blu_b200 *o, int64_t P) {
+    UnitPool &U = o->up;
+    if (P <= U.dcap) return BLU_OK;
+    const size_t m = (size_t)o->d.m, n = (size_t)P;
+    dfree(o, U.rhs); dfree(o, U.lhs); dfree(o, U.work); dfree(o, U.dstatus);
+    U.rhs = U.lhs = U.work = nullptr; U.dstatus = nullptr; U.dcap = 0;
+    int st = dalloc(o, &U.rhs, n * m);
+    if (st == BLU_OK) st = dalloc(o, &U.lhs, n * m);
+    if (st == BLU_OK) st = dalloc(o, &U.work, n * m);
+    if (st == BLU_OK) st = dalloc(o, &U.dstatus, n);
+    if (st == BLU_OK) U.dcap = P;
+    return st;
+}
+static int up_ensure_host(blu_b200 *o, int64_t n) {
+    UnitPool &U = o->up;
+    if (n <= U.hcap) return BLU_OK;
+    if (U.h_ilhs) cudaFreeHost(U.h_ilhs);
+    if (U.h_xout) cudaFreeHost(U.h_xout);
+    U.h_ilhs = nullptr; U.h_xout = nullptr; U.hcap = 0;
+    const int64_t want = std::max<int64_t>(n, 2 * U.hcap);
+    if (cudaMallocHost((void **)&U.h_ilhs, (size_t)want * sizeof(int64_t)) != cudaSuccess ||
+        cudaMallocHost((void **)&U.h_xout, (size_t)want * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return BLU_ERROR_OUT_OF_MEMORY; }
+    U.hcap = want;
+    return BLU_OK;
+}
+
+/* garbage_perm on every basis, so that the units of a basis can read its pivot sequence side by side */
+static int up_compact_all(blu_b200 *o, double *kms) {
+    timer_start(o);
+    BLU_LAUNCH(k_garbage_perm, o->d.nmat, 32, 0, o->stream, o->d);
+    o->launches++;
+    CK(cudaGetLastError());
+    timer_stop(o, 1);
+    *kms += o->last_ms[1];
+    return BLU_OK;
+}
+
+/* solve_sparse (solve_sparse.rs:35-73) for the units of every basis, one warp per unit.  Unit u reads the
+ * factors of its basis and nothing else of its state; marks, stacks and vectors come from the unit pool, and
+ * the flop counters of the basis are added to atomically.  Each chunk's solutions are packed on the device
+ * (only the nz entries of each unit cross the bus) and land in the caller's arrays at the unit's own offset. */
+extern "C" int blu_batch_solve_sparse(blu_batch_t *o, const int64_t *unit_begin, const int64_t *rhs_begin,
+                                      const int64_t *irhs, const double *xrhs,
+                                      int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans) {
+    if (!o || !unit_begin || unit_begin[0] != 0) return BLU_ERROR_INVALID_ARGUMENT;
+    const int64_t nmat = o->d.nmat;
+    const size_t m = (size_t)o->d.m;
+    for (int64_t k = 0; k < nmat; k++) if (unit_begin[k + 1] < unit_begin[k]) return BLU_ERROR_INVALID_ARGUMENT;
+    const int64_t nunits = unit_begin[nmat];
+    if (nunits == 0) return BLU_OK;
+    if (!rhs_begin || !nzlhs || !ilhs || !xlhs) return BLU_ERROR_INVALID_ARGUMENT;
+    const int64_t tot = rhs_begin[nunits];
+    if (tot < 0) return BLU_ERROR_INVALID_ARGUMENT;
+    for (int64_t u = 0; u < nunits; u++) if (rhs_begin[u] < 0 || rhs_begin[u] > tot) return BLU_ERROR_INVALID_ARGUMENT;
+    if (tot > 0 && (!irhs || !xrhs)) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    const double tic = wall_now();
+    const int64_t P = std::min<int64_t>(nunits, o->solve_units);
+    int st = up_ensure_units(o, nunits);
+    if (st == BLU_OK) st = up_ensure_sparse(o, P, tot);
+    if (st != BLU_OK) return st;
+    UnitPool &U = o->up;
+    std::vector<int> hslot((size_t)nunits);
+    for (int64_t k = 0; k < nmat; k++) for (int64_t u = unit_begin[k]; u < unit_begin[k + 1]; u++) hslot[(size_t)u] = (int)k;
+    CK(cudaMemcpyAsync(U.slot, hslot.data(), (size_t)nunits * sizeof(int), cudaMemcpyHostToDevice, o->stream));
+    CK(cudaMemcpyAsync(U.begin, rhs_begin, ((size_t)nunits + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, o->stream));
+    if (tot > 0) {
+        CK(cudaMemcpyAsync(U.irhs, irhs, (size_t)tot * sizeof(int64_t), cudaMemcpyHostToDevice, o->stream));
+        CK(cudaMemcpyAsync(U.xrhs, xrhs, (size_t)tot * sizeof(double), cudaMemcpyHostToDevice, o->stream));
+    }
+    double kms = 0.0;
+    if ((st = up_compact_all(o, &kms)) != BLU_OK) return st;
+    std::vector<int> hs(2 * (size_t)P);
+    std::vector<int64_t> hoff((size_t)P);
+    int worst = BLU_OK;
+    for (int64_t c0 = 0; c0 < nunits; c0 += P) {
+        const int cnt = (int)std::min<int64_t>(P, nunits - c0);
+        CK(cudaMemsetAsync(U.fill, 0, sizeof(blu_u64), o->stream));
+        SpMulti W{cnt, 0, 0, U.ints, U.dbls, U.markers, (const i64 *)U.begin + c0, nullptr, U.slot + c0, U.fill, (i64 *)U.off};
+        timer_start(o);
+        BLU_LAUNCH(k_solve_sparse<true>, cnt, 32, 0, o->stream, o->d, 0, (const i64 *)U.irhs, (const double *)U.xrhs, trans, 0, 1,
+                   U.scal, (i64 *)U.ilhs, U.xout, W);
+        o->launches++;
+        CK(cudaGetLastError());
+        timer_stop(o, 1);
+        kms += o->last_ms[1];
+        blu_u64 fill = 0;
+        CK(cudaMemcpyAsync(hs.data(), U.scal, 2 * (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
+        CK(cudaMemcpyAsync(hoff.data(), U.off, (size_t)cnt * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
+        CK(cudaMemcpyAsync(&fill, U.fill, sizeof(blu_u64), cudaMemcpyDeviceToHost, o->stream));
+        CK(cudaStreamSynchronize(o->stream));
+        if (fill > 0) {
+            if ((st = up_ensure_host(o, (int64_t)fill)) != BLU_OK) return st;
+            CK(cudaMemcpyAsync(U.h_ilhs, U.ilhs, (size_t)fill * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
+            CK(cudaMemcpyAsync(U.h_xout, U.xout, (size_t)fill * sizeof(double), cudaMemcpyDeviceToHost, o->stream));
+            CK(cudaStreamSynchronize(o->stream));
+        }
+        for (int b = 0; b < cnt; b++) {
+            const size_t u = (size_t)(c0 + b);
+            const int s = hs[2 * b], nz = hs[2 * b + 1];
+            if (status) status[u] = s;
+            nzlhs[u] = s == BLU_OK ? nz : -1;
+            if (s == BLU_OK && nz > 0) {
+                memcpy(ilhs + u * m, U.h_ilhs + hoff[b], (size_t)nz * sizeof(int64_t));
+                memcpy(xlhs + u * m, U.h_xout + hoff[b], (size_t)nz * sizeof(double));
+            }
+            if (s != BLU_OK && worst == BLU_OK) worst = s;
+        }
+    }
+    o->last_ms[1] = kms;
+    o->info_dirty = 1;
+    o->time_solve += wall_now() - tic;
+    return worst;
+}
+
+/* solve_dense (solve_dense.rs:24) for nrhs right-hand sides on every basis, one warp per unit (basis k,
+ * right-hand side r) = unit k*nrhs + r.  The right-hand sides and solutions of a chunk are staged through
+ * the pool; the factors are only read. */
+extern "C" int blu_batch_solve_dense_multi(blu_batch_t *o, int64_t nrhs, const double *rhs, double *lhs, char trans, int *status) {
+    if (!o || nrhs < 0 || (nrhs > 0 && (!rhs || !lhs))) return BLU_ERROR_INVALID_ARGUMENT;
+    if (nrhs == 0) return BLU_OK;
+    CK(cudaSetDevice(o->device));
+    const double tic = wall_now();
+    const size_t m = (size_t)o->d.m;
+    const int64_t nunits = (int64_t)o->d.nmat * nrhs;
+    const int64_t P = std::min<int64_t>(nunits, o->solve_units);
+    int st = up_ensure_units(o, nunits);
+    if (st == BLU_OK) st = up_ensure_dense(o, P);
+    if (st != BLU_OK) return st;
+    UnitPool &U = o->up;
+    std::vector<int> hslot((size_t)nunits);
+    for (int64_t u = 0; u < nunits; u++) hslot[(size_t)u] = (int)(u / nrhs);
+    CK(cudaMemcpyAsync(U.slot, hslot.data(), (size_t)nunits * sizeof(int), cudaMemcpyHostToDevice, o->stream));
+    double kms = 0.0;
+    if ((st = up_compact_all(o, &kms)) != BLU_OK) return st;
+    std::vector<int> hs((size_t)P);
+    int worst = BLU_OK;
+    for (int64_t c0 = 0; c0 < nunits; c0 += P) {
+        const int cnt = (int)std::min<int64_t>(P, nunits - c0);
+        CK(cudaMemcpyAsync(U.rhs, rhs + (size_t)c0 * m, (size_t)cnt * m * sizeof(double), cudaMemcpyHostToDevice, o->stream));
+        timer_start(o);
+        BLU_LAUNCH(k_solve_dense, cnt, 32, 0, o->stream, o->d, (const double *)U.rhs, U.lhs, trans, U.dstatus, U.work, cnt,
+                   (const int *)U.slot + c0);
+        o->launches++;
+        CK(cudaGetLastError());
+        timer_stop(o, 1);
+        kms += o->last_ms[1];
+        CK(cudaMemcpyAsync(lhs + (size_t)c0 * m, U.lhs, (size_t)cnt * m * sizeof(double), cudaMemcpyDeviceToHost, o->stream));
+        CK(cudaMemcpyAsync(hs.data(), U.dstatus, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
+        CK(cudaStreamSynchronize(o->stream));
+        for (int b = 0; b < cnt; b++) {
+            if (status) status[c0 + b] = hs[b];
+            if (hs[b] != BLU_OK && worst == BLU_OK) worst = hs[b];
+        }
+    }
+    o->last_ms[1] = kms;
+    o->info_dirty = 1;
+    o->time_solve += wall_now() - tic;
     return worst;
 }
 

@@ -462,9 +462,13 @@ struct SpMulti {
     int *markers;             /* nunits */
     const i64 *rhs_begin;     /* nunits + 1 offsets into irhs64 / xrhs */
     const i64 *rhs_end;       /* null, or nunits end offsets: unit u's right-hand side is [rhs_begin[u], rhs_end[u]) (columns of a resident pool) */
+    /* k_solve_sparse<true> only (blu_batch_solve_sparse): */
+    const int *unit_slot;     /* unit u reads the factors of slot unit_slot[u] */
+    blu_u64 *pack_fill;       /* unit u reserves nz entries of ilhs_out / xout at *pack_fill (the chunk's solutions back to back, */
+    i64 *pack_off;            /* for one short copy) and records where they start in pack_off[u] */
 };
-__device__ __forceinline__ void sp_ctx_init_unit(SpCtx &C, const BluDev &D, const SpMulti &W, int u) {
-    mat_view(C.M, D, 0);
+__device__ __forceinline__ void sp_ctx_init_unit(SpCtx &C, const BluDev &D, const SpMulti &W, int u, int slot) {
+    mat_view(C.M, D, slot);
     const size_t m = (size_t)C.M.m;
     C.m = C.M.m; C.status = BLU_OK;
     int *ib = W.ints + (size_t)u * 7 * m;
@@ -489,24 +493,32 @@ __device__ __forceinline__ void sp_solve_done(SpCtx &C) {
 
 /* solve_sparse (solve_sparse.rs:35-73 + lu/solve_sparse.rs:11-360) and solve_for_update
  * (solve_for_update.rs:72-119 + lu/solve_for_update.rs:12-455).
- * scal[0] = status, scal[1] = nzlhs.  The solution leaves compacted: ilhs_out[n], xout[n]. */
+ * scal[0] = status, scal[1] = nzlhs.  The solution leaves compacted: ilhs_out[n], xout[n].
+ * Unit shapes (W.nunits > 0): per_slot -- unit u is basis u of a batch, on that basis' own scratch; otherwise
+ * units on scratch of their own that only read the factors: of slot 0 (blu_solve_sparse_multi), or with
+ * SLOT_UNITS of slot W.unit_slot[u], the solutions packed (blu_batch_solve_sparse).  SLOT_UNITS is a template
+ * argument so that the other shapes compile as they did without it. */
+template <bool SLOT_UNITS = false>
 __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i64 *irhs64, const double *xrhs, char trans,
                                                       int for_update, int want_solution, int *scal, i64 *ilhs_out, double *xout,
                                                       SpMulti W) {
     __shared__ SpCtx C;
     const int lane = threadIdx.x & 31;
-    const bool units = W.nunits > 0;
-    const bool multi = units && !W.per_slot;     /* several units share ONE basis: its state is read-only */
+    const bool units = SLOT_UNITS || W.nunits > 0;
+    const bool per_slot = !SLOT_UNITS && W.per_slot;
+    const bool multi = units && !per_slot;       /* several units share ONE basis: its state is read-only */
+    if (SLOT_UNITS) for_update = 0;              /* plain solves only: the solve_for_update paths drop out of this instance */
     if (units) {
         /* unit = blockIdx.x: its slice of the right-hand sides and of the outputs */
         const int u = blockIdx.x;
-        if (W.per_slot && D.run && !D.run[u]) return;      /* masked out: neither its state nor its status word is touched */
+        if (per_slot && D.run && !D.run[u]) return;      /* masked out: neither its state nor its status word is touched */
         const i64 b = W.rhs_begin[u], e = W.rhs_end ? W.rhs_end[u] : W.rhs_begin[u + 1];
         irhs64 += b; if (xrhs) xrhs += b;
         nrhs = (e - b < 0 || e - b > 0x7fffffff) ? -1 : (int)(e - b);
-        scal += 2 * u; ilhs_out += (size_t)u * D.m; xout += (size_t)u * D.m;
+        scal += 2 * u;
+        if (!SLOT_UNITS) { ilhs_out += (size_t)u * D.m; xout += (size_t)u * D.m; }
         if (W.rerun && scal[0] != BLU_REALLOCATE) return;
-        if (lane == 0) { if (W.per_slot) sp_ctx_init(C, D, u); else sp_ctx_init_unit(C, D, W, u); }
+        if (lane == 0) { if (per_slot) sp_ctx_init(C, D, u); else sp_ctx_init_unit(C, D, W, u, SLOT_UNITS ? W.unit_slot[u] : 0); }
     } else if (lane == 0) sp_ctx_init(C, D);
     __syncwarp();
     Mat &M = C.M;
@@ -638,6 +650,12 @@ __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i
         if (want_solution) nz = sp_ftran_tail(C, nz); else nz = 0;
     }
     if (for_update && !want_solution) nz = 0;
+    if (SLOT_UNITS) {
+        i64 base = 0;
+        if (lane == 0) { base = (i64)atomicAdd((unsigned long long *)W.pack_fill, (unsigned long long)nz); W.pack_off[blockIdx.x] = base; }
+        base = __shfl_sync(FULLMASK, base, 0);
+        ilhs_out += base; xout += base;
+    }
     /* hand the solution out compacted and leave xlhs all-zero again */
     for (int n = lane; n < nz; n += 32) {
         const int j = C.ilhs[n];

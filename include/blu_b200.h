@@ -161,6 +161,26 @@ int blu_batch_solve_for_update(blu_batch_t *b, const int64_t *rhs_begin, const i
                                int want_solution, int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans);
 int blu_batch_update(blu_batch_t *b, const double *xtbl, int *status);
 
+/* solve_sparse (solve_sparse.rs:35-73) for many right-hand sides on every basis of the batch, one warp per
+ * (basis, right-hand side).  Basis k owns units unit_begin[k] .. unit_begin[k+1) (unit_begin has nmat+1 entries,
+ * unit_begin[0] == 0, non-decreasing; a basis may own none).  Unit u solves with
+ * irhs/xrhs[rhs_begin[u] .. rhs_begin[u+1]) and returns, exactly as blu_solve_sparse_multi does:
+ * nzlhs[u] (-1 on error), the pattern ilhs[u*m ..] in blu_solve_sparse's order, the values compacted in
+ * xlhs[u*m + n], status[u] (may be NULL).  Bit-identical to calling solve_sparse for the units of basis k in
+ * order.  The return value is the first non-OK unit status.  A malformed unit_begin or rhs_begin, or a missing
+ * array: BLU_ERROR_INVALID_ARGUMENT, nothing runs.  A unit's own argument errors (an index >= m, more than m
+ * entries, a basis never factorized) go to its status word; the other units carry on.  A pending
+ * solve_for_update / update sequence is not disturbed.  At most BLU_B200_SOLVE_UNITS units (read from the
+ * environment at batch creation, default 8192) are in flight per launch; their scratch takes 60*m bytes each. */
+int blu_batch_solve_sparse(blu_batch_t *b, const int64_t *unit_begin, const int64_t *rhs_begin,
+                           const int64_t *irhs, const double *xrhs,
+                           int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans);
+
+/* solve_dense (solve_dense.rs:24) for nrhs right-hand sides on every basis: the right-hand side r of basis k is
+ * rhs[(k*nrhs + r)*m ..], its solution lhs[(k*nrhs + r)*m ..], status[k*nrhs + r] (may be NULL).  Bit-identical to
+ * nrhs blu_solve_dense calls on each basis.  Returns the first non-OK status; nrhs < 0: BLU_ERROR_INVALID_ARGUMENT. */
+int blu_batch_solve_dense_multi(blu_batch_t *b, int64_t nrhs, const double *rhs, double *lhs, char trans, int *status);
+
 /* maxvolume (maxvolume.rs:64-224) on every basis of the batch, all bases in lockstep over the pool columns.
  * Basis k has its own pool of ncol columns: column j is a_i/a_x[a_begin[k*ncol+j] .. a_end[k*ncol+j]) (anz_total
  * entries in all, the same convention as blu_batch_factorize).  basis[k*m .. +m) and isbasic[k*ncol .. +ncol) are
