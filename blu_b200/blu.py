@@ -85,6 +85,10 @@ def load_library(path=None):
     L.blu_batch_solve_dense_multi.argtypes = [vp, ctypes.c_int64, f64p, f64p, ctypes.c_char, i32p]
     L.blu_batch_maxvolume.argtypes = [vp, ctypes.c_int64, i64p, i64p, i64p, f64p, ctypes.c_int64, i64p, i64p,
                                       ctypes.c_double, i64p, i32p]
+    L.blu_batch_factorize_subset.argtypes = [vp, ctypes.c_int64, i64p, i64p, i64p, i64p, f64p, ctypes.c_int64, i32p]
+    L.blu_batch_solve_for_update_subset.argtypes = [vp, ctypes.c_int64, i64p, i64p, i64p, f64p, ctypes.c_int, i64p, i64p, f64p,
+                                                    i32p, ctypes.c_char]
+    L.blu_batch_update_subset.argtypes = [vp, ctypes.c_int64, i64p, f64p, i32p]
     L.blu_batch_get_info.argtypes = [vp, ctypes.c_int64, ctypes.c_int]; L.blu_batch_get_info.restype = ctypes.c_double
     L.blu_batch_get_factors.argtypes = [vp, ctypes.c_int64, i64p, i64p, i64p, i64p, f64p, i64p, i64p, f64p]
     L.blu_batch_upload.argtypes = [vp, i64p, i64p, i64p, f64p, ctypes.c_int64, f64p]
@@ -345,6 +349,45 @@ class BLUBatch(_Base):
         x = _f64(xtbl)
         stat = np.zeros(self.nmat, dtype=np.int32)
         st = self._L.blu_batch_update(self._h, _pf(x), stat.ctypes.data_as(i32p))
+        return st, stat
+
+    def factorize_subset(self, sel, b_begin, b_end, b_i, b_x):
+        """Refactorize the bases sel only; column j of the r-th is b_i/b_x[b_begin[r*m+j] : b_end[r*m+j]].  The other
+        bases keep their factors and update history.  Returns (status, status per selected basis)."""
+        s, bb, be, bi, bx = _i64(sel), _i64(b_begin), _i64(b_end), _i64(b_i), _f64(b_x)
+        stat = np.zeros(len(s), dtype=np.int32)
+        st = self._L.blu_batch_factorize_subset(self._h, len(s), _pi(s), _pi(bb), _pi(be), _pi(bi), _pf(bx), len(bi),
+                                                stat.ctypes.data_as(i32p))
+        return st, stat
+
+    def solve_for_update_subset(self, sel, rhs_list, trans="N", want_solution=0):
+        """solve_for_update on the bases sel only, rhs_list[r] = (irhs, xrhs or None) for basis sel[r] ->
+        (status, status per selected basis, [(ilhs, values)] per selected basis or None)"""
+        s = _i64(sel)
+        n = len(s)
+        begin = np.zeros(n + 1, dtype=np.int64)
+        for r, (ii, _) in enumerate(rhs_list):
+            begin[r + 1] = begin[r] + len(np.asarray(ii).reshape(-1))
+        irhs = _i64(np.concatenate([np.asarray(ii, dtype=np.int64).reshape(-1) for ii, _ in rhs_list])) if n else np.zeros(0, np.int64)
+        have_x = n > 0 and rhs_list[0][1] is not None
+        xrhs = _f64(np.concatenate([np.asarray(xx, dtype=np.float64) for _, xx in rhs_list])) if have_x else None
+        stat = np.zeros(n, dtype=np.int32)
+        if want_solution:
+            nz = np.zeros(n, dtype=np.int64); il = np.zeros(max(n, 1) * self.m, dtype=np.int64); xl = np.zeros(max(n, 1) * self.m)
+            st = self._L.blu_batch_solve_for_update_subset(self._h, n, _pi(s), _pi(begin), _pi(irhs), _pf(xrhs), 1, _pi(nz), _pi(il),
+                                                           _pf(xl), stat.ctypes.data_as(i32p), _ch(trans))
+            out = [(il[r * self.m:r * self.m + max(int(nz[r]), 0)].copy(), xl[r * self.m:r * self.m + max(int(nz[r]), 0)].copy())
+                   for r in range(n)]
+            return st, stat, out
+        st = self._L.blu_batch_solve_for_update_subset(self._h, n, _pi(s), _pi(begin), _pi(irhs), _pf(xrhs), 0, None, None, None,
+                                                       stat.ctypes.data_as(i32p), _ch(trans))
+        return st, stat, None
+
+    def update_subset(self, sel, xtbl):
+        """update on the bases sel only, basis sel[r] with xtbl[r] -> (status, status per selected basis)"""
+        s, x = _i64(sel), _f64(xtbl)
+        stat = np.zeros(len(s), dtype=np.int32)
+        st = self._L.blu_batch_update_subset(self._h, len(s), _pi(s), _pf(x), stat.ctypes.data_as(i32p))
         return st, stat
 
     def solve_sparse(self, rhs_lists, trans="N"):

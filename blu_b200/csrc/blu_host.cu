@@ -12,6 +12,7 @@
 #include "blu_solve.cuh"
 #include "blu_sparse.cuh"
 #include "blu_maxvolume.cuh"
+#include "blu_subset.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -85,6 +86,7 @@ struct blu_b200 {
     int have_b;                 /* B resident on device (for re-runs) */
     int b_external;             /* B lives in the caller's device buffers (blu_batch_factorize_dev) */
     cudaGraph_t graph; cudaGraphExec_t graph_exec; int have_graph; char graph_trans;   /* blu_batch_graph_* */
+    std::vector<char> hrun;     /* host copy of d.run during a subset call (empty: every slot runs) */
     double time_factorize, time_solve, time_update;
 };
 
@@ -445,7 +447,7 @@ static int grow_hungry_slots(blu_b200 *o) {
     auto rnd = [](size_t b) { return (b + 255) & ~(size_t)255; };
     for (int k = 0; k < d.nmat; k++) {
         const BluInfo &I = o->hinfo[(size_t)k];
-        if (I.status != BLU_REALLOCATE) continue;
+        if (I.status != BLU_REALLOCATE || (!o->hrun.empty() && !o->hrun[(size_t)k])) continue;
         const BluSlotStore &e = o->hslot[(size_t)k];
         Need n = {k, 0, 0, 0};
         if (I.addmem_l > 0) n.l = (int64_t)(f * (double)((e.l_idx ? e.l_mem : d.l_mem) + I.addmem_l)) + 1;
@@ -522,8 +524,10 @@ static int factorize_resident(blu_b200 *o, int hungry_known = 0, int escape_real
 #endif
         if ((st = fetch_info(o)) != BLU_OK) return st;
         int64_t al = 0, au = 0, aw = 0; int need = 0;
-        for (auto &I : o->hinfo) {
-            if (I.status == BLU_REALLOCATE) { need = 1; al = std::max<int64_t>(al, I.addmem_l); au = std::max<int64_t>(au, I.addmem_u); aw = std::max<int64_t>(aw, I.addmem_w); }
+        for (size_t k = 0; k < o->hinfo.size(); k++) {
+            const BluInfo &I = o->hinfo[k];
+            /* (a masked-out slot may still say Reallocate from a call that ran out of memory: it does not run here) */
+            if (I.status == BLU_REALLOCATE && (o->hrun.empty() || o->hrun[k])) { need = 1; al = std::max<int64_t>(al, I.addmem_l); au = std::max<int64_t>(au, I.addmem_u); aw = std::max<int64_t>(aw, I.addmem_w); }
         }
         if (!need) {
             if (o->single && d.ur_idx) {   /* sorted row-wise U for the wavefront U sweeps (object API) */
@@ -1714,8 +1718,8 @@ extern "C" int blu_batch_solve_dense_multi(blu_batch_t *o, int64_t nrhs, const d
 /* batch: maxvolume on every basis at once (maxvolume.rs:64-224)       */
 /* ------------------------------------------------------------------ */
 
-/* device buffers and pinned words of one blu_batch_maxvolume call; released on every way out, and the run mask
- * is taken off the batch again so that later launches run every slot */
+/* device buffers and pinned words of one masked batch call (blu_batch_maxvolume, the subset calls); released on
+ * every way out, and the run mask is taken off the batch again so that later launches run every slot */
 struct MvCall {
     blu_b200 *o;
     std::vector<void *> mem;
@@ -1730,6 +1734,7 @@ struct MvCall {
     ~MvCall() {
         cudaStreamSynchronize(o->stream);
         o->d.run = nullptr;
+        o->hrun.clear();
         for (void *p : mem) dfree(o, p);
         if (h_cnt) cudaFreeHost(h_cnt);
         if (h_st) cudaFreeHost(h_st);
@@ -1974,6 +1979,254 @@ extern "C" int blu_batch_maxvolume(blu_batch_t *o, int64_t ncol, const int64_t *
         if (hst[k] != BLU_OK && worst == BLU_OK) worst = hst[k];
     }
     return failed != BLU_OK ? failed : worst;
+}
+
+/* ------------------------------------------------------------------ */
+/* batch: refactorize / change the basis of chosen bases only          */
+/* ------------------------------------------------------------------ */
+
+/* The selection of a subset call: nsel distinct slots in [0, nmat).  pos[k] = r for the r-th selected slot, -1 for
+ * the others. */
+static int subset_select(blu_b200 *o, int64_t nsel, const int64_t *sel, std::vector<int> &pos) {
+    if (!o || o->single || nsel < 0 || nsel > o->d.nmat || (nsel > 0 && !sel)) return BLU_ERROR_INVALID_ARGUMENT;
+    pos.assign((size_t)o->d.nmat, -1);
+    for (int64_t r = 0; r < nsel; r++) {
+        if (sel[r] < 0 || sel[r] >= o->d.nmat || pos[(size_t)sel[r]] >= 0) return BLU_ERROR_INVALID_ARGUMENT;
+        pos[(size_t)sel[r]] = (int)r;
+    }
+    return BLU_OK;
+}
+
+/* the run mask of the selected slots on the batch until c goes out of scope */
+static int subset_mask(blu_b200 *o, MvCall &c, const std::vector<int> &pos) {
+    const size_t n = pos.size();
+    std::vector<int> run(n);
+    for (size_t k = 0; k < n; k++) run[k] = pos[k] >= 0;
+    int *d_run = nullptr;
+    int st = c.alloc(&d_run, n);
+    if (st != BLU_OK) return st;
+    CK(cudaMemcpyAsync(d_run, run.data(), n * sizeof(int), cudaMemcpyHostToDevice, o->stream));
+    CK(cudaStreamSynchronize(o->stream));      /* (pageable source) */
+    o->d.run = d_run;
+    o->hrun.assign(run.begin(), run.end());
+    return BLU_OK;
+}
+
+/* first non-OK status in selection order; a Reallocate left over means a store could not grow */
+static int subset_statuses(int64_t nsel, std::vector<int> &st_r, int *status) {
+    int worst = BLU_OK;
+    for (int64_t r = 0; r < nsel; r++) {
+        int s = st_r[(size_t)r];
+        if (s == BLU_REALLOCATE) s = BLU_ERROR_OUT_OF_MEMORY;
+        if (status) status[r] = s;
+        if (s != BLU_OK && worst == BLU_OK) worst = s;
+    }
+    return worst;
+}
+
+/* The resident B becomes, for every basis, the B it was last factorized from: the selected slots' new columns, the
+ * others' old ones, compacted into fresh library-owned buffers that replace the old ones.  *maxnz: the most entries
+ * of one selected B.  On failure the old resident B stays. */
+static int subset_rebuild_b(blu_b200 *o, MvCall &c, const std::vector<int> &pos, int64_t nsel, const int64_t *b_begin,
+                            const int64_t *b_end, const int64_t *b_i, const double *b_x, int64_t bnz_total, int64_t *maxnz) {
+    BluDev &d = o->d;
+    const size_t n = (size_t)d.nmat, M = (size_t)d.m, cols = (size_t)nsel * M;
+    const cudaStream_t s = o->stream;
+    /* the B the bases were last factorized from (all-empty columns before the first factorization) */
+    const blu_i64 *ob = o->b_external ? d.b_begin : (const blu_i64 *)o->db_begin, *oe = o->b_external ? d.b_end : (const blu_i64 *)o->db_end;
+    const blu_i64 *oi = o->b_external ? d.b_i : (const blu_i64 *)o->db_i;
+    const double *ox = o->b_external ? d.b_x : o->db_x;
+    const blu_i64 ototal = o->have_b ? d.b_total : 0;
+    blu_i64 *nb = nullptr, *ne = nullptr, *ni = nullptr, *tot = nullptr, *soff = nullptr; double *nx = nullptr; int *dpos = nullptr;
+    int st = c.alloc(&nb, cols);
+    if (st == BLU_OK) st = c.alloc(&ne, cols);
+    if (st == BLU_OK) st = c.alloc(&ni, (size_t)bnz_total);
+    if (st == BLU_OK) st = c.alloc(&nx, (size_t)bnz_total);
+    if (st == BLU_OK) st = c.alloc(&tot, n);
+    if (st == BLU_OK) st = c.alloc(&soff, n);
+    if (st == BLU_OK) st = c.alloc(&dpos, n);
+    if (st != BLU_OK) return st;
+    int64_t *rb = nullptr, *re = nullptr, *ri = nullptr; double *rx = nullptr;      /* the new resident B */
+    auto drop = [&]() { dfree(o, rb); dfree(o, re); dfree(o, ri); dfree(o, rx); };
+    if ((st = dalloc(o, &rb, n * M)) != BLU_OK || (st = dalloc(o, &re, n * M)) != BLU_OK) { drop(); return st; }
+    CK(cudaMemcpyAsync(nb, b_begin, cols * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ne, b_end, cols * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    if (bnz_total > 0) {
+        CK(cudaMemcpyAsync(ni, b_i, (size_t)bnz_total * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(nx, b_x, (size_t)bnz_total * sizeof(double), cudaMemcpyHostToDevice, s));
+    }
+    CK(cudaMemcpyAsync(dpos, pos.data(), n * sizeof(int), cudaMemcpyHostToDevice, s));
+    timer_start(o);
+    BLU_LAUNCH(k_sub_lengths, (int)n, 32, 0, s, d.m, (const int *)dpos, ob, oe, ototal, (const blu_i64 *)nb, (const blu_i64 *)ne,
+               (blu_i64 *)re, (blu_i64 *)rb, tot);
+    o->launches++;
+    CK(cudaGetLastError());
+    std::vector<int64_t> htot(n), hoff(n);
+    CK(cudaMemcpyAsync(htot.data(), tot, n * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    int64_t total = 0;
+    *maxnz = 0;
+    for (size_t k = 0; k < n; k++) {
+        hoff[k] = total; total += htot[k];
+        if (pos[k] >= 0) *maxnz = std::max<int64_t>(*maxnz, htot[k]);
+    }
+    if ((st = dalloc(o, &ri, (size_t)total)) != BLU_OK || (st = dalloc(o, &rx, (size_t)total)) != BLU_OK) { drop(); return st; }
+    CK(cudaMemcpyAsync(soff, hoff.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    BLU_LAUNCH(k_sub_copy, (int)n, 256, 0, s, d.m, (const int *)dpos, ob, oi, ox, (const blu_i64 *)nb, (const blu_i64 *)ni, (const double *)nx,
+               (const blu_i64 *)soff, (blu_i64 *)rb, (blu_i64 *)re, (blu_i64 *)ri, rx);
+    o->launches++;
+    CK(cudaGetLastError());
+    timer_stop(o, 0);      /* (synchronizes: the old B is read no more) */
+    dfree(o, o->db_begin); dfree(o, o->db_end); dfree(o, o->db_i); dfree(o, o->db_x);
+    o->db_begin = rb; o->db_end = re; o->db_i = ri; o->db_x = rx; o->b_cap = total;
+    o->have_b = 1; o->b_external = 0;
+    d.b_total = total;
+    /* a captured graph reads the old B */
+#ifndef BLU_EMU
+    if (o->have_graph) { cudaGraphExecDestroy(o->graph_exec); cudaGraphDestroy(o->graph); }
+#endif
+    o->have_graph = 0;
+    return BLU_OK;
+}
+
+/* blu_batch_factorize for the selected bases only: the resident B is rebuilt, then factorize_resident runs under the
+ * run mask (its Reallocate loop and grow_hungry_slots look at the selected slots only). */
+extern "C" int blu_batch_factorize_subset(blu_batch_t *o, int64_t nsel, const int64_t *sel,
+                                          const int64_t *b_begin, const int64_t *b_end,
+                                          const int64_t *b_i, const double *b_x, int64_t bnz_total, int *status) {
+    std::vector<int> pos;
+    int st = subset_select(o, nsel, sel, pos);
+    if (st != BLU_OK) return st;
+    if (nsel > 0 && (!b_begin || !b_end)) return BLU_ERROR_INVALID_ARGUMENT;
+    if (bnz_total < 0 || (bnz_total > 0 && (!b_i || !b_x))) return BLU_ERROR_INVALID_ARGUMENT;
+    const size_t cols = (size_t)nsel * (size_t)o->d.m;
+    for (size_t q = 0; q < cols; q++)
+        if (b_begin[q] < 0 || b_begin[q] > bnz_total || b_end[q] < 0 || b_end[q] > bnz_total) return BLU_ERROR_INVALID_ARGUMENT;
+    if (nsel == 0) return BLU_OK;
+    CK(cudaSetDevice(o->device));
+    MvCall c(o);
+    int64_t maxnz = 0;
+    if ((st = subset_rebuild_b(o, c, pos, nsel, b_begin, b_end, b_i, b_x, bnz_total, &maxnz)) != BLU_OK) return st;
+    const double rebuild_ms = o->last_ms[0];
+    if ((st = mv_ensure_bt_cap(o, maxnz)) != BLU_OK) return st;
+    if ((st = subset_mask(o, c, pos)) != BLU_OK) return st;
+    const int fst = factorize_resident(o);
+    o->last_ms[0] += rebuild_ms;
+    std::vector<int> st_r((size_t)nsel);
+    for (int64_t r = 0; r < nsel; r++) st_r[(size_t)r] = o->hinfo[(size_t)sel[r]].status;
+    const int worst = subset_statuses(nsel, st_r, status);
+    return fst != BLU_OK ? fst : worst;
+}
+
+/* blu_batch_solve_for_update for the selected bases only: the per-slot kernel under the run mask, right-hand sides
+ * through per-slot begin/end offsets; the solutions of the selected slots are packed on the device and cross the
+ * bus in one copy. */
+extern "C" int blu_batch_solve_for_update_subset(blu_batch_t *o, int64_t nsel, const int64_t *sel, const int64_t *rhs_begin,
+                                                 const int64_t *irhs, const double *xrhs, int want_solution,
+                                                 int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans) {
+    std::vector<int> pos;
+    int st = subset_select(o, nsel, sel, pos);
+    if (st != BLU_OK) return st;
+    if (nsel == 0) return BLU_OK;
+    if (!rhs_begin || (want_solution && (!nzlhs || !ilhs || !xlhs))) return BLU_ERROR_INVALID_ARGUMENT;
+    const int64_t tot = rhs_begin[nsel];
+    if (tot < 0 || (tot > 0 && !irhs)) return BLU_ERROR_INVALID_ARGUMENT;
+    for (int64_t r = 0; r < nsel; r++) if (rhs_begin[r] < 0 || rhs_begin[r] > tot) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    const size_t n = (size_t)o->d.nmat, m = (size_t)o->d.m;
+    const cudaStream_t s = o->stream;
+    MvCall c(o);
+    if ((st = ensure_batch_sparse(o, tot)) != BLU_OK) return st;
+    std::vector<int64_t> hb(n, 0), he(n, 0);
+    for (int64_t r = 0; r < nsel; r++) { hb[(size_t)sel[r]] = rhs_begin[r]; he[(size_t)sel[r]] = rhs_begin[r + 1]; }
+    blu_i64 *db = nullptr, *de = nullptr;
+    if ((st = c.alloc(&db, n)) != BLU_OK || (st = c.alloc(&de, n)) != BLU_OK) return st;
+    CK(cudaMemcpyAsync(db, hb.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(de, he.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    if (tot > 0) CK(cudaMemcpyAsync(o->sm_irhs, irhs, (size_t)tot * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    if (tot > 0 && xrhs) CK(cudaMemcpyAsync(o->sm_xrhs, xrhs, (size_t)tot * sizeof(double), cudaMemcpyHostToDevice, s));
+    if ((st = subset_mask(o, c, pos)) != BLU_OK) return st;
+    std::vector<int> hs(2 * n), st_r((size_t)nsel);
+    for (int attempt = 0; attempt < 40; attempt++) {
+        SpMulti W{(int)n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)db, (const i64 *)de};
+        BLU_LAUNCH(k_solve_sparse, (int)n, 32, 0, s, o->d, 0, (const i64 *)o->sm_irhs, xrhs ? (const double *)o->sm_xrhs : (const double *)nullptr,
+                   trans, 1, want_solution ? 1 : 0, o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
+        o->launches++;
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(hs.data(), o->sm_scal, 2 * n * sizeof(int), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        bool again = false;      /* (the words of the masked-out slots are stale) */
+        for (int64_t r = 0; r < nsel; r++) again = again || hs[2 * (size_t)sel[r]] == BLU_REALLOCATE;
+        if (!again) break;
+        if (grow_batch_stores(o) != BLU_OK) break;      /* blu.rs:268-291; what still says Reallocate is reported as out of memory */
+    }
+    for (int64_t r = 0; r < nsel; r++) st_r[(size_t)r] = hs[2 * (size_t)sel[r]];
+    const int worst = subset_statuses(nsel, st_r, status);
+    o->info_dirty = 1;
+    if (!want_solution) return worst;
+    std::vector<int64_t> hoff((size_t)nsel + 1, 0);
+    for (int64_t r = 0; r < nsel; r++) {
+        const size_t k = (size_t)sel[r];
+        nzlhs[r] = st_r[(size_t)r] == BLU_OK ? hs[2 * k + 1] : -1;
+        hoff[(size_t)r + 1] = hoff[(size_t)r] + std::max<int64_t>(nzlhs[r], 0);
+    }
+    const int64_t fill = hoff[(size_t)nsel];
+    if (fill == 0) return worst;
+    blu_i64 *dsel = nullptr, *doff = nullptr, *pi = nullptr; double *px = nullptr;
+    if ((st = c.alloc(&dsel, (size_t)nsel)) != BLU_OK || (st = c.alloc(&doff, (size_t)nsel + 1)) != BLU_OK ||
+        (st = c.alloc(&pi, (size_t)fill)) != BLU_OK || (st = c.alloc(&px, (size_t)fill)) != BLU_OK) return st;
+    if ((st = up_ensure_host(o, fill)) != BLU_OK) return st;
+    UnitPool &U = o->up;
+    CK(cudaMemcpyAsync(dsel, sel, (size_t)nsel * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(doff, hoff.data(), ((size_t)nsel + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    BLU_LAUNCH(k_sub_pack, (int)nsel, 128, 0, s, (int)m, (const blu_i64 *)dsel, (const blu_i64 *)doff, (const blu_i64 *)o->sm_ilhs,
+               (const double *)o->sm_xout, pi, px);
+    o->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(U.h_ilhs, pi, (size_t)fill * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(U.h_xout, px, (size_t)fill * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    for (int64_t r = 0; r < nsel; r++) {
+        const size_t q = (size_t)hoff[(size_t)r], nz = (size_t)(hoff[(size_t)r + 1] - hoff[(size_t)r]);
+        if (nz) {
+            memcpy(ilhs + (size_t)r * m, U.h_ilhs + q, nz * sizeof(int64_t));
+            memcpy(xlhs + (size_t)r * m, U.h_xout + q, nz * sizeof(double));
+        }
+    }
+    return worst;
+}
+
+/* blu_batch_update for the selected bases only, basis sel[r] with xtbl[r] */
+extern "C" int blu_batch_update_subset(blu_batch_t *o, int64_t nsel, const int64_t *sel, const double *xtbl, int *status) {
+    std::vector<int> pos;
+    int st = subset_select(o, nsel, sel, pos);
+    if (st != BLU_OK) return st;
+    if (nsel == 0) return BLU_OK;
+    if (!xtbl) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    const size_t n = (size_t)o->d.nmat;
+    const cudaStream_t s = o->stream;
+    MvCall c(o);
+    if ((st = ensure_batch_sparse(o, 0)) != BLU_OK) return st;
+    std::vector<double> hx(n, 0.0);
+    for (int64_t r = 0; r < nsel; r++) hx[(size_t)sel[r]] = xtbl[r];
+    CK(cudaMemcpyAsync(o->sm_dbls, hx.data(), n * sizeof(double), cudaMemcpyHostToDevice, s));
+    if ((st = subset_mask(o, c, pos)) != BLU_OK) return st;
+    std::vector<int> hs(n), st_r((size_t)nsel);
+    for (int attempt = 0; attempt < 40; attempt++) {
+        BLU_LAUNCH(k_update, (int)n, 32, 0, s, o->d, 0.0, o->sm_scal, (const double *)o->sm_dbls, attempt > 0 ? 1 : 0);
+        o->launches++;
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(hs.data(), o->sm_scal, n * sizeof(int), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        bool again = false;
+        for (int64_t r = 0; r < nsel; r++) again = again || hs[(size_t)sel[r]] == BLU_REALLOCATE;
+        if (!again) break;
+        if (grow_batch_stores(o) != BLU_OK) break;      /* blu.rs:319-334 */
+    }
+    for (int64_t r = 0; r < nsel; r++) st_r[(size_t)r] = hs[(size_t)sel[r]];
+    o->info_dirty = 1;
+    return subset_statuses(nsel, st_r, status);
 }
 
 /* ------------------------------------------------------------------ */

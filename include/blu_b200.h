@@ -194,6 +194,31 @@ int blu_batch_maxvolume(blu_batch_t *b, int64_t ncol, const int64_t *a_begin, co
                         const int64_t *a_i, const double *a_x, int64_t anz_total,
                         int64_t *basis, int64_t *isbasic, double volumetol, int64_t *nupdate, int *status);
 
+/* The batch calls on a subset of the bases, so that each basis keeps its own schedule: the bases sel[0..nsel)
+ * (distinct, in [0, nmat), any order) run, every other basis keeps its factors, its update history, a pending
+ * solve_for_update, its getters and its status.  Each selected basis ends exactly as its own BLU object would after
+ * the calls it was selected in.  status[r] (may be NULL) receives the code of basis sel[r]; the return value is the
+ * first non-OK one.  nsel < 0 or > nmat, an index outside [0, nmat), a duplicate index, a missing array when
+ * nsel > 0, a malformed rhs_begin, a b_begin/b_end value outside [0, bnz_total], or an object from blu_create:
+ * BLU_ERROR_INVALID_ARGUMENT, nothing runs.  nsel == 0: BLU_OK, nothing runs.  A basis' own errors (a column with
+ * b_end < b_begin, a row index >= m, an update without both solves, ...) go to its status word, the other selected
+ * bases carry on.  Reallocate never escapes.
+ *
+ * blu_batch_factorize_subset: column j of the r-th selected basis is b_i/b_x[b_begin[r*m+j] .. b_end[r*m+j]).
+ * Afterwards the resident B (blu_batch_factorize_resident) holds, for every basis, the B it was last factorized
+ * from, in library-owned memory; a graph captured before (blu_batch_graph_capture) is dropped, and
+ * blu_batch_graph_launch answers BLU_ERROR_INVALID_CALL until the next capture. */
+int blu_batch_factorize_subset(blu_batch_t *b, int64_t nsel, const int64_t *sel,
+                               const int64_t *b_begin, const int64_t *b_end,
+                               const int64_t *b_i, const double *b_x, int64_t bnz_total, int *status);
+/* blu_batch_solve_for_update for the selected bases only; right-hand side r is irhs/xrhs[rhs_begin[r] .. rhs_begin[r+1]),
+ * outputs compacted by r: nzlhs[r], ilhs[r*m ..], xlhs[r*m + n], status[r]. */
+int blu_batch_solve_for_update_subset(blu_batch_t *b, int64_t nsel, const int64_t *sel, const int64_t *rhs_begin,
+                                      const int64_t *irhs, const double *xrhs, int want_solution,
+                                      int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans);
+/* blu_batch_update for the selected bases only, basis sel[r] with xtbl[r] */
+int blu_batch_update_subset(blu_batch_t *b, int64_t nsel, const int64_t *sel, const double *xtbl, int *status);
+
 /* Device-resident variants for throughput measurement: upload once, then time kernels only. */
 int blu_batch_upload(blu_batch_t *b, const int64_t *b_begin, const int64_t *b_end,
                      const int64_t *b_i, const double *b_x, int64_t bnz_total, const double *rhs);
