@@ -97,6 +97,11 @@ def load_library(path=None):
     L.blu_batch_download.argtypes = [vp, f64p, i32p]
     L.blu_batch_factorize_dev.argtypes = [vp, vp, vp, vp, vp, ctypes.c_int64]
     L.blu_batch_solve_dense_dev.argtypes = [vp, vp, vp, ctypes.c_char, vp]
+    L.blu_batch_factorize_subset_dev.argtypes = [vp, vp, vp, vp, vp, vp, ctypes.c_int64, vp]
+    L.blu_batch_solve_for_update_dev.argtypes = [vp, vp, vp, vp, vp, ctypes.c_int, vp, vp, vp, vp, ctypes.c_char]
+    L.blu_batch_update_dev.argtypes = [vp, vp, vp, vp]
+    L.blu_batch_solve_sparse_dev.argtypes = [vp, ctypes.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.c_char]
+    L.blu_batch_solve_dense_multi_dev.argtypes = [vp, ctypes.c_int64, vp, vp, ctypes.c_char, vp]
     L.blu_batch_graph_capture.argtypes = [vp, ctypes.c_char]
     L.blu_batch_graph_launch.argtypes = [vp]
     L.blu_batch_stream.argtypes = [vp]; L.blu_batch_stream.restype = vp
@@ -297,6 +302,7 @@ class BLUBatch(_Base):
             raise RuntimeError(f"blu_batch_create failed with status {st} (no CUDA device? there is no CPU path)")
         self._h = h
         self.nmat, self.m = int(nmat), int(m)
+        self._device = int(device)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -474,6 +480,151 @@ class BLUBatch(_Base):
 
     def solve_dense_dev(self, d_rhs, d_lhs, trans="N", d_status=None):
         return self._L.blu_batch_solve_dense_dev(self._h, d_rhs, d_lhs, _ch(trans), d_status)
+
+    # The basis-change step on torch tensors in device memory (blu_batch_*_dev).  Index arrays are int64, values
+    # float64, masks and statuses int32 (a mask may also be bool); every tensor is contiguous and on the batch's CUDA
+    # device.  On the SIMT emulator library, "device" memory is host memory, and CPU tensors are what it takes.
+    # Outputs come back as tensors; out tensors passed in are written in place, and the entries of bases or units that
+    # do not run keep what they held (zeros when the call allocates them).
+
+    def _torch_device(self):
+        import torch
+        if b"emulation" in self._L.blu_version():      # the SIMT emulation build: its "device" memory is host memory
+            return torch.device("cpu")
+        if getattr(self, "_cuda_index", None) is None:
+            object.__setattr__(self, "_cuda_index", self._device if self._device >= 0 else torch.cuda.current_device())
+        return torch.device("cuda", self._cuda_index)
+
+    def _tensor(self, t, dtype, numel, name, dev):
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{name}: a torch.Tensor is expected")
+        if t.dtype != dtype:
+            raise TypeError(f"{name}: dtype {t.dtype}, expected {dtype}")
+        if t.device != dev:
+            raise ValueError(f"{name}: tensor on {t.device}, the batch is on {dev}")
+        if not t.is_contiguous():
+            raise ValueError(f"{name}: not contiguous")
+        if numel is not None and t.numel() != numel:
+            raise ValueError(f"{name}: {t.numel()} elements, expected {numel}")
+        return t
+
+    def _out(self, t, dtype, numel, name, dev, shape):
+        import torch
+        if t is None:
+            return torch.zeros(shape, dtype=dtype, device=dev)
+        return self._tensor(t, dtype, numel, name, dev)
+
+    def _run_mask(self, run, dev):
+        import torch
+        if run is None:
+            return None
+        if isinstance(run, torch.Tensor) and run.dtype == torch.bool:
+            self._tensor(run, torch.bool, self.nmat, "run", dev)
+            return run.to(torch.int32)
+        return self._tensor(run, torch.int32, self.nmat, "run", dev)
+
+    @staticmethod
+    def _ptr(t):
+        return ctypes.c_void_p(t.data_ptr()) if t is not None and t.numel() > 0 else None
+
+    def _on_stream(self, dev, fn):
+        """run fn (one library call) after everything torch has queued on its current stream of dev"""
+        import torch
+        if dev.type == "cuda":
+            s = torch.cuda.ExternalStream(self._L.blu_batch_stream(self._h), device=dev)
+            s.wait_stream(torch.cuda.current_stream(dev))
+        return fn()
+
+    def factorize_subset_dev(self, b_begin, b_end, b_i, b_x, run=None, status=None):
+        """Refactorize the bases whose run flag is set (every basis for run=None) from B in device memory: column j of
+        basis k is b_i/b_x[b_begin[k*m+j] : b_end[k*m+j]].  Returns (status, status per basis)."""
+        import torch
+        dev = self._torch_device()
+        n, m = self.nmat, self.m
+        bb = self._tensor(b_begin, torch.int64, n * m, "b_begin", dev)
+        be = self._tensor(b_end, torch.int64, n * m, "b_end", dev)
+        bi = self._tensor(b_i, torch.int64, None, "b_i", dev)
+        bx = self._tensor(b_x, torch.float64, bi.numel(), "b_x", dev)
+        r = self._run_mask(run, dev)
+        stat = self._out(status, torch.int32, n, "status", dev, (n,))
+        st = self._on_stream(dev, lambda: self._L.blu_batch_factorize_subset_dev(
+            self._h, self._ptr(r), self._ptr(bb), self._ptr(be), self._ptr(bi), self._ptr(bx), bi.numel(), self._ptr(stat)))
+        return st, stat
+
+    def solve_for_update_dev(self, rhs_begin, irhs, xrhs=None, trans="N", want_solution=0, run=None,
+                             status=None, nzlhs=None, ilhs=None, xlhs=None):
+        """solve_for_update on the bases whose run flag is set: basis k's right-hand side is
+        irhs/xrhs[rhs_begin[k] : rhs_begin[k+1]].  Returns (status, status[nmat], nzlhs[nmat], ilhs[nmat, m],
+        xlhs[nmat, m]); the last three are None without want_solution.  Entry n of basis k's solution is
+        lhs[ilhs[k, n]] = xlhs[k, n] for n < nzlhs[k]."""
+        import torch
+        dev = self._torch_device()
+        n, m = self.nmat, self.m
+        rb = self._tensor(rhs_begin, torch.int64, n + 1, "rhs_begin", dev)
+        ir = self._tensor(irhs, torch.int64, None, "irhs", dev)
+        xr = self._tensor(xrhs, torch.float64, ir.numel(), "xrhs", dev) if xrhs is not None else None
+        r = self._run_mask(run, dev)
+        stat = self._out(status, torch.int32, n, "status", dev, (n,))
+        nz = il = xl = None
+        if want_solution:
+            nz = self._out(nzlhs, torch.int64, n, "nzlhs", dev, (n,))
+            il = self._out(ilhs, torch.int64, n * m, "ilhs", dev, (n, m))
+            xl = self._out(xlhs, torch.float64, n * m, "xlhs", dev, (n, m))
+        st = self._on_stream(dev, lambda: self._L.blu_batch_solve_for_update_dev(
+            self._h, self._ptr(r), self._ptr(rb), self._ptr(ir), self._ptr(xr), 1 if want_solution else 0,
+            self._ptr(nz), self._ptr(il), self._ptr(xl), self._ptr(stat), _ch(trans)))
+        return st, stat, nz, il, xl
+
+    def update_dev(self, xtbl, run=None, status=None):
+        """update on the bases whose run flag is set, basis k with xtbl[k].  Returns (status, status[nmat])."""
+        import torch
+        dev = self._torch_device()
+        x = self._tensor(xtbl, torch.float64, self.nmat, "xtbl", dev)
+        r = self._run_mask(run, dev)
+        stat = self._out(status, torch.int32, self.nmat, "status", dev, (self.nmat,))
+        st = self._on_stream(dev, lambda: self._L.blu_batch_update_dev(self._h, self._ptr(r), self._ptr(x), self._ptr(stat)))
+        return st, stat
+
+    def solve_sparse_dev(self, unit_begin, rhs_begin, irhs, xrhs, trans="N", nunits=None,
+                         status=None, nzlhs=None, ilhs=None, xlhs=None):
+        """solve_sparse for every unit: basis k owns units unit_begin[k] : unit_begin[k+1], unit u solves with
+        irhs/xrhs[rhs_begin[u] : rhs_begin[u+1]].  nunits is read from unit_begin[-1] when not given (one small copy
+        to the host).  Returns (status, status[nunits], nzlhs[nunits], ilhs[nunits, m], xlhs[nunits, m])."""
+        import torch
+        dev = self._torch_device()
+        m = self.m
+        ub = self._tensor(unit_begin, torch.int64, self.nmat + 1, "unit_begin", dev)
+        nu = int(ub[-1].item()) if nunits is None else int(nunits)
+        if nu < 0:
+            raise ValueError("nunits < 0")
+        rb = self._tensor(rhs_begin, torch.int64, nu + 1, "rhs_begin", dev)
+        ir = self._tensor(irhs, torch.int64, None, "irhs", dev)
+        xr = self._tensor(xrhs, torch.float64, ir.numel(), "xrhs", dev)
+        stat = self._out(status, torch.int32, nu, "status", dev, (nu,))
+        nz = self._out(nzlhs, torch.int64, nu, "nzlhs", dev, (nu,))
+        il = self._out(ilhs, torch.int64, nu * m, "ilhs", dev, (nu, m))
+        xl = self._out(xlhs, torch.float64, nu * m, "xlhs", dev, (nu, m))
+        st = self._on_stream(dev, lambda: self._L.blu_batch_solve_sparse_dev(
+            self._h, nu, self._ptr(ub), self._ptr(rb), self._ptr(ir), self._ptr(xr), self._ptr(nz), self._ptr(il), self._ptr(xl),
+            self._ptr(stat), _ch(trans)))
+        return st, stat, nz, il, xl
+
+    def solve_dense_multi_dev(self, rhs, trans="N", lhs=None, status=None):
+        """rhs[nmat, nrhs, m] (any contiguous tensor of nmat*nrhs*m values) -> (status, lhs[nmat, nrhs, m],
+        status[nmat, nrhs]): solve_dense for every right-hand side of every basis."""
+        import torch
+        dev = self._torch_device()
+        n, m = self.nmat, self.m
+        r = self._tensor(rhs, torch.float64, None, "rhs", dev)
+        if r.numel() % (n * m):
+            raise ValueError("rhs: not a whole number of right-hand sides per basis")
+        nrhs = r.numel() // (n * m)
+        x = self._out(lhs, torch.float64, r.numel(), "lhs", dev, (n, nrhs, m))
+        stat = self._out(status, torch.int32, n * nrhs, "status", dev, (n, nrhs))
+        st = self._on_stream(dev, lambda: self._L.blu_batch_solve_dense_multi_dev(
+            self._h, nrhs, self._ptr(r), self._ptr(x), _ch(trans), self._ptr(stat)))
+        return st, x, stat
 
     def graph_capture(self, trans="N"):
         return self._L.blu_batch_graph_capture(self._h, _ch(trans))

@@ -13,6 +13,7 @@
 #include "blu_sparse.cuh"
 #include "blu_maxvolume.cuh"
 #include "blu_subset.cuh"
+#include "blu_dev_calls.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -87,6 +88,7 @@ struct blu_b200 {
     int b_external;             /* B lives in the caller's device buffers (blu_batch_factorize_dev) */
     cudaGraph_t graph; cudaGraphExec_t graph_exec; int have_graph; char graph_trans;   /* blu_batch_graph_* */
     std::vector<char> hrun;     /* host copy of d.run during a subset call (empty: every slot runs) */
+    blu_u64 *d_sum, *h_sum;     /* the summary of a device-resident call (blu_dev_calls.cuh) and its pinned landing place */
     double time_factorize, time_solve, time_update;
 };
 
@@ -240,6 +242,7 @@ static int create_common(blu_b200 **out, int64_t nmat, int64_t m, int64_t bnz_ca
     o->solve_units = 8192;      /* configs[1], 16,384 units (DESIGN.md §5): beyond this the kernels gain ~10 %, the call nothing */
     if (const char *e = getenv("BLU_B200_SOLVE_UNITS")) { long v = atol(e); if (v >= 1 && v <= (1L << 24)) o->solve_units = (int)v; }   /* tuning / test knob */
     o->h_scal = nullptr; o->h_ilhs = nullptr; o->h_xout = nullptr;
+    o->d_sum = nullptr; o->h_sum = nullptr;
     o->time_factorize = o->time_solve = o->time_update = 0.0;
     BluDev &d = o->d;
     memset(&d, 0, sizeof d);
@@ -331,6 +334,7 @@ static void destroy_common(blu_b200 *o) {
     if (o->h_xout) cudaFreeHost(o->h_xout);
     if (o->up.h_ilhs) cudaFreeHost(o->up.h_ilhs);
     if (o->up.h_xout) cudaFreeHost(o->up.h_xout);
+    if (o->h_sum) cudaFreeHost(o->h_sum);
 #ifndef BLU_EMU
     cudaEventDestroy(o->ev0); cudaEventDestroy(o->ev1);
     for (int q = 0; q < 4; q++) cudaEventDestroy(o->ev_k[q]);
@@ -2024,54 +2028,89 @@ static int subset_statuses(int64_t nsel, std::vector<int> &st_r, int *status) {
     return worst;
 }
 
-/* The resident B becomes, for every basis, the B it was last factorized from: the selected slots' new columns, the
- * others' old ones, compacted into fresh library-owned buffers that replace the old ones.  *maxnz: the most entries
- * of one selected B.  On failure the old resident B stays. */
-static int subset_rebuild_b(blu_b200 *o, MvCall &c, const std::vector<int> &pos, int64_t nsel, const int64_t *b_begin,
-                            const int64_t *b_end, const int64_t *b_i, const double *b_x, int64_t bnz_total, int64_t *maxnz) {
+/* The summary of a device-resident call (blu_dev_calls.cuh): allocated on first use, cleared before each launch
+ * attempt, read into pinned memory after it (DEV_SUM_N words, whatever the size of the batch). */
+static int dev_sum_ensure(blu_b200 *o) {
+    if (o->d_sum) return BLU_OK;
+    int st = dalloc(o, &o->d_sum, DEV_SUM_N);
+    if (st != BLU_OK) return st;
+    if (cudaMallocHost((void **)&o->h_sum, DEV_SUM_N * sizeof(blu_u64)) != cudaSuccess) { cudaGetLastError(); o->h_sum = nullptr; dfree(o, o->d_sum); o->d_sum = nullptr; return BLU_ERROR_OUT_OF_MEMORY; }
+    return BLU_OK;
+}
+static int dev_sum_reset(blu_b200 *o) {
+    CK(cudaMemsetAsync(o->d_sum, 0, DEV_SUM_N * sizeof(blu_u64), o->stream));
+    CK(cudaMemsetAsync(o->d_sum + DEV_SUM_FIRST, 0xff, sizeof(blu_u64), o->stream));
+    return BLU_OK;
+}
+static int dev_sum_read(blu_b200 *o) {
+    CK(cudaMemcpyAsync(o->h_sum, o->d_sum, DEV_SUM_N * sizeof(blu_u64), cudaMemcpyDeviceToHost, o->stream));
+    CK(cudaStreamSynchronize(o->stream));
+    return BLU_OK;
+}
+/* the first non-OK status of the summary (index order), BLU_OK if there is none */
+static int dev_sum_first(const blu_b200 *o) {
+    const blu_u64 f = o->h_sum[DEV_SUM_FIRST];
+    return f == DEV_SUM_NONE ? BLU_OK : (int)(unsigned)(f & 0xffffffffu);
+}
+static int grid_of(int64_t n, int per) { return (int)std::max<int64_t>(1, std::min<int64_t>((n + per - 1) / per, 4096)); }
+/* k_dev_finish over n slots or units; nothing to do for n == 0 */
+static int dev_finish(blu_b200 *o, int n, int64_t idx0, const int *run, const int *scal, int stride, int *status, int64_t *nzlhs) {
+    if (n <= 0) return BLU_OK;
+    BLU_LAUNCH(k_dev_finish, grid_of(n, 256), 256, 0, o->stream, n, (blu_i64)idx0, run, scal, stride, status, (blu_i64 *)nzlhs, o->d_sum);
+    o->launches++;
+    CK(cudaGetLastError());
+    return BLU_OK;
+}
+
+/* The resident B becomes, for every basis, the B it was last factorized from: the new columns of the slots with
+ * pos[k] >= 0 (column j of slot k at nb/ne[pos[k]*m + j], entries in ni/nx, all in device memory), the others' old
+ * ones, compacted into fresh library-owned buffers that replace the old ones.  *maxnz: the most entries of one new B.
+ * The slots' entry counts are scanned on the host when it has the selection (hpos, the host copy of dpos), and on
+ * the device otherwise, so that only the new total and *maxnz come back.  On failure the old resident B stays. */
+static int rebuild_b(blu_b200 *o, MvCall &c, const int *dpos, const std::vector<int> *hpos, const blu_i64 *nb, const blu_i64 *ne,
+                     const blu_i64 *ni, const double *nx, int64_t *maxnz) {
     BluDev &d = o->d;
-    const size_t n = (size_t)d.nmat, M = (size_t)d.m, cols = (size_t)nsel * M;
+    const size_t n = (size_t)d.nmat, M = (size_t)d.m;
     const cudaStream_t s = o->stream;
     /* the B the bases were last factorized from (all-empty columns before the first factorization) */
     const blu_i64 *ob = o->b_external ? d.b_begin : (const blu_i64 *)o->db_begin, *oe = o->b_external ? d.b_end : (const blu_i64 *)o->db_end;
     const blu_i64 *oi = o->b_external ? d.b_i : (const blu_i64 *)o->db_i;
     const double *ox = o->b_external ? d.b_x : o->db_x;
     const blu_i64 ototal = o->have_b ? d.b_total : 0;
-    blu_i64 *nb = nullptr, *ne = nullptr, *ni = nullptr, *tot = nullptr, *soff = nullptr; double *nx = nullptr; int *dpos = nullptr;
-    int st = c.alloc(&nb, cols);
-    if (st == BLU_OK) st = c.alloc(&ne, cols);
-    if (st == BLU_OK) st = c.alloc(&ni, (size_t)bnz_total);
-    if (st == BLU_OK) st = c.alloc(&nx, (size_t)bnz_total);
-    if (st == BLU_OK) st = c.alloc(&tot, n);
+    blu_i64 *tot = nullptr, *soff = nullptr;
+    int st = c.alloc(&tot, n);
     if (st == BLU_OK) st = c.alloc(&soff, n);
-    if (st == BLU_OK) st = c.alloc(&dpos, n);
+    if (st == BLU_OK && !hpos) st = dev_sum_ensure(o);
     if (st != BLU_OK) return st;
     int64_t *rb = nullptr, *re = nullptr, *ri = nullptr; double *rx = nullptr;      /* the new resident B */
     auto drop = [&]() { dfree(o, rb); dfree(o, re); dfree(o, ri); dfree(o, rx); };
     if ((st = dalloc(o, &rb, n * M)) != BLU_OK || (st = dalloc(o, &re, n * M)) != BLU_OK) { drop(); return st; }
-    CK(cudaMemcpyAsync(nb, b_begin, cols * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ne, b_end, cols * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-    if (bnz_total > 0) {
-        CK(cudaMemcpyAsync(ni, b_i, (size_t)bnz_total * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(nx, b_x, (size_t)bnz_total * sizeof(double), cudaMemcpyHostToDevice, s));
-    }
-    CK(cudaMemcpyAsync(dpos, pos.data(), n * sizeof(int), cudaMemcpyHostToDevice, s));
     timer_start(o);
-    BLU_LAUNCH(k_sub_lengths, (int)n, 32, 0, s, d.m, (const int *)dpos, ob, oe, ototal, (const blu_i64 *)nb, (const blu_i64 *)ne,
-               (blu_i64 *)re, (blu_i64 *)rb, tot);
+    BLU_LAUNCH(k_sub_lengths, (int)n, 32, 0, s, d.m, dpos, ob, oe, ototal, nb, ne, (blu_i64 *)re, (blu_i64 *)rb, tot);
     o->launches++;
     CK(cudaGetLastError());
-    std::vector<int64_t> htot(n), hoff(n);
-    CK(cudaMemcpyAsync(htot.data(), tot, n * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
     int64_t total = 0;
     *maxnz = 0;
-    for (size_t k = 0; k < n; k++) {
-        hoff[k] = total; total += htot[k];
-        if (pos[k] >= 0) *maxnz = std::max<int64_t>(*maxnz, htot[k]);
+    if (hpos) {
+        std::vector<int64_t> htot(n), hoff(n);
+        CK(cudaMemcpyAsync(htot.data(), tot, n * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        for (size_t k = 0; k < n; k++) {
+            hoff[k] = total; total += htot[k];
+            if ((*hpos)[k] >= 0) *maxnz = std::max<int64_t>(*maxnz, htot[k]);
+        }
+        CK(cudaMemcpyAsync(soff, hoff.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        CK(cudaStreamSynchronize(s));      /* (pageable source) */
+    } else {
+        if ((st = dev_sum_reset(o)) != BLU_OK) return st;
+        BLU_LAUNCH(k_dev_scan, 1, 256, 0, s, (int)n, dpos, (const blu_i64 *)tot, soff, o->d_sum);
+        o->launches++;
+        CK(cudaGetLastError());
+        if ((st = dev_sum_read(o)) != BLU_OK) return st;
+        total = (int64_t)o->h_sum[DEV_SUM_TOTAL];
+        *maxnz = (int64_t)o->h_sum[DEV_SUM_MAXNZ];
     }
     if ((st = dalloc(o, &ri, (size_t)total)) != BLU_OK || (st = dalloc(o, &rx, (size_t)total)) != BLU_OK) { drop(); return st; }
-    CK(cudaMemcpyAsync(soff, hoff.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     BLU_LAUNCH(k_sub_copy, (int)n, 256, 0, s, d.m, (const int *)dpos, ob, oi, ox, (const blu_i64 *)nb, (const blu_i64 *)ni, (const double *)nx,
                (const blu_i64 *)soff, (blu_i64 *)rb, (blu_i64 *)re, (blu_i64 *)ri, rx);
     o->launches++;
@@ -2087,6 +2126,29 @@ static int subset_rebuild_b(blu_b200 *o, MvCall &c, const std::vector<int> &pos,
 #endif
     o->have_graph = 0;
     return BLU_OK;
+}
+
+/* rebuild_b from host arrays: the selection's new B (column j of the r-th selected basis at b_begin/b_end[r*m + j])
+ * goes up to the device first */
+static int subset_rebuild_b(blu_b200 *o, MvCall &c, const std::vector<int> &pos, int64_t nsel, const int64_t *b_begin,
+                            const int64_t *b_end, const int64_t *b_i, const double *b_x, int64_t bnz_total, int64_t *maxnz) {
+    const size_t n = (size_t)o->d.nmat, cols = (size_t)nsel * (size_t)o->d.m;
+    const cudaStream_t s = o->stream;
+    blu_i64 *nb = nullptr, *ne = nullptr, *ni = nullptr; double *nx = nullptr; int *dpos = nullptr;
+    int st = c.alloc(&nb, cols);
+    if (st == BLU_OK) st = c.alloc(&ne, cols);
+    if (st == BLU_OK) st = c.alloc(&ni, (size_t)bnz_total);
+    if (st == BLU_OK) st = c.alloc(&nx, (size_t)bnz_total);
+    if (st == BLU_OK) st = c.alloc(&dpos, n);
+    if (st != BLU_OK) return st;
+    CK(cudaMemcpyAsync(nb, b_begin, cols * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ne, b_end, cols * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    if (bnz_total > 0) {
+        CK(cudaMemcpyAsync(ni, b_i, (size_t)bnz_total * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(nx, b_x, (size_t)bnz_total * sizeof(double), cudaMemcpyHostToDevice, s));
+    }
+    CK(cudaMemcpyAsync(dpos, pos.data(), n * sizeof(int), cudaMemcpyHostToDevice, s));
+    return rebuild_b(o, c, dpos, &pos, nb, ne, ni, nx, maxnz);
 }
 
 /* blu_batch_factorize for the selected bases only: the resident B is rebuilt, then factorize_resident runs under the
@@ -2227,6 +2289,222 @@ extern "C" int blu_batch_update_subset(blu_batch_t *o, int64_t nsel, const int64
     for (int64_t r = 0; r < nsel; r++) st_r[(size_t)r] = hs[(size_t)sel[r]];
     o->info_dirty = 1;
     return subset_statuses(nsel, st_r, status);
+}
+
+/* ------------------------------------------------------------------ */
+/* batch: the basis-change step on caller-owned device buffers         */
+/* ------------------------------------------------------------------ */
+
+/* The argument check of a device-resident call: the kernel queued by `check` counts violations into the summary,
+ * which the host reads before anything else is queued. */
+template <typename F> static int dev_validate(blu_b200 *o, F check) {
+    int st = dev_sum_reset(o);
+    if (st != BLU_OK) return st;
+    check();
+    o->launches++;
+    CK(cudaGetLastError());
+    if ((st = dev_sum_read(o)) != BLU_OK) return st;
+    return o->h_sum[DEV_SUM_BAD] ? BLU_ERROR_INVALID_ARGUMENT : BLU_OK;
+}
+
+/* blu_batch_factorize_subset with a device run mask and B in the caller's device memory, per-basis layout.  The host
+ * reads the mask (to know the selection) and the info block (as factorize_resident does); the resident B is rebuilt
+ * on the device from the old one and the caller's. */
+extern "C" int blu_batch_factorize_subset_dev(blu_batch_t *o, const int *d_run, const int64_t *d_b_begin, const int64_t *d_b_end,
+                                              const int64_t *d_b_i, const double *d_b_x, int64_t bnz_total, int *d_status) {
+    if (!o || o->single || !d_b_begin || !d_b_end || bnz_total < 0 || (bnz_total > 0 && (!d_b_i || !d_b_x))) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    BluDev &d = o->d;
+    const int n = d.nmat;
+    const cudaStream_t s = o->stream;
+    std::vector<int> run((size_t)n, 1);
+    if (d_run) {
+        CK(cudaMemcpyAsync(run.data(), d_run, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    if (std::none_of(run.begin(), run.end(), [](int r) { return r != 0; })) return BLU_OK;
+    int st = dev_sum_ensure(o);
+    if (st != BLU_OK) return st;
+    st = dev_validate(o, [&]() {
+        BLU_LAUNCH(k_dev_check_b, n, 128, 0, s, d.m, d_run, (const blu_i64 *)d_b_begin, (const blu_i64 *)d_b_end, (blu_i64)bnz_total, o->d_sum);
+    });
+    if (st != BLU_OK) return st;
+    MvCall c(o);
+    int *dpos = nullptr, *scal = nullptr;
+    if ((st = c.alloc(&dpos, (size_t)n)) != BLU_OK || (st = c.alloc(&scal, (size_t)n)) != BLU_OK) return st;
+    BLU_LAUNCH(k_dev_pos, grid_of(n, 256), 256, 0, s, n, d_run, dpos);
+    o->launches++;
+    CK(cudaGetLastError());
+    int64_t maxnz = 0;
+    if ((st = rebuild_b(o, c, dpos, nullptr, (const blu_i64 *)d_b_begin, (const blu_i64 *)d_b_end, (const blu_i64 *)d_b_i, d_b_x, &maxnz)) != BLU_OK)
+        return st;
+    const double rebuild_ms = o->last_ms[0];
+    if ((st = mv_ensure_bt_cap(o, maxnz)) != BLU_OK) return st;
+    if (d_run) { d.run = d_run; o->hrun.assign(run.begin(), run.end()); }
+    const int fst = factorize_resident(o);
+    o->last_ms[0] += rebuild_ms;
+    BLU_LAUNCH(k_dev_info_status, grid_of(n, 256), 256, 0, s, n, (const BluInfo *)d.info, scal);
+    o->launches++;
+    CK(cudaGetLastError());
+    if ((st = dev_sum_reset(o)) != BLU_OK || (st = dev_finish(o, n, 0, d_run, scal, 1, d_status, nullptr)) != BLU_OK) return st;
+    int worst = BLU_OK;
+    for (int k = 0; k < n && worst == BLU_OK; k++) {
+        const int sk = o->hinfo[(size_t)k].status;
+        if (run[(size_t)k] && sk != BLU_OK) worst = sk == BLU_REALLOCATE ? BLU_ERROR_OUT_OF_MEMORY : sk;
+    }
+    return fst != BLU_OK ? fst : worst;
+}
+
+/* blu_batch_solve_for_update (d_run == NULL) or blu_batch_solve_for_update_subset (the set bits of d_run) on device
+ * buffers: the per-slot kernel reads the caller's right-hand sides and writes the caller's ilhs / xlhs at k * m;
+ * k_dev_finish turns the status words into the caller's status and nzlhs.  Per launch attempt the host reads the
+ * summary, nothing else. */
+extern "C" int blu_batch_solve_for_update_dev(blu_batch_t *o, const int *d_run, const int64_t *d_rhs_begin, const int64_t *d_irhs,
+                                              const double *d_xrhs, int want_solution, int64_t *d_nzlhs, int64_t *d_ilhs, double *d_xlhs,
+                                              int *d_status, char trans) {
+    if (!o || o->single || !d_rhs_begin || (want_solution && (!d_nzlhs || !d_ilhs || !d_xlhs))) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    const int n = o->d.nmat;
+    const cudaStream_t s = o->stream;
+    int st = ensure_batch_sparse(o, 0);
+    if (st == BLU_OK) st = dev_sum_ensure(o);
+    if (st != BLU_OK) return st;
+    st = dev_validate(o, [&]() {
+        BLU_LAUNCH(k_dev_check_rhs, grid_of(n + 1, 256), 256, 0, s, n, d_run, (const blu_i64 *)d_rhs_begin, d_irhs ? 0 : 1, o->d_sum);
+    });
+    if (st != BLU_OK) return st;
+    MvCall c(o);
+    o->d.run = d_run;
+    i64 *il = want_solution ? (i64 *)d_ilhs : (i64 *)o->sm_ilhs;
+    double *xl = want_solution ? d_xlhs : o->sm_xout;
+    for (int attempt = 0; attempt < 40; attempt++) {
+        SpMulti W{n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)d_rhs_begin, nullptr};
+        BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, o->d, 0, (const i64 *)d_irhs, d_xrhs, trans, 1, want_solution ? 1 : 0, o->sm_scal, il, xl, W);
+        o->launches++;
+        CK(cudaGetLastError());
+        if ((st = dev_sum_reset(o)) != BLU_OK || (st = dev_finish(o, n, 0, d_run, o->sm_scal, 2, d_status, want_solution ? d_nzlhs : nullptr)) != BLU_OK ||
+            (st = dev_sum_read(o)) != BLU_OK) return st;
+        if (!o->h_sum[DEV_SUM_REALLOC]) break;
+        /* blu.rs:268-291: grow and run those bases again; what still says Reallocate is reported as out of memory */
+        if (grow_batch_stores(o) != BLU_OK) break;
+    }
+    o->info_dirty = 1;
+    return dev_sum_first(o);
+}
+
+/* blu_batch_update / blu_batch_update_subset on device buffers: basis k with d_xtbl[k] */
+extern "C" int blu_batch_update_dev(blu_batch_t *o, const int *d_run, const double *d_xtbl, int *d_status) {
+    if (!o || o->single || !d_xtbl) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    const int n = o->d.nmat;
+    const cudaStream_t s = o->stream;
+    int st = ensure_batch_sparse(o, 0);
+    if (st == BLU_OK) st = dev_sum_ensure(o);
+    if (st != BLU_OK) return st;
+    MvCall c(o);
+    o->d.run = d_run;
+    for (int attempt = 0; attempt < 40; attempt++) {
+        BLU_LAUNCH(k_update, n, 32, 0, s, o->d, 0.0, o->sm_scal, d_xtbl, attempt > 0 ? 1 : 0);
+        o->launches++;
+        CK(cudaGetLastError());
+        if ((st = dev_sum_reset(o)) != BLU_OK || (st = dev_finish(o, n, 0, d_run, o->sm_scal, 1, d_status, nullptr)) != BLU_OK ||
+            (st = dev_sum_read(o)) != BLU_OK) return st;
+        if (!o->h_sum[DEV_SUM_REALLOC]) break;
+        if (grow_batch_stores(o) != BLU_OK) break;      /* blu.rs:319-334 */
+    }
+    o->info_dirty = 1;
+    return dev_sum_first(o);
+}
+
+/* blu_batch_solve_sparse on device buffers.  The unit table is built on the device; the chunks run back to back, each
+ * one's solutions moved from the pool to the caller's ilhs / xlhs at u * m by k_dev_unpack; one summary read at the
+ * end. */
+extern "C" int blu_batch_solve_sparse_dev(blu_batch_t *o, int64_t nunits, const int64_t *d_unit_begin, const int64_t *d_rhs_begin,
+                                          const int64_t *d_irhs, const double *d_xrhs, int64_t *d_nzlhs, int64_t *d_ilhs, double *d_xlhs,
+                                          int *d_status, char trans) {
+    if (!o || o->single || nunits < 0 || nunits > 0x7fffffff || !d_unit_begin) return BLU_ERROR_INVALID_ARGUMENT;
+    if (nunits > 0 && (!d_rhs_begin || !d_nzlhs || !d_ilhs || !d_xlhs)) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    const double tic = wall_now();
+    const int nmat = o->d.nmat;
+    const size_t m = (size_t)o->d.m;
+    const cudaStream_t s = o->stream;
+    int st = dev_sum_ensure(o);
+    if (st != BLU_OK) return st;
+    st = dev_validate(o, [&]() {
+        BLU_LAUNCH(k_dev_check_units, grid_of(std::max<int64_t>(nmat, nunits), 256), 256, 0, s, nmat, (const blu_i64 *)d_unit_begin,
+                   (blu_i64)nunits, (const blu_i64 *)d_rhs_begin, (d_irhs && d_xrhs) ? 0 : 1, o->d_sum);
+    });
+    if (st != BLU_OK || nunits == 0) return st;
+    const int64_t P = std::min<int64_t>(nunits, o->solve_units);
+    st = up_ensure_units(o, nunits);
+    if (st == BLU_OK) st = up_ensure_sparse(o, P, 0);
+    if (st != BLU_OK) return st;
+    UnitPool &U = o->up;
+    BLU_LAUNCH(k_dev_unit_slots, grid_of(nunits, 256), 256, 0, s, nmat, (blu_i64)nunits, (const blu_i64 *)d_unit_begin, U.slot);
+    o->launches++;
+    CK(cudaGetLastError());
+    timer_start(o);
+    BLU_LAUNCH(k_garbage_perm, nmat, 32, 0, s, o->d);
+    o->launches++;
+    CK(cudaGetLastError());
+    if ((st = dev_sum_reset(o)) != BLU_OK) return st;
+    for (int64_t c0 = 0; c0 < nunits; c0 += P) {
+        const int cnt = (int)std::min<int64_t>(P, nunits - c0);
+        CK(cudaMemsetAsync(U.fill, 0, sizeof(blu_u64), s));
+        SpMulti W{cnt, 0, 0, U.ints, U.dbls, U.markers, (const i64 *)d_rhs_begin + c0, nullptr, U.slot + c0, U.fill, (i64 *)U.off};
+        BLU_LAUNCH(k_solve_sparse<true>, cnt, 32, 0, s, o->d, 0, (const i64 *)d_irhs, d_xrhs, trans, 0, 1, U.scal, (i64 *)U.ilhs, U.xout, W);
+        BLU_LAUNCH(k_dev_unpack, cnt, 128, 0, s, (int)m, (const int *)U.scal, (const blu_i64 *)U.off, (const blu_i64 *)U.ilhs,
+                   (const double *)U.xout, (blu_i64 *)d_ilhs + (size_t)c0 * m, d_xlhs + (size_t)c0 * m);
+        o->launches += 2;
+        CK(cudaGetLastError());
+        if ((st = dev_finish(o, cnt, c0, nullptr, U.scal, 2, d_status, d_nzlhs)) != BLU_OK) return st;
+    }
+    timer_stop(o, 1);
+    if ((st = dev_sum_read(o)) != BLU_OK) return st;
+    o->info_dirty = 1;
+    o->time_solve += wall_now() - tic;
+    return dev_sum_first(o);
+}
+
+/* blu_batch_solve_dense_multi on device buffers: the chunks read d_rhs and write d_lhs in place, back to back, with one
+ * summary read at the end */
+extern "C" int blu_batch_solve_dense_multi_dev(blu_batch_t *o, int64_t nrhs, const double *d_rhs, double *d_lhs, char trans, int *d_status) {
+    if (!o || o->single || nrhs < 0 || (nrhs > 0 && (!d_rhs || !d_lhs))) return BLU_ERROR_INVALID_ARGUMENT;
+    if (nrhs == 0) return BLU_OK;
+    CK(cudaSetDevice(o->device));
+    const double tic = wall_now();
+    const size_t m = (size_t)o->d.m;
+    const int64_t nunits = (int64_t)o->d.nmat * nrhs;
+    if (nunits > 0x7fffffff) return BLU_ERROR_INVALID_ARGUMENT;
+    const int64_t P = std::min<int64_t>(nunits, o->solve_units);
+    const cudaStream_t s = o->stream;
+    int st = dev_sum_ensure(o);
+    if (st == BLU_OK) st = up_ensure_units(o, nunits);
+    if (st == BLU_OK) st = up_ensure_dense(o, P);
+    if (st != BLU_OK) return st;
+    UnitPool &U = o->up;
+    BLU_LAUNCH(k_dev_dense_slots, grid_of(nunits, 256), 256, 0, s, (blu_i64)nunits, (blu_i64)nrhs, U.slot);
+    o->launches++;
+    CK(cudaGetLastError());
+    timer_start(o);
+    BLU_LAUNCH(k_garbage_perm, o->d.nmat, 32, 0, s, o->d);
+    o->launches++;
+    CK(cudaGetLastError());
+    if ((st = dev_sum_reset(o)) != BLU_OK) return st;
+    for (int64_t c0 = 0; c0 < nunits; c0 += P) {
+        const int cnt = (int)std::min<int64_t>(P, nunits - c0);
+        BLU_LAUNCH(k_solve_dense, cnt, 32, 0, s, o->d, d_rhs + (size_t)c0 * m, d_lhs + (size_t)c0 * m, trans, U.dstatus, U.work, cnt,
+                   (const int *)U.slot + c0);
+        o->launches++;
+        CK(cudaGetLastError());
+        if ((st = dev_finish(o, cnt, c0, nullptr, U.dstatus, 1, d_status, nullptr)) != BLU_OK) return st;
+    }
+    timer_stop(o, 1);
+    if ((st = dev_sum_read(o)) != BLU_OK) return st;
+    o->info_dirty = 1;
+    o->time_solve += wall_now() - tic;
+    return dev_sum_first(o);
 }
 
 /* ------------------------------------------------------------------ */

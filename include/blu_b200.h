@@ -231,6 +231,56 @@ int blu_batch_download(blu_batch_t *b, double *lhs, int *status);
 int blu_batch_factorize_dev(blu_batch_t *b, const int64_t *d_b_begin, const int64_t *d_b_end,
                             const int64_t *d_b_i, const double *d_b_x, int64_t bnz_total);
 int blu_batch_solve_dense_dev(blu_batch_t *b, const double *d_rhs, double *d_lhs, char trans, int *d_status);
+/* The basis-change step of a batch on caller-owned DEVICE buffers, for a driver that keeps its state on the GPU.
+ * Every array argument is device memory on the batch's device, in the layout of the host variant, except that the
+ * per-basis arrays of a masked call keep the per-basis layout (index k) and are not compacted by selection.
+ * d_run: NULL = every basis runs; otherwise nmat ints on the device, nonzero = this basis runs.
+ *
+ * - Same results: every basis that runs ends exactly as the host variant leaves it, bit for bit (statuses, nzlhs, the
+ *   order of ilhs, the values, every getter including l_flops / u_flops / r_flops / update_cost / nupdate, later solves
+ *   and get_factors).  A masked call matches the *_subset call whose sel is the set bits of d_run, in index order; with
+ *   d_run == NULL the whole-batch call.
+ * - A basis that does not run does not move: its state, a pending solve_for_update pair, its getters, and its entries
+ *   of d_status, d_nzlhs, d_ilhs, d_xlhs, d_xtbl are neither read nor written.  An all-zero mask changes nothing and
+ *   returns BLU_OK.
+ * - The arguments the host cannot see are checked on the device before anything runs: rhs_begin offsets of running
+ *   bases (and rhs_begin[nmat] >= 0), B offsets of running bases within [0, bnz_total], unit_begin[0] == 0, unit_begin
+ *   non-decreasing, unit_begin[nmat] == nunits, unit rhs_begin offsets within [0, rhs_begin[nunits]], a non-empty
+ *   right-hand side set without its index (or value) array.  A violation: BLU_ERROR_INVALID_ARGUMENT, no state change, no
+ *   output written.  A missing pointer, nrhs < 0 or nunits < 0 is rejected on the host the same way.  A basis' or unit's
+ *   own errors go to its status word, as in the host variants.
+ * - The return value is the first non-OK status among the running bases or units in index order, found on the device.
+ * - Reallocate never escapes: the stores are grown and the bases that asked run again (at most 40 attempts); only then
+ *   does the host read per-basis data (the info block).
+ * - Host traffic: solve_for_update_dev, update_dev, solve_sparse_dev and solve_dense_multi_dev copy nothing between host
+ *   and device whose size grows with nmat, nunits, m or the right-hand sides: per launch attempt (and once for the
+ *   argument check) the host reads a summary of DEV_SUM_N = 5 words from pinned memory.  solve_sparse_dev runs its chunks
+ *   of BLU_B200_SOLVE_UNITS units back to back and writes the solutions to d_ilhs[u*m ..] / d_xlhs[u*m ..].
+ * - The calls queue on the batch's stream (blu_batch_set_stream applies) and return when their outputs are complete.
+ *   last_kernel_ms and launch_count account for them as for the host variants.
+ * - d_status and, when want_solution == 0, d_nzlhs / d_ilhs / d_xlhs may be NULL.
+ *
+ * blu_batch_factorize_subset_dev: column j of basis k is d_b_i/d_b_x[d_b_begin[k*m+j] .. d_b_end[k*m+j]).  As after
+ * blu_batch_factorize_subset, the resident B holds, for every basis, the B it was last factorized from in library-owned
+ * memory (the caller's buffers need not outlive the call; it is rebuilt on the device and only its new size comes
+ * back), a captured graph is dropped and blu_batch_graph_launch answers BLU_ERROR_INVALID_CALL until the next capture.
+ * This call reads the mask (nmat ints) and the info block on the host. */
+int blu_batch_factorize_subset_dev(blu_batch_t *b, const int *d_run,
+                                   const int64_t *d_b_begin, const int64_t *d_b_end, const int64_t *d_b_i, const double *d_b_x,
+                                   int64_t bnz_total, int *d_status);
+/* right-hand side of basis k: d_irhs/d_xrhs[d_rhs_begin[k] .. d_rhs_begin[k+1]) (nmat+1 offsets); outputs d_nzlhs[k],
+ * d_ilhs[k*m ..], d_xlhs[k*m + n], d_status[k] */
+int blu_batch_solve_for_update_dev(blu_batch_t *b, const int *d_run, const int64_t *d_rhs_begin,
+                                   const int64_t *d_irhs, const double *d_xrhs, int want_solution,
+                                   int64_t *d_nzlhs, int64_t *d_ilhs, double *d_xlhs, int *d_status, char trans);
+/* basis k with d_xtbl[k], status in d_status[k] */
+int blu_batch_update_dev(blu_batch_t *b, const int *d_run, const double *d_xtbl, int *d_status);
+/* blu_batch_solve_sparse with nunits given by the caller (checked against d_unit_begin[nmat] on the device) */
+int blu_batch_solve_sparse_dev(blu_batch_t *b, int64_t nunits, const int64_t *d_unit_begin,
+                               const int64_t *d_rhs_begin, const int64_t *d_irhs, const double *d_xrhs,
+                               int64_t *d_nzlhs, int64_t *d_ilhs, double *d_xlhs, int *d_status, char trans);
+int blu_batch_solve_dense_multi_dev(blu_batch_t *b, int64_t nrhs, const double *d_rhs, double *d_lhs,
+                                    char trans, int *d_status);
 /* The steady-state step of a resident batch (factorization launches + condest/residual_test + solve_dense of the
  * uploaded rhs) captured into a CUDA graph once, then replayed with one launch per step; a basis that answers
  * Reallocate during a replay is grown and re-run by the classic path before the call returns. */
