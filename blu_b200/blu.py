@@ -102,6 +102,8 @@ def load_library(path=None):
     L.blu_batch_update_dev.argtypes = [vp, vp, vp, vp]
     L.blu_batch_solve_sparse_dev.argtypes = [vp, ctypes.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.c_char]
     L.blu_batch_solve_dense_multi_dev.argtypes = [vp, ctypes.c_int64, vp, vp, ctypes.c_char, vp]
+    L.blu_batch_copy.argtypes = [vp, ctypes.c_int64, i64p, i64p]
+    L.blu_batch_copy_dev.argtypes = [vp, vp]
     L.blu_batch_graph_capture.argtypes = [vp, ctypes.c_char]
     L.blu_batch_graph_launch.argtypes = [vp]
     L.blu_batch_stream.argtypes = [vp]; L.blu_batch_stream.restype = vp
@@ -625,6 +627,22 @@ class BLUBatch(_Base):
         st = self._on_stream(dev, lambda: self._L.blu_batch_solve_dense_multi_dev(
             self._h, nrhs, self._ptr(r), self._ptr(x), _ch(trans), self._ptr(stat)))
         return st, x, stat
+
+    def copy(self, dst, src):
+        """Basis dst[r] becomes a copy of basis src[r] (factors, update history, a pending solve_for_update, getters,
+        store capacities and resident B): from then on it behaves as src[r] would.  Returns the status."""
+        d, s = _i64(dst).reshape(-1), _i64(src).reshape(-1)
+        if len(d) != len(s):
+            raise ValueError("dst and src differ in length")
+        return self._L.blu_batch_copy(self._h, len(d), _pi(d), _pi(s))
+
+    def copy_dev(self, from_):
+        """copy with the map in device memory: from_ is an int32 tensor of nmat entries on the batch's device,
+        from_[k] = -1 keeps basis k, otherwise basis k becomes a copy of basis from_[k].  Returns the status."""
+        import torch
+        dev = self._torch_device()
+        f = self._tensor(from_, torch.int32, self.nmat, "from_", dev)
+        return self._on_stream(dev, lambda: self._L.blu_batch_copy_dev(self._h, self._ptr(f)))
 
     def graph_capture(self, trans="N"):
         return self._L.blu_batch_graph_capture(self._h, _ch(trans))

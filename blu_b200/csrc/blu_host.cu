@@ -14,6 +14,7 @@
 #include "blu_maxvolume.cuh"
 #include "blu_subset.cuh"
 #include "blu_dev_calls.cuh"
+#include "blu_copy.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -2505,6 +2506,108 @@ extern "C" int blu_batch_solve_dense_multi_dev(blu_batch_t *o, int64_t nrhs, con
     o->info_dirty = 1;
     o->time_solve += wall_now() - tic;
     return dev_sum_first(o);
+}
+
+/* ------------------------------------------------------------------ */
+/* batch: copy bases within the batch (fork a basis into other slots)  */
+/* ------------------------------------------------------------------ */
+
+/* the pairs of a copy call: distinct destinations, no destination that is also a source, no self-copy */
+static int copy_check(blu_b200 *o, int64_t ncopy, const int64_t *dst, const int64_t *src) {
+    if (!o || o->single || ncopy < 0 || ncopy > o->d.nmat || (ncopy > 0 && (!dst || !src))) return BLU_ERROR_INVALID_ARGUMENT;
+    const int64_t n = o->d.nmat;
+    std::vector<char> isdst((size_t)n, 0), issrc((size_t)n, 0);
+    for (int64_t r = 0; r < ncopy; r++) {
+        if (dst[r] < 0 || dst[r] >= n || src[r] < 0 || src[r] >= n || dst[r] == src[r] || isdst[(size_t)dst[r]]) return BLU_ERROR_INVALID_ARGUMENT;
+        isdst[(size_t)dst[r]] = 1; issrc[(size_t)src[r]] = 1;
+    }
+    for (int64_t r = 0; r < ncopy; r++) if (issrc[(size_t)dst[r]]) return BLU_ERROR_INVALID_ARGUMENT;
+    return BLU_OK;
+}
+
+/* blu_batch_copy after copy_check: the destinations take the sources' store capacities (new private stores in one
+ * block, as grow_hungry_slots allocates them; the uniform store where the source has no private one), then one launch
+ * of k_copy_slots copies the state and the resident B rows. */
+static int copy_run(blu_b200 *o, int64_t ncopy, const int64_t *dst, const int64_t *src) {
+    if (ncopy == 0) return BLU_OK;
+    CK(cudaSetDevice(o->device));
+    BluDev &d = o->d;
+    const size_t n = (size_t)d.nmat, M = (size_t)d.m;
+    const cudaStream_t s = o->stream;
+    auto rnd = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    size_t bytes = 0;
+    for (int64_t r = 0; r < ncopy; r++) {
+        const BluSlotStore &e = o->hslot[(size_t)src[r]];
+        if (e.l_idx) bytes += rnd((size_t)(e.l_mem + PADDING) * 4) + rnd((size_t)(e.l_mem + PADDING) * 8);
+        if (e.u_idx) bytes += rnd((size_t)(e.u_mem + PADDING) * 4) + rnd((size_t)(e.u_mem + PADDING) * 8);
+        if (e.w_idx) bytes += rnd((size_t)(2 * e.w_mem + PADDING) * 4) + rnd((size_t)(2 * e.w_mem + PADDING) * 8);
+    }
+    MvCall c(o);
+    int *dpairs = nullptr;
+    int st = c.alloc(&dpairs, 2 * (size_t)ncopy);
+    if (st != BLU_OK) return st;
+    unsigned char *blk = nullptr;
+    if (bytes && (st = dalloc(o, &blk, bytes)) != BLU_OK) return st;
+    /* nothing has changed so far; from here on the call completes */
+    if (blk) o->ext_blocks.push_back(blk);
+    size_t off = 0;
+    auto take = [&](size_t b) { unsigned char *p = blk + off; off += rnd(b); return p; };
+    std::vector<int> pairs(2 * (size_t)ncopy);
+    for (int64_t r = 0; r < ncopy; r++) {
+        const BluSlotStore &e = o->hslot[(size_t)src[r]];
+        BluSlotStore f; memset(&f, 0, sizeof f);
+        if (e.l_idx) { f.l_idx = (int *)take((size_t)(e.l_mem + PADDING) * 4); f.l_val = (double *)take((size_t)(e.l_mem + PADDING) * 8); f.l_mem = e.l_mem; }
+        if (e.u_idx) { f.u_idx = (int *)take((size_t)(e.u_mem + PADDING) * 4); f.u_val = (double *)take((size_t)(e.u_mem + PADDING) * 8); f.u_mem = e.u_mem; }
+        if (e.w_idx) { f.w_idx = (int *)take((size_t)(2 * e.w_mem + PADDING) * 4); f.w_val = (double *)take((size_t)(2 * e.w_mem + PADDING) * 8); f.w_mem = e.w_mem; }
+        o->hslot[(size_t)dst[r]] = f;      /* (an old private block of dst is reclaimed at the next whole-batch store change) */
+        pairs[2 * (size_t)r] = (int)dst[r]; pairs[2 * (size_t)r + 1] = (int)src[r];
+    }
+    o->have_overrides = 0;
+    for (const BluSlotStore &e : o->hslot) if (e.l_idx || e.u_idx || e.w_idx) o->have_overrides = 1;
+    CK(cudaMemcpyAsync(o->d_slot, o->hslot.data(), n * sizeof(BluSlotStore), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(dpairs, pairs.data(), pairs.size() * sizeof(int), cudaMemcpyHostToDevice, s));
+    /* caller-owned B: its column pointers move into the library-owned rows, which the copy then edits (b_i / b_x stay
+     * the caller's) */
+    if (o->b_external && d.b_begin != (const blu_i64 *)o->db_begin) {      /* (a later copy finds them moved already) */
+        CK(cudaMemcpyAsync(o->db_begin, d.b_begin, n * M * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
+        CK(cudaMemcpyAsync(o->db_end, d.b_end, n * M * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
+        d.b_begin = (const blu_i64 *)o->db_begin; d.b_end = (const blu_i64 *)o->db_end;
+    }
+    timer_start(o);
+    BLU_LAUNCH(k_copy_slots, (int)(ncopy * COPY_PARTS), COPY_THREADS, 0, s, d, (const int *)dpairs, (blu_i64 *)o->db_begin, (blu_i64 *)o->db_end);
+    o->launches++;
+    CK(cudaGetLastError());
+    timer_stop(o, 0);      /* (synchronizes: the pageable sources above are read) */
+    for (int64_t r = 0; r < ncopy; r++) o->hinfo[(size_t)dst[r]] = o->hinfo[(size_t)src[r]];
+#ifndef BLU_EMU
+    if (o->have_graph) { cudaGraphExecDestroy(o->graph_exec); cudaGraphDestroy(o->graph); }
+#endif
+    o->have_graph = 0;
+    return BLU_OK;
+}
+
+extern "C" int blu_batch_copy(blu_batch_t *o, int64_t ncopy, const int64_t *dst, const int64_t *src) {
+    const int st = copy_check(o, ncopy, dst, src);
+    return st != BLU_OK ? st : copy_run(o, ncopy, dst, src);
+}
+
+/* d_from[k] = -1 keeps basis k, otherwise basis k becomes a copy of basis d_from[k]; the map is read on the host */
+extern "C" int blu_batch_copy_dev(blu_batch_t *o, const int *d_from) {
+    if (!o || o->single || !d_from) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(o->device));
+    const int n = o->d.nmat;
+    std::vector<int> from((size_t)n);
+    CK(cudaMemcpyAsync(from.data(), d_from, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
+    CK(cudaStreamSynchronize(o->stream));
+    std::vector<int64_t> dst, src;
+    for (int k = 0; k < n; k++) {
+        if (from[(size_t)k] == -1) continue;
+        if (from[(size_t)k] < 0) return BLU_ERROR_INVALID_ARGUMENT;      /* (>= nmat, self and chains: copy_check) */
+        dst.push_back(k); src.push_back(from[(size_t)k]);
+    }
+    const int64_t ncopy = (int64_t)dst.size();
+    const int st = copy_check(o, ncopy, dst.data(), src.data());
+    return st != BLU_OK ? st : copy_run(o, ncopy, dst.data(), src.data());
 }
 
 /* ------------------------------------------------------------------ */

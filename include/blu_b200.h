@@ -281,6 +281,34 @@ int blu_batch_solve_sparse_dev(blu_batch_t *b, int64_t nunits, const int64_t *d_
                                int64_t *d_nzlhs, int64_t *d_ilhs, double *d_xlhs, int *d_status, char trans);
 int blu_batch_solve_dense_multi_dev(blu_batch_t *b, int64_t nrhs, const double *d_rhs, double *d_lhs,
                                     char trans, int *d_status);
+
+/* Copy bases within a batch (Clone of a BLU, for branch-and-bound and strong-branching drivers that start child LPs
+ * from a parent's basis).  Basis dst[r] becomes a copy of basis src[r], for r < ncopy: factors, update history (etas,
+ * nforrest, nupdate, ...), a pending solve_for_update of either direction, every per-basis getter, the resident B, and
+ * the capacities of its L/U/W stores.  From then on dst[r] behaves, bit for bit, as src[r] would under the same calls
+ * (and as a BLU object that went through src[r]'s history).  Sources and all bases not named in dst do not move.
+ * - Capacities: a destination takes its source's L, U and W capacities exactly -- a private store of the same size
+ *   where the source has one (all new private stores of a call in one block), the uniform store otherwise.  So the
+ *   copy's later Reallocates and garbage collections happen exactly where the source's would.  A private store a
+ *   destination held before is reclaimed at the next whole-batch store change, as the store of a re-grown basis is.
+ * - Only the live part of each store is copied: L up to the end of the row-eta file, U up to u_begin[m] (plus a pending
+ *   spike), the live half of W up to its fill pointer, the row-wise B up to its last entry; and the O(m) state arrays.
+ * - The resident B: the destination's column pointers become the source's (offsets into the one b_i / b_x of the batch,
+ *   also when B is caller-owned after blu_batch_factorize_dev or after maxvolume), so blu_batch_factorize_resident
+ *   refactorizes the destination from the source's B, and a later blu_batch_factorize_subset keeps it.
+ * - A source that was never factorized is copied as it is: the copy is never factorized either (nupdate None).
+ * - ncopy < 0 or > nmat, an index outside [0, nmat), a repeated dst, dst[r] == src[r], a dst that is also a src of
+ *   the same call (no chains, so the result never depends on order), a missing array when ncopy > 0, or an object from
+ *   blu_create: BLU_ERROR_INVALID_ARGUMENT, nothing changes.  One src may appear many times (fan-out).  ncopy == 0:
+ *   BLU_OK, nothing changes.
+ * - A captured graph is dropped; blu_batch_graph_launch answers BLU_ERROR_INVALID_CALL until the next capture.
+ * - The copy queues on the batch's stream (blu_batch_set_stream applies), is complete when the call returns, and is
+ *   one launch in blu_batch_launch_count. */
+int blu_batch_copy(blu_batch_t *b, int64_t ncopy, const int64_t *dst, const int64_t *src);
+/* d_from: nmat ints on the device; d_from[k] = -1 keeps basis k, otherwise basis k becomes a copy of d_from[k].  The
+ * map is read on the host (nmat ints) and checked as blu_batch_copy checks its pairs (any other negative value is
+ * rejected as well); then the call is blu_batch_copy with the pairs in index order. */
+int blu_batch_copy_dev(blu_batch_t *b, const int *d_from);
 /* The steady-state step of a resident batch (factorization launches + condest/residual_test + solve_dense of the
  * uploaded rhs) captured into a CUDA graph once, then replayed with one launch per step; a basis that answers
  * Reallocate during a replay is grown and re-run by the classic path before the call returns. */
