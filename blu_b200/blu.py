@@ -104,6 +104,10 @@ def load_library(path=None):
     L.blu_batch_solve_dense_multi_dev.argtypes = [vp, ctypes.c_int64, vp, vp, ctypes.c_char, vp]
     L.blu_batch_copy.argtypes = [vp, ctypes.c_int64, i64p, i64p]
     L.blu_batch_copy_dev.argtypes = [vp, vp]
+    for f in ("blu_batch_save", "blu_batch_save_dev"):
+        getattr(L, f).argtypes = [vp, ctypes.c_int64, i64p, ctypes.POINTER(vp), i64p, i64p]
+    for f in ("blu_batch_restore", "blu_batch_restore_dev"):
+        getattr(L, f).argtypes = [vp, ctypes.c_int64, i64p, ctypes.POINTER(vp), i64p]
     L.blu_batch_graph_capture.argtypes = [vp, ctypes.c_char]
     L.blu_batch_graph_launch.argtypes = [vp]
     L.blu_batch_stream.argtypes = [vp]; L.blu_batch_stream.restype = vp
@@ -643,6 +647,90 @@ class BLUBatch(_Base):
         dev = self._torch_device()
         f = self._tensor(from_, torch.int32, self.nmat, "from_", dev)
         return self._on_stream(dev, lambda: self._L.blu_batch_copy_dev(self._h, self._ptr(f)))
+
+    # Images (blu_batch_save / blu_batch_restore): a basis' factorization and update history as bytes the caller owns,
+    # restorable into any slot of any batch of the same m.
+
+    def _save(self, fn, idx, bufs):
+        """one save call; bufs = None: the size query.  Returns (status, sizes)."""
+        s = _i64(idx).reshape(-1)
+        n = len(s)
+        nbytes = np.zeros(n, np.int64)
+        if bufs is None:
+            return fn(self._h, n, _pi(s), None, None, _pi(nbytes)), nbytes
+        ptrs = (ctypes.c_void_p * max(n, 1))(*[b[0] for b in bufs])
+        cap = _i64([b[1] for b in bufs])
+        return fn(self._h, n, _pi(s), ptrs, _pi(cap), _pi(nbytes)), nbytes
+
+    @staticmethod
+    def _aligned_host(nbytes):
+        """a numpy.uint8 array of nbytes whose data starts 16-byte aligned"""
+        raw = np.zeros(int(nbytes) + 16, np.uint8)
+        k = (-raw.ctypes.data) % 16
+        return raw[k:k + int(nbytes)]
+
+    def save(self, idx):
+        """The images of bases idx (repeats allowed) as a list of numpy.uint8 arrays.  Raises on a failed call."""
+        L = self._L.blu_batch_save
+        st, nbytes = self._save(L, idx, None)
+        if st != 0:
+            raise ValueError(f"blu_batch_save: status {st}")
+        out = [self._aligned_host(b) for b in nbytes]
+        st, _ = self._save(L, idx, [(a.ctypes.data, a.size) for a in out])
+        if st != 0:
+            raise ValueError(f"blu_batch_save: status {st}")
+        return out
+
+    def restore(self, dst, images):
+        """Basis dst[r] becomes the basis saved in images[r] (a buffer of bytes: numpy.uint8 arrays, bytes, ...).
+        Returns the status."""
+        d = _i64(dst).reshape(-1)
+        if len(d) != len(images):
+            raise ValueError("dst and images differ in length")
+        bufs = []
+        for im in images:
+            a = np.frombuffer(im, np.uint8) if not isinstance(im, np.ndarray) else np.ascontiguousarray(im).view(np.uint8).reshape(-1)
+            if a.ctypes.data % 16:
+                b = self._aligned_host(a.size)
+                b[:] = a
+                a = b
+            bufs.append(a)
+        ptrs = (ctypes.c_void_p * max(len(d), 1))(*[a.ctypes.data for a in bufs])
+        cap = _i64([a.size for a in bufs])
+        return self._L.blu_batch_restore(self._h, len(d), _pi(d), ptrs, _pi(cap))
+
+    def save_dev(self, idx):
+        """The images of bases idx as a list of 1-D torch.uint8 tensors on the batch's device: views into one
+        allocation, each starting 256-byte aligned.  Ordered after torch's current stream.  Raises on a failed call."""
+        import torch
+        dev = self._torch_device()
+        L = self._L.blu_batch_save_dev
+        st, nbytes = self._on_stream(dev, lambda: self._save(L, idx, None))
+        if st != 0:
+            raise ValueError(f"blu_batch_save_dev: status {st}")
+        size = [(int(b) + 255) & ~255 for b in nbytes]
+        block = torch.empty(sum(size) + 256, dtype=torch.uint8, device=dev)
+        at = (-block.data_ptr()) % 256
+        out = []
+        for b, z in zip(nbytes, size):
+            out.append(block[at:at + int(b)])
+            at += z
+        st, _ = self._on_stream(dev, lambda: self._save(L, idx, [(t.data_ptr(), t.numel()) for t in out]))
+        if st != 0:
+            raise ValueError(f"blu_batch_save_dev: status {st}")
+        return out
+
+    def restore_dev(self, dst, images):
+        """restore from contiguous torch.uint8 tensors on the batch's device.  Returns the status."""
+        import torch
+        dev = self._torch_device()
+        d = _i64(dst).reshape(-1)
+        if len(d) != len(images):
+            raise ValueError("dst and images differ in length")
+        ts = [self._tensor(t, torch.uint8, None, f"images[{r}]", dev) for r, t in enumerate(images)]
+        ptrs = (ctypes.c_void_p * max(len(d), 1))(*[t.data_ptr() for t in ts])
+        cap = _i64([t.numel() for t in ts])
+        return self._on_stream(dev, lambda: self._L.blu_batch_restore_dev(self._h, len(d), _pi(d), ptrs, _pi(cap)))
 
     def graph_capture(self, trans="N"):
         return self._L.blu_batch_graph_capture(self._h, _ch(trans))

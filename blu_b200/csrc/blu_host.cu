@@ -15,6 +15,7 @@
 #include "blu_subset.cuh"
 #include "blu_dev_calls.cuh"
 #include "blu_copy.cuh"
+#include "blu_save.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -2063,6 +2064,15 @@ static int dev_finish(blu_b200 *o, int n, int64_t idx0, const int *run, const in
     return BLU_OK;
 }
 
+/* the B the bases were last factorized from (all-empty columns before the first factorization): column j of basis k is
+ * i / x[b[k * m + j] : e[k * m + j]], entries [0, total) */
+struct ResidentB { const blu_i64 *b, *e, *i; const double *x; blu_i64 total; };
+static ResidentB resident_b(const blu_b200 *o) {
+    const BluDev &d = o->d;
+    if (o->b_external) return ResidentB{d.b_begin, d.b_end, d.b_i, d.b_x, o->have_b ? d.b_total : 0};
+    return ResidentB{(const blu_i64 *)o->db_begin, (const blu_i64 *)o->db_end, (const blu_i64 *)o->db_i, o->db_x, o->have_b ? d.b_total : 0};
+}
+
 /* The resident B becomes, for every basis, the B it was last factorized from: the new columns of the slots with
  * pos[k] >= 0 (column j of slot k at nb/ne[pos[k]*m + j], entries in ni/nx, all in device memory), the others' old
  * ones, compacted into fresh library-owned buffers that replace the old ones.  *maxnz: the most entries of one new B.
@@ -2073,11 +2083,10 @@ static int rebuild_b(blu_b200 *o, MvCall &c, const int *dpos, const std::vector<
     BluDev &d = o->d;
     const size_t n = (size_t)d.nmat, M = (size_t)d.m;
     const cudaStream_t s = o->stream;
-    /* the B the bases were last factorized from (all-empty columns before the first factorization) */
-    const blu_i64 *ob = o->b_external ? d.b_begin : (const blu_i64 *)o->db_begin, *oe = o->b_external ? d.b_end : (const blu_i64 *)o->db_end;
-    const blu_i64 *oi = o->b_external ? d.b_i : (const blu_i64 *)o->db_i;
-    const double *ox = o->b_external ? d.b_x : o->db_x;
-    const blu_i64 ototal = o->have_b ? d.b_total : 0;
+    const ResidentB B = resident_b(o);
+    const blu_i64 *ob = B.b, *oe = B.e, *oi = B.i;
+    const double *ox = B.x;
+    const blu_i64 ototal = B.total;
     blu_i64 *tot = nullptr, *soff = nullptr;
     int st = c.alloc(&tot, n);
     if (st == BLU_OK) st = c.alloc(&soff, n);
@@ -2608,6 +2617,263 @@ extern "C" int blu_batch_copy_dev(blu_batch_t *o, const int *d_from) {
     const int64_t ncopy = (int64_t)dst.size();
     const int st = copy_check(o, ncopy, dst.data(), src.data());
     return st != BLU_OK ? st : copy_run(o, ncopy, dst.data(), src.data());
+}
+
+/* ------------------------------------------------------------------ */
+/* batch: save bases to images and restore them into any slot          */
+/* ------------------------------------------------------------------ */
+
+/* device scratch of the host variants: the images pass through it in chunks of at most this many bytes (or one image) */
+#define IMG_SCRATCH ((size_t)1 << 30)
+
+static bool img_aligned(const void *p) { return p && ((size_t)p & 15) == 0; }
+
+/* the arguments of a save: idx in [0, nmat) (repeats allowed); buf (when given) with a 16-byte aligned pointer and a
+ * capacity for every image */
+static int save_check(blu_b200 *o, int64_t n, const int64_t *idx, void *const *buf, const int64_t *cap, int64_t *bytes) {
+    if (!o || o->single || n < 0 || (n > 0 && (!idx || !bytes)) || (n > 0 && buf && !cap)) return BLU_ERROR_INVALID_ARGUMENT;
+    for (int64_t r = 0; r < n; r++) {
+        if (idx[r] < 0 || idx[r] >= o->d.nmat) return BLU_ERROR_INVALID_ARGUMENT;
+        if (buf && !img_aligned(buf[r])) return BLU_ERROR_INVALID_ARGUMENT;
+    }
+    return BLU_OK;
+}
+
+/* the headers of the images of bases idx (on the device, checksum 0) and their sizes (bytes, on the host) */
+static int save_extents(blu_b200 *o, MvCall &c, int64_t n, const int64_t *idx, int **didx, BluImage **dhdr, int64_t *bytes) {
+    const cudaStream_t s = o->stream;
+    blu_i64 *dbytes = nullptr;
+    int st = c.alloc(didx, (size_t)n);
+    if (st == BLU_OK) st = c.alloc(dhdr, (size_t)n);
+    if (st == BLU_OK) st = c.alloc(&dbytes, (size_t)n);
+    if (st != BLU_OK) return st;
+    std::vector<int> hidx(idx, idx + n);
+    CK(cudaMemcpyAsync(*didx, hidx.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, s));
+    const ResidentB B = resident_b(o);
+    BLU_LAUNCH(k_save_extents, (int)n, 32, 0, s, o->d, (const int *)*didx, B.b, B.e, B.total, *dhdr, dbytes);
+    o->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(bytes, dbytes, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return BLU_OK;
+}
+
+/* the images of bases didx into the device buffers dimg (n pointers, on the device), checksums included */
+static int save_write(blu_b200 *o, MvCall &c, int64_t n, const int *didx, const BluImage *dhdr, unsigned char *const *dimg) {
+    const cudaStream_t s = o->stream;
+    blu_u64 *part = nullptr;
+    int st = c.alloc(&part, (size_t)n * SAVE_PARTS);
+    if (st != BLU_OK) return st;
+    const ResidentB B = resident_b(o);
+    BLU_LAUNCH(k_save_slots, (int)(n * SAVE_PARTS), SAVE_THREADS, 0, s, o->d, didx, dhdr, dimg, B.b, B.e, B.i, B.x, B.total, part);
+    o->launches++;
+    CK(cudaGetLastError());
+    BLU_LAUNCH(k_save_sum, grid_of(n, 256), 256, 0, s, (int)n, (const blu_u64 *)part, dimg);
+    o->launches++;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(s));
+    return BLU_OK;
+}
+
+extern "C" int blu_batch_save_dev(blu_batch_t *o, int64_t n, const int64_t *idx, void *const *d_buf, const int64_t *cap, int64_t *bytes) {
+    int st = save_check(o, n, idx, d_buf, cap, bytes);
+    if (st != BLU_OK || n == 0) return st;
+    CK(cudaSetDevice(o->device));
+    MvCall c(o);
+    int *didx = nullptr; BluImage *dhdr = nullptr;
+    if ((st = save_extents(o, c, n, idx, &didx, &dhdr, bytes)) != BLU_OK || !d_buf) return st;
+    for (int64_t r = 0; r < n; r++) if (cap[r] < bytes[r]) return BLU_ERROR_INVALID_ARGUMENT;
+    unsigned char **dimg = nullptr;
+    if ((st = c.alloc(&dimg, (size_t)n)) != BLU_OK) return st;
+    CK(cudaMemcpyAsync(dimg, d_buf, (size_t)n * sizeof(void *), cudaMemcpyHostToDevice, o->stream));
+    return save_write(o, c, n, didx, dhdr, dimg);
+}
+
+/* the 256-byte rounded bytes of the images [r0, r1) that go through the scratch together, starting at r0 */
+static int64_t img_chunk_end(int64_t r0, int64_t n, const std::vector<size_t> &sz, size_t scratch) {
+    size_t put = sz[(size_t)r0];
+    int64_t r1 = r0 + 1;
+    while (r1 < n && put + sz[(size_t)r1] <= scratch) put += sz[(size_t)r1++];
+    return r1;
+}
+static size_t img_scratch(const std::vector<size_t> &sz) {
+    size_t tot = 0, big = 0;
+    for (size_t b : sz) { tot += b; big = std::max(big, b); }
+    return std::min(tot, std::max(IMG_SCRATCH, big));
+}
+
+extern "C" int blu_batch_save(blu_batch_t *o, int64_t n, const int64_t *idx, void *const *buf, const int64_t *cap, int64_t *bytes) {
+    int st = save_check(o, n, idx, buf, cap, bytes);
+    if (st != BLU_OK || n == 0) return st;
+    CK(cudaSetDevice(o->device));
+    const cudaStream_t s = o->stream;
+    MvCall c(o);
+    int *didx = nullptr; BluImage *dhdr = nullptr;
+    if ((st = save_extents(o, c, n, idx, &didx, &dhdr, bytes)) != BLU_OK || !buf) return st;
+    for (int64_t r = 0; r < n; r++) if (cap[r] < bytes[r]) return BLU_ERROR_INVALID_ARGUMENT;
+    std::vector<size_t> sz((size_t)n);
+    for (int64_t r = 0; r < n; r++) sz[(size_t)r] = ((size_t)bytes[r] + 255) & ~(size_t)255;
+    const size_t scratch = img_scratch(sz);
+    unsigned char *scr = nullptr, **dimg = nullptr;
+    if ((st = c.alloc(&scr, scratch)) != BLU_OK || (st = c.alloc(&dimg, (size_t)n)) != BLU_OK) return st;
+    std::vector<unsigned char *> hp((size_t)n);
+    for (int64_t r0 = 0, r1; r0 < n; r0 = r1) {
+        r1 = img_chunk_end(r0, n, sz, scratch);
+        for (int64_t r = r0, off = 0; r < r1; off += (int64_t)sz[(size_t)r], r++) hp[(size_t)r] = scr + off;
+        CK(cudaMemcpyAsync(dimg + r0, hp.data() + r0, (size_t)(r1 - r0) * sizeof(void *), cudaMemcpyHostToDevice, s));
+        if ((st = save_write(o, c, r1 - r0, didx + r0, dhdr + r0, dimg + r0)) != BLU_OK) return st;
+        for (int64_t r = r0; r < r1; r++) CK(cudaMemcpyAsync(buf[r], hp[(size_t)r], (size_t)bytes[r], cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    return BLU_OK;
+}
+
+/* the arguments of a restore: n distinct destinations in [0, nmat), every buffer 16-byte aligned and holding a header */
+static int restore_check(blu_b200 *o, int64_t n, const int64_t *dst, const void *const *buf, const int64_t *cap) {
+    if (!o || o->single || n < 0 || n > o->d.nmat || (n > 0 && (!dst || !buf || !cap))) return BLU_ERROR_INVALID_ARGUMENT;
+    std::vector<char> seen((size_t)o->d.nmat, 0);
+    for (int64_t r = 0; r < n; r++) {
+        if (dst[r] < 0 || dst[r] >= o->d.nmat || seen[(size_t)dst[r]]) return BLU_ERROR_INVALID_ARGUMENT;
+        seen[(size_t)dst[r]] = 1;
+        if (!img_aligned(buf[r]) || cap[r] < (int64_t)sizeof(BluImage)) return BLU_ERROR_INVALID_ARGUMENT;
+    }
+    return BLU_OK;
+}
+
+/* a header this build can restore into a batch of dimension m from a buffer of cap bytes: its length is the one its
+ * extents give, every extent within its capacity */
+static bool img_header_ok(const BluImage &h, int m, int64_t cap) {
+    if (h.magic != IMG_MAGIC || h.version != IMG_VERSION || h.m != m || h.info_bytes != (int)sizeof(BluInfo)) return false;
+    if (h.length < (int64_t)sizeof(BluImage) || h.length > cap || (h.length & 15)) return false;
+    if (h.l_mem < 1 || h.l_mem > 0x3fffffff || h.u_mem < 1 || h.u_mem > 0x3fffffff || h.w_mem < 1 || h.w_mem > 0x1fffffff) return false;
+    if (h.l_n < 0 || h.l_n > h.l_mem || h.u_n < 0 || h.u_n > h.u_mem || h.w_n < 0 || h.w_n > h.w_mem) return false;
+    if (h.bt_n < 0 || h.bt_n > 0x3fffffff || h.b_nz < 0 || h.b_nz > cap / 16) return false;
+    return img_offset(h, IMG_NSEC) == h.length;
+}
+
+/* The images at the device pointers dimg (host array): their headers come up and are checked, then (verify) their
+ * checksums on the device; nothing has changed when either fails.  commit: basis dst[r] becomes the basis of image r. */
+static int restore_images(blu_b200 *o, MvCall &c, int64_t n, const int64_t *dst, const unsigned char *const *dimg_h, const int64_t *cap,
+                          bool verify, bool commit) {
+    BluDev &d = o->d;
+    const cudaStream_t s = o->stream;
+    const size_t N = (size_t)d.nmat, M = (size_t)d.m;
+    unsigned char **dimg = nullptr; BluImage *dhdr = nullptr;
+    int st = c.alloc(&dimg, (size_t)n);
+    if (st == BLU_OK) st = c.alloc(&dhdr, (size_t)n);
+    if (st != BLU_OK) return st;
+    CK(cudaMemcpyAsync(dimg, dimg_h, (size_t)n * sizeof(void *), cudaMemcpyHostToDevice, s));
+    BLU_LAUNCH(k_img_headers, (int)n, SAVE_THREADS, 0, s, (const unsigned char *const *)dimg, dhdr);
+    o->launches++;
+    CK(cudaGetLastError());
+    std::vector<BluImage> h((size_t)n);
+    CK(cudaMemcpyAsync(h.data(), dhdr, (size_t)n * sizeof(BluImage), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    for (int64_t r = 0; r < n; r++) if (!img_header_ok(h[(size_t)r], d.m, cap[r])) return BLU_ERROR_INVALID_ARGUMENT;
+    if (verify) {
+        blu_u64 *part = nullptr;
+        if ((st = c.alloc(&part, (size_t)n * SAVE_PARTS)) != BLU_OK || (st = dev_sum_ensure(o)) != BLU_OK) return st;
+        BLU_LAUNCH(k_img_sum, (int)(n * SAVE_PARTS), SAVE_THREADS, 0, s, (const unsigned char *const *)dimg, (const BluImage *)dhdr, part);
+        o->launches++;
+        CK(cudaGetLastError());
+        st = dev_validate(o, [&]() { BLU_LAUNCH(k_img_verdict, grid_of(n, 256), 256, 0, s, (int)n, (const blu_u64 *)part, (const BluImage *)dhdr, o->d_sum); });
+        if (st != BLU_OK) return st;
+    }
+    if (!commit) return BLU_OK;
+    /* the row-wise B's room, the destinations' private stores, the images' resident B staged for rebuild_b */
+    auto rnd = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    int64_t btmax = 0, btot = 0;
+    size_t bytes = 0;
+    std::vector<int64_t> base((size_t)n);
+    std::vector<int> pos(N, -1), hdst((size_t)n);
+    for (int64_t r = 0; r < n; r++) {
+        const BluImage &e = h[(size_t)r];
+        btmax = std::max<int64_t>(btmax, e.bt_n);
+        base[(size_t)r] = btot; btot += e.b_nz;
+        if (e.l_mem != d.l_mem) bytes += rnd((size_t)(e.l_mem + PADDING) * 4) + rnd((size_t)(e.l_mem + PADDING) * 8);
+        if (e.u_mem != d.u_mem) bytes += rnd((size_t)(e.u_mem + PADDING) * 4) + rnd((size_t)(e.u_mem + PADDING) * 8);
+        if (e.w_mem != d.w_mem) bytes += rnd((size_t)(2 * e.w_mem + PADDING) * 4) + rnd((size_t)(2 * e.w_mem + PADDING) * 8);
+        pos[(size_t)dst[r]] = (int)r; hdst[(size_t)r] = (int)dst[r];
+    }
+    if ((st = mv_ensure_bt_cap(o, btmax)) != BLU_OK) return st;
+    blu_i64 *nb = nullptr, *ne = nullptr, *ni = nullptr, *dbase = nullptr; double *nx = nullptr; int *dpos = nullptr, *ddst = nullptr;
+    if ((st = c.alloc(&nb, (size_t)n * M)) != BLU_OK || (st = c.alloc(&ne, (size_t)n * M)) != BLU_OK ||
+        (st = c.alloc(&ni, (size_t)btot)) != BLU_OK || (st = c.alloc(&nx, (size_t)btot)) != BLU_OK ||
+        (st = c.alloc(&dbase, (size_t)n)) != BLU_OK || (st = c.alloc(&dpos, N)) != BLU_OK || (st = c.alloc(&ddst, (size_t)n)) != BLU_OK)
+        return st;
+    CK(cudaMemcpyAsync(dbase, base.data(), (size_t)n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(dpos, pos.data(), N * sizeof(int), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ddst, hdst.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, s));
+    BLU_LAUNCH(k_img_stage_b, (int)n, SAVE_THREADS, 0, s, d.m, (const unsigned char *const *)dimg, (const BluImage *)dhdr,
+               (const blu_i64 *)dbase, nb, ne, ni, nx);
+    o->launches++;
+    CK(cudaGetLastError());
+    unsigned char *blk = nullptr;
+    if (bytes && (st = dalloc(o, &blk, bytes)) != BLU_OK) return st;
+    int64_t maxnz = 0;
+    if ((st = rebuild_b(o, c, dpos, nullptr, nb, ne, ni, nx, &maxnz)) != BLU_OK) { dfree(o, blk); return st; }
+    /* the resident B is the new one (a captured graph is dropped); from here on the call completes */
+    if (blk) o->ext_blocks.push_back(blk);
+    size_t off = 0;
+    auto take = [&](size_t b) { unsigned char *p = blk + off; off += rnd(b); return p; };
+    for (int64_t r = 0; r < n; r++) {
+        const BluImage &e = h[(size_t)r];
+        BluSlotStore f; memset(&f, 0, sizeof f);
+        if (e.l_mem != d.l_mem) { f.l_idx = (int *)take((size_t)(e.l_mem + PADDING) * 4); f.l_val = (double *)take((size_t)(e.l_mem + PADDING) * 8); f.l_mem = e.l_mem; }
+        if (e.u_mem != d.u_mem) { f.u_idx = (int *)take((size_t)(e.u_mem + PADDING) * 4); f.u_val = (double *)take((size_t)(e.u_mem + PADDING) * 8); f.u_mem = e.u_mem; }
+        if (e.w_mem != d.w_mem) { f.w_idx = (int *)take((size_t)(2 * e.w_mem + PADDING) * 4); f.w_val = (double *)take((size_t)(2 * e.w_mem + PADDING) * 8); f.w_mem = e.w_mem; }
+        o->hslot[(size_t)dst[r]] = f;      /* (an old private block of dst is reclaimed at the next whole-batch store change) */
+    }
+    o->have_overrides = 0;
+    for (const BluSlotStore &e : o->hslot) if (e.l_idx || e.u_idx || e.w_idx) o->have_overrides = 1;
+    CK(cudaMemcpyAsync(o->d_slot, o->hslot.data(), N * sizeof(BluSlotStore), cudaMemcpyHostToDevice, s));
+    BLU_LAUNCH(k_restore_slots, (int)(n * SAVE_PARTS), SAVE_THREADS, 0, s, d, (const int *)ddst, (const BluImage *)dhdr, (const unsigned char *const *)dimg);
+    o->launches++;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(s));      /* (pageable sources above) */
+    for (int64_t r = 0; r < n; r++) o->hinfo[(size_t)dst[r]] = h[(size_t)r].info;
+    return BLU_OK;
+}
+
+extern "C" int blu_batch_restore_dev(blu_batch_t *o, int64_t n, const int64_t *dst, const void *const *d_buf, const int64_t *cap) {
+    const int st = restore_check(o, n, dst, d_buf, cap);
+    if (st != BLU_OK || n == 0) return st;
+    CK(cudaSetDevice(o->device));
+    MvCall c(o);
+    return restore_images(o, c, n, dst, (const unsigned char *const *)d_buf, cap, true, true);
+}
+
+/* Through the device scratch in chunks; with more than one chunk, every chunk is verified before the first is
+ * restored, so that a rejected image still changes nothing. */
+extern "C" int blu_batch_restore(blu_batch_t *o, int64_t n, const int64_t *dst, const void *const *buf, const int64_t *cap) {
+    int st = restore_check(o, n, dst, buf, cap);
+    if (st != BLU_OK || n == 0) return st;
+    std::vector<size_t> sz((size_t)n);
+    for (int64_t r = 0; r < n; r++) {
+        BluImage h;
+        memcpy(&h, buf[r], sizeof h);
+        if (!img_header_ok(h, o->d.m, cap[r])) return BLU_ERROR_INVALID_ARGUMENT;
+        sz[(size_t)r] = ((size_t)h.length + 255) & ~(size_t)255;
+    }
+    CK(cudaSetDevice(o->device));
+    const cudaStream_t s = o->stream;
+    MvCall c(o);
+    const size_t scratch = img_scratch(sz);
+    unsigned char *scr = nullptr;
+    if ((st = c.alloc(&scr, scratch)) != BLU_OK) return st;
+    const bool one = img_chunk_end(0, n, sz, scratch) == n;
+    std::vector<const unsigned char *> hp((size_t)n);
+    for (int pass = one ? 1 : 0; pass < 2; pass++) {
+        for (int64_t r0 = 0, r1; r0 < n; r0 = r1) {
+            r1 = img_chunk_end(r0, n, sz, scratch);
+            for (int64_t r = r0, off = 0; r < r1; off += (int64_t)sz[(size_t)r], r++) {
+                hp[(size_t)r] = scr + off;
+                CK(cudaMemcpyAsync(scr + off, buf[r], (size_t)((const BluImage *)buf[r])->length, cudaMemcpyHostToDevice, s));
+            }
+            if ((st = restore_images(o, c, r1 - r0, dst + r0, hp.data() + r0, cap + r0, one || pass == 0, pass == 1)) != BLU_OK) return st;
+        }
+    }
+    return BLU_OK;
 }
 
 /* ------------------------------------------------------------------ */

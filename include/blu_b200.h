@@ -309,6 +309,54 @@ int blu_batch_copy(blu_batch_t *b, int64_t ncopy, const int64_t *dst, const int6
  * map is read on the host (nmat ints) and checked as blu_batch_copy checks its pairs (any other negative value is
  * rejected as well); then the call is blu_batch_copy with the pairs in index order. */
 int blu_batch_copy_dev(blu_batch_t *b, const int *d_from);
+
+/* Save bases to images in caller memory and restore them into any slot of any batch of the same m (park more open nodes
+ * of a branch-and-bound or strong-branching driver than the batch has slots, move a basis to another batch or GPU,
+ * checkpoint a run, recreate a batch with more slots).  An image is a self-contained byte string: the factors, the
+ * update history, a pending solve_for_update of either direction, every per-basis getter and the status word, the
+ * L/U/W capacities, and the basis' resident B as entries (not as offsets into this batch's B).  It carries no
+ * parameters: the destination batch's apply from the restore on.  Images are meant for the same build of the library,
+ * in this process or written to disk and read back in another; there is no compatibility across versions.  Layout: a
+ * fixed-size header (magic word, format version, m, sizeof(BluInfo), total length, the three capacities, the section
+ * extents, the BluInfo, a 64-bit checksum of the whole image computed on the device), then the sections
+ * (blu_b200/csrc/blu_save.cuh).  Every buf[r] is 16-byte aligned.
+ *
+ * blu_batch_save: the image of basis idx[r] into buf[r] (cap[r] bytes), its size into bytes[r], for r < n.  idx may
+ * repeat.  buf == NULL: only bytes[] is written (a size query).  Save changes nothing: no state, no store, and a
+ * captured graph stays valid.
+ * - A cap[r] smaller than the image: BLU_ERROR_INVALID_ARGUMENT after bytes[] is written, and no image is written.
+ * - n < 0, an idx outside [0, nmat), a missing idx / bytes (n > 0) or cap (buf given), a buf[r] that is NULL or not
+ *   16-byte aligned, or an object from blu_create: BLU_ERROR_INVALID_ARGUMENT.
+ *
+ * blu_batch_restore: basis dst[r] becomes the basis saved in image buf[r] (cap[r] bytes readable), for r < n.
+ * - Same batch: restoring into slot d the image of basis s of the same batch leaves d exactly as blu_batch_copy(d <- s)
+ *   would, bit for bit, in every getter, solve, get_factors and later call.  Another batch (same m, same or another
+ *   device): the restored basis behaves as the saved one would under the same calls and the same parameters.
+ * - Capacities: the destination takes the image's L, U and W capacities exactly -- the uniform store where the
+ *   capacity equals the batch's uniform one, otherwise a private store of that size (all new private stores of a call
+ *   in one block; a destination's old private block is reclaimed at the next whole-batch store change, as after a
+ *   copy).  If the image's row-wise B needs more room than the batch's bnz_cap, that room grows first.
+ * - Resident B: the destination's becomes the image's columns (a column with a negative length stays negative; a
+ *   never-factorized basis has all-empty columns), with the whole resident B rebuilt in library-owned memory as
+ *   blu_batch_factorize_subset rebuilds it (a caller-owned B from blu_batch_factorize_dev moves into library memory).
+ *   blu_batch_factorize_resident then refactorizes the destination from the saved basis' B.  A captured graph is
+ *   dropped: blu_batch_graph_launch answers BLU_ERROR_INVALID_CALL until the next capture.
+ * - BLU_ERROR_INVALID_ARGUMENT, and nothing changes: a wrong magic word, version, m or sizeof(BluInfo); a length
+ *   greater than cap[r]; an extent outside its capacity; a checksum mismatch; a buf[r] that is NULL or not 16-byte
+ *   aligned; n < 0 or n > nmat; a dst outside [0, nmat) or a repeated dst; a missing array when n > 0; an object from
+ *   blu_create.  The same image may be restored into several slots (fan-out).  n == 0: BLU_OK, nothing changes.
+ * - The host variants move the images through device scratch in chunks of about 1 GB; a restore of more than one chunk
+ *   checks every image before it changes anything.
+ *
+ * Both calls queue on the batch's stream (blu_batch_set_stream applies), are complete on return, and are counted in
+ * blu_batch_launch_count. */
+int blu_batch_save(blu_batch_t *b, int64_t n, const int64_t *idx, void *const *buf, const int64_t *cap, int64_t *bytes);
+int blu_batch_restore(blu_batch_t *b, int64_t n, const int64_t *dst, const void *const *buf, const int64_t *cap);
+/* The same two calls with every buf[r] in device memory on the batch's device (idx, dst, cap, bytes and the pointer
+ * arrays stay on the host).  Host traffic: save reads the n image sizes back; restore reads the n fixed-size headers
+ * and a checksum verdict; nothing else whose size grows with the images crosses the bus. */
+int blu_batch_save_dev(blu_batch_t *b, int64_t n, const int64_t *idx, void *const *d_buf, const int64_t *cap, int64_t *bytes);
+int blu_batch_restore_dev(blu_batch_t *b, int64_t n, const int64_t *dst, const void *const *d_buf, const int64_t *cap);
 /* The steady-state step of a resident batch (factorization launches + condest/residual_test + solve_dense of the
  * uploaded rhs) captured into a CUDA graph once, then replayed with one launch per step; a basis that answers
  * Reallocate during a replay is grown and re-run by the classic path before the call returns. */
