@@ -1172,6 +1172,35 @@ static int grow_store_keep(blu_b200 *o, int which, int64_t addmem) {
     return BLU_OK;
 }
 
+/* the single object's answer to Reallocate: every store the last run asked more room for grows, content kept */
+static int grow_object_stores(blu_b200 *o) {
+    int st = fetch_info(o);
+    if (st != BLU_OK) return st;
+    const BluInfo &I = o->hinfo[0];
+    if (I.addmem_l > 0) st = grow_store_keep(o, 0, I.addmem_l);
+    if (st == BLU_OK && I.addmem_u > 0) st = grow_store_keep(o, 1, I.addmem_u);
+    if (st == BLU_OK && I.addmem_w > 0) st = grow_store_keep(o, 2, I.addmem_w);
+    return st;
+}
+
+/* The Reallocate loop of the basis-change calls (BLU::solve_for_update / update, blu.rs:268-291, 319-334):
+ * run(rerun, &asks) queues one run's launches (rerun: not the first run), reads back what the call reads and sets asks
+ * when a running basis still says Reallocate; grow(o) makes room before the next run.  At most 40 runs.  Returns run's
+ * error as it is, BLU_OK once no basis asks, and otherwise BLU_REALLOCATE with *grown (when given) the status of the
+ * last grow, BLU_OK when the 40th run still asks.  What a basis still asking means is the caller's policy. */
+template <typename Run> static int rerun_on_realloc(blu_b200 *o, int (*grow)(blu_b200 *), Run run, int *grown = nullptr) {
+    int gst = BLU_OK;
+    for (int attempt = 0; attempt < 40 && gst == BLU_OK; attempt++) {
+        bool asks = false;
+        const int st = run(attempt > 0, &asks);
+        if (st != BLU_OK) return st;
+        if (!asks) return BLU_OK;
+        if (attempt < 39) gst = grow(o);
+    }
+    if (grown) *grown = gst;
+    return BLU_REALLOCATE;
+}
+
 static double wall_now() {
     struct timespec ts;
     clock_gettime(CLOCK_MONOTONIC, &ts);
@@ -1198,8 +1227,8 @@ static int sparse_call(blu_b200 *o, int64_t nzrhs, const int64_t *irhs, const do
     }
     const int nrhs = (nzrhs < 0 || nzrhs > m) ? -1 : (int)nzrhs;
     const double *dx = (xrhs && !(for_update && tr)) ? o->d_xrhs : nullptr;
-    int status = BLU_ERROR_INTERNAL, nz = 0;
-    for (int attempt = 0; attempt < 40; attempt++) {
+    int status = BLU_OK, nz = 0, grown;
+    const int rs = rerun_on_realloc(o, grow_object_stores, [&](bool, bool *asks) -> int {
         BLU_LAUNCH(k_solve_sparse, 1, 32, 0, o->stream, o->d, nrhs, (const i64 *)o->d_irhs, dx, trans, for_update, want,
                    o->d_scal, (i64 *)o->d_ilhs, o->d_xout, SpMulti{0, 0, 0, nullptr, nullptr, nullptr, nullptr});
         o->launches++;
@@ -1208,17 +1237,13 @@ static int sparse_call(blu_b200 *o, int64_t nzrhs, const int64_t *irhs, const do
         CK(cudaStreamSynchronize(o->stream));
         status = o->h_scal[0]; nz = o->h_scal[1];
         o->info_dirty = 1;
-        if (status != BLU_REALLOCATE) break;
-        /* BLU::solve_for_update loops on Reallocate, blu.rs:268-291 */
-        int st = fetch_info(o);
-        if (st != BLU_OK) return st;
-        const BluInfo &I = o->hinfo[0];
-        if (I.addmem_l > 0) st = grow_store_keep(o, 0, I.addmem_l);
-        if (st == BLU_OK && I.addmem_u > 0) st = grow_store_keep(o, 1, I.addmem_u);
-        if (st == BLU_OK && I.addmem_w > 0) st = grow_store_keep(o, 2, I.addmem_w);
-        if (st != BLU_OK) return st;
-        status = BLU_ERROR_INTERNAL;
-    }
+        *asks = status == BLU_REALLOCATE;
+        return BLU_OK;
+    }, &grown);
+    /* a store that cannot grow: its error; still Reallocate after 40 runs: an internal error */
+    if (rs == BLU_REALLOCATE && grown != BLU_OK) return grown;
+    if (rs == BLU_REALLOCATE) status = BLU_ERROR_INTERNAL;
+    else if (rs != BLU_OK) return rs;
     if (status == BLU_OK && want) {
         if (nz > 0) {
             CK(cudaMemcpyAsync(o->h_ilhs, o->d_ilhs, (size_t)nz * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
@@ -1246,8 +1271,8 @@ extern "C" int blu_update(blu_t *o, double xtbl) {
     if (!o || !o->single) return BLU_ERROR_INVALID_ARGUMENT;
     CK(cudaSetDevice(o->device));
     const double tic = wall_now();
-    int status = BLU_ERROR_INTERNAL;
-    for (int attempt = 0; attempt < 40; attempt++) {
+    int status = BLU_OK, grown;
+    const int rs = rerun_on_realloc(o, grow_object_stores, [&](bool, bool *asks) -> int {
         BLU_LAUNCH(k_update, 1, 32, 0, o->stream, o->d, xtbl, o->d_scal, (const double *)nullptr, 0);
         o->launches++;
         CK(cudaGetLastError());
@@ -1255,17 +1280,12 @@ extern "C" int blu_update(blu_t *o, double xtbl) {
         CK(cudaStreamSynchronize(o->stream));
         status = o->h_scal[0];
         o->info_dirty = 1;
-        if (status != BLU_REALLOCATE) break;
-        /* BLU::update loops on Reallocate, blu.rs:319-334 */
-        int st = fetch_info(o);
-        if (st != BLU_OK) return st;
-        const BluInfo &I = o->hinfo[0];
-        if (I.addmem_l > 0) st = grow_store_keep(o, 0, I.addmem_l);
-        if (st == BLU_OK && I.addmem_u > 0) st = grow_store_keep(o, 1, I.addmem_u);
-        if (st == BLU_OK && I.addmem_w > 0) st = grow_store_keep(o, 2, I.addmem_w);
-        if (st != BLU_OK) return st;
-        status = BLU_ERROR_INTERNAL;
-    }
+        *asks = status == BLU_REALLOCATE;
+        return BLU_OK;
+    }, &grown);
+    if (rs == BLU_REALLOCATE && grown != BLU_OK) return grown;      /* as in sparse_call */
+    if (rs == BLU_REALLOCATE) status = BLU_ERROR_INTERNAL;
+    else if (rs != BLU_OK) return rs;
     o->time_update += wall_now() - tic;
     return status;
 }
@@ -1436,6 +1456,21 @@ static int ensure_batch_sparse(blu_b200 *o, int64_t tot) {
     return BLU_OK;
 }
 
+/* The caller's statuses of a host batch call, in result order: result r is the status word words[stride * k] of slot
+ * k = sel[r] (k = r without sel) and, with nzlhs, its nonzero count next to it (nzlhs[r] = -1 unless OK).  A Reallocate
+ * left over means a store could not grow.  Returns the first non-OK status. */
+static int tally_statuses(const int *words, int stride, int64_t nres, const int64_t *sel, int *status, int64_t *nzlhs) {
+    int worst = BLU_OK;
+    for (int64_t r = 0; r < nres; r++) {
+        const size_t w = (size_t)stride * (size_t)(sel ? sel[r] : r);
+        const int s = words[w] == BLU_REALLOCATE ? BLU_ERROR_OUT_OF_MEMORY : words[w];
+        if (status) status[r] = s;
+        if (nzlhs) nzlhs[r] = s == BLU_OK ? words[w + 1] : -1;
+        if (s != BLU_OK && worst == BLU_OK) worst = s;
+    }
+    return worst;
+}
+
 /* solve_for_update (blu.rs:257) on every basis of the batch, basis k with its own right-hand side
  * irhs/xrhs[rhs_begin[k] .. rhs_begin[k+1]) (for trans 't'/'T': one index, the column to leave; xrhs may be
  * NULL).  want_solution != 0: nzlhs[k], ilhs[k*m ..] and the values xlhs[k*m + n] as in
@@ -1455,35 +1490,25 @@ extern "C" int blu_batch_solve_for_update(blu_batch_t *o, const int64_t *rhs_beg
     CK(cudaMemcpyAsync(o->sm_irhs, irhs, (size_t)tot * sizeof(int64_t), cudaMemcpyHostToDevice, o->stream));
     if (xrhs) CK(cudaMemcpyAsync(o->sm_xrhs, xrhs, (size_t)tot * sizeof(double), cudaMemcpyHostToDevice, o->stream));
     std::vector<int> hs(2 * n);
-    for (int attempt = 0; attempt < 40; attempt++) {
-        SpMulti W{(int)n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)o->sm_begin};
+    st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
+        SpMulti W{(int)n, rerun, 1, nullptr, nullptr, nullptr, (const i64 *)o->sm_begin};
         BLU_LAUNCH(k_solve_sparse, (int)n, 32, 0, o->stream, o->d, 0, (const i64 *)o->sm_irhs, xrhs ? (const double *)o->sm_xrhs : (const double *)nullptr,
                    trans, 1, want_solution ? 1 : 0, o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
         o->launches++;
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(hs.data(), o->sm_scal, 2 * n * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
         CK(cudaStreamSynchronize(o->stream));
-        bool again = false;
-        for (size_t k = 0; k < n; k++) again = again || hs[2 * k] == BLU_REALLOCATE;
-        if (!again) break;
-        /* blu.rs:268-291: grow and run those bases again (the others keep their results) */
-        if (grow_batch_stores(o) != BLU_OK) break;      /* what still says Reallocate is reported as out of memory below */
-    }
+        for (size_t k = 0; k < n; k++) *asks = *asks || hs[2 * k] == BLU_REALLOCATE;
+        return BLU_OK;
+    });
+    if (st != BLU_OK && st != BLU_REALLOCATE) return st;      /* Reallocate left over: a store could not grow */
     if (want_solution) {
         CK(cudaMemcpyAsync(ilhs, o->sm_ilhs, n * m * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
         CK(cudaMemcpyAsync(xlhs, o->sm_xout, n * m * sizeof(double), cudaMemcpyDeviceToHost, o->stream));
     }
     CK(cudaStreamSynchronize(o->stream));
-    int worst = BLU_OK;
-    for (size_t k = 0; k < n; k++) {
-        int s = hs[2 * k];
-        if (s == BLU_REALLOCATE) s = BLU_ERROR_OUT_OF_MEMORY;
-        if (status) status[k] = s;
-        if (want_solution) nzlhs[k] = s == BLU_OK ? hs[2 * k + 1] : -1;
-        if (s != BLU_OK && worst == BLU_OK) worst = s;
-    }
     o->info_dirty = 1;
-    return worst;
+    return tally_statuses(hs.data(), 2, (int64_t)n, nullptr, status, want_solution ? nzlhs : nullptr);
 }
 
 /* update (blu.rs:319) on every basis of the batch, basis k with xtbl[k] */
@@ -1495,26 +1520,18 @@ extern "C" int blu_batch_update(blu_batch_t *o, const double *xtbl, int *status)
     if (st != BLU_OK) return st;
     CK(cudaMemcpyAsync(o->sm_dbls, xtbl, n * sizeof(double), cudaMemcpyHostToDevice, o->stream));
     std::vector<int> hs(n);
-    for (int attempt = 0; attempt < 40; attempt++) {
-        BLU_LAUNCH(k_update, (int)n, 32, 0, o->stream, o->d, 0.0, o->sm_scal, (const double *)o->sm_dbls, attempt > 0 ? 1 : 0);
+    st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
+        BLU_LAUNCH(k_update, (int)n, 32, 0, o->stream, o->d, 0.0, o->sm_scal, (const double *)o->sm_dbls, rerun ? 1 : 0);
         o->launches++;
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(hs.data(), o->sm_scal, n * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
         CK(cudaStreamSynchronize(o->stream));
-        bool again = false;
-        for (size_t k = 0; k < n; k++) again = again || hs[k] == BLU_REALLOCATE;
-        if (!again) break;
-        if (grow_batch_stores(o) != BLU_OK) break;      /* blu.rs:319-334 */
-    }
-    int worst = BLU_OK;
-    for (size_t k = 0; k < n; k++) {
-        int s = hs[k];
-        if (s == BLU_REALLOCATE) s = BLU_ERROR_OUT_OF_MEMORY;
-        if (status) status[k] = s;
-        if (s != BLU_OK && worst == BLU_OK) worst = s;
-    }
+        for (size_t k = 0; k < n; k++) *asks = *asks || hs[k] == BLU_REALLOCATE;
+        return BLU_OK;
+    });
+    if (st != BLU_OK && st != BLU_REALLOCATE) return st;      /* Reallocate left over: a store could not grow */
     o->info_dirty = 1;
-    return worst;
+    return tally_statuses(hs.data(), 1, (int64_t)n, nullptr, status, nullptr);
 }
 
 /* ------------------------------------------------------------------ */
@@ -1724,20 +1741,21 @@ extern "C" int blu_batch_solve_dense_multi(blu_batch_t *o, int64_t nrhs, const d
 /* batch: maxvolume on every basis at once (maxvolume.rs:64-224)       */
 /* ------------------------------------------------------------------ */
 
-/* device buffers and pinned words of one masked batch call (blu_batch_maxvolume, the subset calls); released on
- * every way out, and the run mask is taken off the batch again so that later launches run every slot */
-struct MvCall {
+/* The scope of one masked batch call (maxvolume, the subset, _dev, copy, save and restore calls): its device buffers
+ * and pinned words, released on every way out, and the run mask, taken off the batch again so that later launches run
+ * every slot. */
+struct MaskedCall {
     blu_b200 *o;
     std::vector<void *> mem;
     unsigned long long *h_cnt = nullptr;
     int *h_st = nullptr;
-    explicit MvCall(blu_b200 *b) : o(b) {}
+    explicit MaskedCall(blu_b200 *b) : o(b) {}
     template <typename T> int alloc(T **p, size_t n) {
         int st = dalloc(o, p, n);
         if (st == BLU_OK) mem.push_back(*p);
         return st;
     }
-    ~MvCall() {
+    ~MaskedCall() {
         cudaStreamSynchronize(o->stream);
         o->d.run = nullptr;
         o->hrun.clear();
@@ -1764,7 +1782,7 @@ static int mv_ensure_bt_cap(blu_b200 *o, int64_t maxnz) {
 /* the bases with run = 1 are factorized (B as written by k_mv_decide), Reallocate handled as blu.rs:95-118
  * (grow the bases that asked, run them again), then condest/residual_test; every basis whose factorization is
  * not OK stops.  maxnz: the most entries of one of those B. */
-static int mv_factorize(blu_b200 *o, MvCall &c, const MvDev &V, int64_t maxnz) {
+static int mv_factorize(blu_b200 *o, MaskedCall &c, const MvDev &V, int64_t maxnz) {
     BluDev &d = o->d;
     const int n = d.nmat, g = (n + 127) / 128;
     { int st = mv_ensure_bt_cap(o, maxnz); if (st != BLU_OK) return st; }
@@ -1795,7 +1813,7 @@ static int mv_factorize(blu_b200 *o, MvCall &c, const MvDev &V, int64_t maxnz) {
 
 /* statuses of the last masked launch (stride words apart) and the counters: does a basis ask for more memory?
  * (a masked-out slot keeps the word of an earlier launch, which is never Reallocate once that launch is done) */
-static int mv_any_realloc(blu_b200 *o, MvCall &c, const MvDev &V, const int *d_st, int stride, bool *any) {
+static int mv_any_realloc(blu_b200 *o, MaskedCall &c, const MvDev &V, const int *d_st, int stride, bool *any) {
     const size_t n = (size_t)o->d.nmat;
     CK(cudaMemcpyAsync(c.h_st, d_st, n * stride * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
     CK(cudaMemcpyAsync(c.h_cnt, V.cnt, MV_CNT_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, o->stream));
@@ -1828,7 +1846,7 @@ extern "C" int blu_batch_maxvolume(blu_batch_t *o, int64_t ncol, const int64_t *
         if (a_begin[q] < 0 || a_begin[q] > anz_total || a_end[q] < 0 || a_end[q] > anz_total) return reject();
     CK(cudaSetDevice(o->device));
     BluDev &d = o->d;
-    MvCall c(o);
+    MaskedCall c(o);
     int st = ensure_b_cap(o, std::max<int64_t>(anz_total, 1));      /* the pool lives where B does; never a null pointer */
     if (st == BLU_OK) st = ensure_batch_sparse(o, 0);
     MvDev V;
@@ -1903,52 +1921,50 @@ extern "C" int blu_batch_maxvolume(blu_batch_t *o, int64_t ncol, const int64_t *
 
     /* the next column: ~0 from k_mv_next means that no basis is running any more */
     auto next_col = [&]() { return (int64_t)std::min<unsigned long long>(c.h_cnt[MV_CNT_NEXT], (unsigned long long)ncol); };
+    /* a store that cannot grow, or a basis still asking after 40 runs, stops the pass */
+    auto rerun = [&](auto run) -> int {
+        int grown;
+        const int rs = rerun_on_realloc(o, grow_batch_stores, run, &grown);
+        return rs != BLU_REALLOCATE ? rs : grown != BLU_OK ? grown : BLU_ERROR_OUT_OF_MEMORY;
+    };
     auto pass = [&]() -> int {
         /* the first factorization, maxvolume.rs:92-95 */
         if ((st = decide_next(nullptr, 0)) != BLU_OK || (st = read_cnt()) != BLU_OK) return st;
         if ((st = mv_factorize(o, c, V, (int64_t)c.h_cnt[MV_CNT_MAXNZ])) != BLU_OK) return st;
         if ((st = next_after_factorize(0)) != BLU_OK) return st;
         for (int64_t j = next_col(); j < ncol; j = next_col()) {
-            bool again = false;
             /* B^{-1} a_j straight from the pool, maxvolume.rs:100-118 */
             BLU_LAUNCH(k_mv_setup, g, 128, 0, s, V, (blu_i64)j);
             o->launches++;
-            for (int attempt = 0;; attempt++) {
-                SpMulti W{n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)V.rhs_begin, (const i64 *)V.rhs_end};
+            st = rerun([&](bool again, bool *asks) -> int {
+                SpMulti W{n, again, 1, nullptr, nullptr, nullptr, (const i64 *)V.rhs_begin, (const i64 *)V.rhs_end};
                 BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, d, 0, (const i64 *)o->db_i, (const double *)o->db_x, 'N', 1, 1,
                            o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
                 o->launches++;
                 CK(cudaGetLastError());
-                if ((st = mv_any_realloc(o, c, V, o->sm_scal, 2, &again)) != BLU_OK) return st;
-                if (!again) break;
-                if (attempt == 39) return BLU_ERROR_OUT_OF_MEMORY;
-                if ((st = grow_batch_stores(o)) != BLU_OK) return st;      /* blu.rs:268-291 */
-            }
+                return mv_any_realloc(o, c, V, o->sm_scal, 2, asks);
+            });
+            if (st != BLU_OK) return st;
             BLU_LAUNCH(k_mv_select, n, 32, 0, s, V, (blu_i64)j, (const int *)o->sm_scal, (const blu_i64 *)o->sm_ilhs, (const double *)o->sm_xout, volumetol);
             o->launches++;
             /* the leaving row, maxvolume.rs:143-150 */
-            for (int attempt = 0;; attempt++) {
-                SpMulti W{n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)iota, nullptr};
+            st = rerun([&](bool again, bool *asks) -> int {
+                SpMulti W{n, again, 1, nullptr, nullptr, nullptr, (const i64 *)iota, nullptr};
                 BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, d, 0, (const i64 *)V.leave, (const double *)nullptr, 'T', 1, 0,
                            o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
                 BLU_LAUNCH(k_mv_absorb, g, 128, 0, s, V, (const int *)o->sm_scal, 2);
                 o->launches += 2;
                 CK(cudaGetLastError());
-                if ((st = mv_any_realloc(o, c, V, o->sm_scal, 2, &again)) != BLU_OK) return st;
-                if (!again) break;
-                if (attempt == 39) return BLU_ERROR_OUT_OF_MEMORY;
-                if ((st = grow_batch_stores(o)) != BLU_OK) return st;
-            }
+                return mv_any_realloc(o, c, V, o->sm_scal, 2, asks);
+            });
+            if (st != BLU_OK) return st;
             /* update and the refactorization policy, maxvolume.rs:151-170 */
-            for (int attempt = 0;; attempt++) {
-                BLU_LAUNCH(k_update, n, 32, 0, s, d, 0.0, ust, (const double *)V.xtbl, attempt > 0 ? 1 : 0);
+            st = rerun([&](bool again, bool *asks) -> int {
+                BLU_LAUNCH(k_update, n, 32, 0, s, d, 0.0, ust, (const double *)V.xtbl, again ? 1 : 0);
                 o->launches++;
-                if ((st = decide_next(ust, j + 1)) != BLU_OK) return st;
-                if ((st = mv_any_realloc(o, c, V, ust, 1, &again)) != BLU_OK) return st;
-                if (!again) break;
-                if (attempt == 39) return BLU_ERROR_OUT_OF_MEMORY;
-                if ((st = grow_batch_stores(o)) != BLU_OK) return st;      /* blu.rs:319-334 */
-            }
+                return (st = decide_next(ust, j + 1)) != BLU_OK ? st : mv_any_realloc(o, c, V, ust, 1, asks);
+            });
+            if (st != BLU_OK) return st;
             if (c.h_cnt[MV_CNT_REFACTOR] > 0) {
                 if ((st = mv_factorize(o, c, V, (int64_t)c.h_cnt[MV_CNT_MAXNZ])) != BLU_OK) return st;
                 if ((st = next_after_factorize(j + 1)) != BLU_OK) return st;
@@ -2004,7 +2020,7 @@ static int subset_select(blu_b200 *o, int64_t nsel, const int64_t *sel, std::vec
 }
 
 /* the run mask of the selected slots on the batch until c goes out of scope */
-static int subset_mask(blu_b200 *o, MvCall &c, const std::vector<int> &pos) {
+static int subset_mask(blu_b200 *o, MaskedCall &c, const std::vector<int> &pos) {
     const size_t n = pos.size();
     std::vector<int> run(n);
     for (size_t k = 0; k < n; k++) run[k] = pos[k] >= 0;
@@ -2016,18 +2032,6 @@ static int subset_mask(blu_b200 *o, MvCall &c, const std::vector<int> &pos) {
     o->d.run = d_run;
     o->hrun.assign(run.begin(), run.end());
     return BLU_OK;
-}
-
-/* first non-OK status in selection order; a Reallocate left over means a store could not grow */
-static int subset_statuses(int64_t nsel, std::vector<int> &st_r, int *status) {
-    int worst = BLU_OK;
-    for (int64_t r = 0; r < nsel; r++) {
-        int s = st_r[(size_t)r];
-        if (s == BLU_REALLOCATE) s = BLU_ERROR_OUT_OF_MEMORY;
-        if (status) status[r] = s;
-        if (s != BLU_OK && worst == BLU_OK) worst = s;
-    }
-    return worst;
 }
 
 /* The summary of a device-resident call (blu_dev_calls.cuh): allocated on first use, cleared before each launch
@@ -2078,7 +2082,7 @@ static ResidentB resident_b(const blu_b200 *o) {
  * ones, compacted into fresh library-owned buffers that replace the old ones.  *maxnz: the most entries of one new B.
  * The slots' entry counts are scanned on the host when it has the selection (hpos, the host copy of dpos), and on
  * the device otherwise, so that only the new total and *maxnz come back.  On failure the old resident B stays. */
-static int rebuild_b(blu_b200 *o, MvCall &c, const int *dpos, const std::vector<int> *hpos, const blu_i64 *nb, const blu_i64 *ne,
+static int rebuild_b(blu_b200 *o, MaskedCall &c, const int *dpos, const std::vector<int> *hpos, const blu_i64 *nb, const blu_i64 *ne,
                      const blu_i64 *ni, const double *nx, int64_t *maxnz) {
     BluDev &d = o->d;
     const size_t n = (size_t)d.nmat, M = (size_t)d.m;
@@ -2140,7 +2144,7 @@ static int rebuild_b(blu_b200 *o, MvCall &c, const int *dpos, const std::vector<
 
 /* rebuild_b from host arrays: the selection's new B (column j of the r-th selected basis at b_begin/b_end[r*m + j])
  * goes up to the device first */
-static int subset_rebuild_b(blu_b200 *o, MvCall &c, const std::vector<int> &pos, int64_t nsel, const int64_t *b_begin,
+static int subset_rebuild_b(blu_b200 *o, MaskedCall &c, const std::vector<int> &pos, int64_t nsel, const int64_t *b_begin,
                             const int64_t *b_end, const int64_t *b_i, const double *b_x, int64_t bnz_total, int64_t *maxnz) {
     const size_t n = (size_t)o->d.nmat, cols = (size_t)nsel * (size_t)o->d.m;
     const cudaStream_t s = o->stream;
@@ -2176,7 +2180,7 @@ extern "C" int blu_batch_factorize_subset(blu_batch_t *o, int64_t nsel, const in
         if (b_begin[q] < 0 || b_begin[q] > bnz_total || b_end[q] < 0 || b_end[q] > bnz_total) return BLU_ERROR_INVALID_ARGUMENT;
     if (nsel == 0) return BLU_OK;
     CK(cudaSetDevice(o->device));
-    MvCall c(o);
+    MaskedCall c(o);
     int64_t maxnz = 0;
     if ((st = subset_rebuild_b(o, c, pos, nsel, b_begin, b_end, b_i, b_x, bnz_total, &maxnz)) != BLU_OK) return st;
     const double rebuild_ms = o->last_ms[0];
@@ -2184,9 +2188,9 @@ extern "C" int blu_batch_factorize_subset(blu_batch_t *o, int64_t nsel, const in
     if ((st = subset_mask(o, c, pos)) != BLU_OK) return st;
     const int fst = factorize_resident(o);
     o->last_ms[0] += rebuild_ms;
-    std::vector<int> st_r((size_t)nsel);
-    for (int64_t r = 0; r < nsel; r++) st_r[(size_t)r] = o->hinfo[(size_t)sel[r]].status;
-    const int worst = subset_statuses(nsel, st_r, status);
+    std::vector<int> st_k(o->hinfo.size());
+    for (size_t k = 0; k < st_k.size(); k++) st_k[k] = o->hinfo[k].status;
+    const int worst = tally_statuses(st_k.data(), 1, nsel, sel, status, nullptr);
     return fst != BLU_OK ? fst : worst;
 }
 
@@ -2207,7 +2211,7 @@ extern "C" int blu_batch_solve_for_update_subset(blu_batch_t *o, int64_t nsel, c
     CK(cudaSetDevice(o->device));
     const size_t n = (size_t)o->d.nmat, m = (size_t)o->d.m;
     const cudaStream_t s = o->stream;
-    MvCall c(o);
+    MaskedCall c(o);
     if ((st = ensure_batch_sparse(o, tot)) != BLU_OK) return st;
     std::vector<int64_t> hb(n, 0), he(n, 0);
     for (int64_t r = 0; r < nsel; r++) { hb[(size_t)sel[r]] = rhs_begin[r]; he[(size_t)sel[r]] = rhs_begin[r + 1]; }
@@ -2218,30 +2222,25 @@ extern "C" int blu_batch_solve_for_update_subset(blu_batch_t *o, int64_t nsel, c
     if (tot > 0) CK(cudaMemcpyAsync(o->sm_irhs, irhs, (size_t)tot * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     if (tot > 0 && xrhs) CK(cudaMemcpyAsync(o->sm_xrhs, xrhs, (size_t)tot * sizeof(double), cudaMemcpyHostToDevice, s));
     if ((st = subset_mask(o, c, pos)) != BLU_OK) return st;
-    std::vector<int> hs(2 * n), st_r((size_t)nsel);
-    for (int attempt = 0; attempt < 40; attempt++) {
-        SpMulti W{(int)n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)db, (const i64 *)de};
+    std::vector<int> hs(2 * n);
+    st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
+        SpMulti W{(int)n, rerun, 1, nullptr, nullptr, nullptr, (const i64 *)db, (const i64 *)de};
         BLU_LAUNCH(k_solve_sparse, (int)n, 32, 0, s, o->d, 0, (const i64 *)o->sm_irhs, xrhs ? (const double *)o->sm_xrhs : (const double *)nullptr,
                    trans, 1, want_solution ? 1 : 0, o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
         o->launches++;
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(hs.data(), o->sm_scal, 2 * n * sizeof(int), cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
-        bool again = false;      /* (the words of the masked-out slots are stale) */
-        for (int64_t r = 0; r < nsel; r++) again = again || hs[2 * (size_t)sel[r]] == BLU_REALLOCATE;
-        if (!again) break;
-        if (grow_batch_stores(o) != BLU_OK) break;      /* blu.rs:268-291; what still says Reallocate is reported as out of memory */
-    }
-    for (int64_t r = 0; r < nsel; r++) st_r[(size_t)r] = hs[2 * (size_t)sel[r]];
-    const int worst = subset_statuses(nsel, st_r, status);
+        /* (the words of the masked-out slots are stale) */
+        for (int64_t r = 0; r < nsel; r++) *asks = *asks || hs[2 * (size_t)sel[r]] == BLU_REALLOCATE;
+        return BLU_OK;
+    });
+    if (st != BLU_OK && st != BLU_REALLOCATE) return st;      /* Reallocate left over: a store could not grow */
+    const int worst = tally_statuses(hs.data(), 2, nsel, sel, status, want_solution ? nzlhs : nullptr);
     o->info_dirty = 1;
     if (!want_solution) return worst;
     std::vector<int64_t> hoff((size_t)nsel + 1, 0);
-    for (int64_t r = 0; r < nsel; r++) {
-        const size_t k = (size_t)sel[r];
-        nzlhs[r] = st_r[(size_t)r] == BLU_OK ? hs[2 * k + 1] : -1;
-        hoff[(size_t)r + 1] = hoff[(size_t)r] + std::max<int64_t>(nzlhs[r], 0);
-    }
+    for (int64_t r = 0; r < nsel; r++) hoff[(size_t)r + 1] = hoff[(size_t)r] + std::max<int64_t>(nzlhs[r], 0);
     const int64_t fill = hoff[(size_t)nsel];
     if (fill == 0) return worst;
     blu_i64 *dsel = nullptr, *doff = nullptr, *pi = nullptr; double *px = nullptr;
@@ -2278,27 +2277,25 @@ extern "C" int blu_batch_update_subset(blu_batch_t *o, int64_t nsel, const int64
     CK(cudaSetDevice(o->device));
     const size_t n = (size_t)o->d.nmat;
     const cudaStream_t s = o->stream;
-    MvCall c(o);
+    MaskedCall c(o);
     if ((st = ensure_batch_sparse(o, 0)) != BLU_OK) return st;
     std::vector<double> hx(n, 0.0);
     for (int64_t r = 0; r < nsel; r++) hx[(size_t)sel[r]] = xtbl[r];
     CK(cudaMemcpyAsync(o->sm_dbls, hx.data(), n * sizeof(double), cudaMemcpyHostToDevice, s));
     if ((st = subset_mask(o, c, pos)) != BLU_OK) return st;
-    std::vector<int> hs(n), st_r((size_t)nsel);
-    for (int attempt = 0; attempt < 40; attempt++) {
-        BLU_LAUNCH(k_update, (int)n, 32, 0, s, o->d, 0.0, o->sm_scal, (const double *)o->sm_dbls, attempt > 0 ? 1 : 0);
+    std::vector<int> hs(n);
+    st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
+        BLU_LAUNCH(k_update, (int)n, 32, 0, s, o->d, 0.0, o->sm_scal, (const double *)o->sm_dbls, rerun ? 1 : 0);
         o->launches++;
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(hs.data(), o->sm_scal, n * sizeof(int), cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
-        bool again = false;
-        for (int64_t r = 0; r < nsel; r++) again = again || hs[(size_t)sel[r]] == BLU_REALLOCATE;
-        if (!again) break;
-        if (grow_batch_stores(o) != BLU_OK) break;      /* blu.rs:319-334 */
-    }
-    for (int64_t r = 0; r < nsel; r++) st_r[(size_t)r] = hs[(size_t)sel[r]];
+        for (int64_t r = 0; r < nsel; r++) *asks = *asks || hs[(size_t)sel[r]] == BLU_REALLOCATE;
+        return BLU_OK;
+    });
+    if (st != BLU_OK && st != BLU_REALLOCATE) return st;      /* Reallocate left over: a store could not grow */
     o->info_dirty = 1;
-    return subset_statuses(nsel, st_r, status);
+    return tally_statuses(hs.data(), 1, nsel, sel, status, nullptr);
 }
 
 /* ------------------------------------------------------------------ */
@@ -2339,7 +2336,7 @@ extern "C" int blu_batch_factorize_subset_dev(blu_batch_t *o, const int *d_run, 
         BLU_LAUNCH(k_dev_check_b, n, 128, 0, s, d.m, d_run, (const blu_i64 *)d_b_begin, (const blu_i64 *)d_b_end, (blu_i64)bnz_total, o->d_sum);
     });
     if (st != BLU_OK) return st;
-    MvCall c(o);
+    MaskedCall c(o);
     int *dpos = nullptr, *scal = nullptr;
     if ((st = c.alloc(&dpos, (size_t)n)) != BLU_OK || (st = c.alloc(&scal, (size_t)n)) != BLU_OK) return st;
     BLU_LAUNCH(k_dev_pos, grid_of(n, 256), 256, 0, s, n, d_run, dpos);
@@ -2383,21 +2380,21 @@ extern "C" int blu_batch_solve_for_update_dev(blu_batch_t *o, const int *d_run, 
         BLU_LAUNCH(k_dev_check_rhs, grid_of(n + 1, 256), 256, 0, s, n, d_run, (const blu_i64 *)d_rhs_begin, d_irhs ? 0 : 1, o->d_sum);
     });
     if (st != BLU_OK) return st;
-    MvCall c(o);
+    MaskedCall c(o);
     o->d.run = d_run;
     i64 *il = want_solution ? (i64 *)d_ilhs : (i64 *)o->sm_ilhs;
     double *xl = want_solution ? d_xlhs : o->sm_xout;
-    for (int attempt = 0; attempt < 40; attempt++) {
-        SpMulti W{n, attempt > 0, 1, nullptr, nullptr, nullptr, (const i64 *)d_rhs_begin, nullptr};
+    st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
+        SpMulti W{n, rerun, 1, nullptr, nullptr, nullptr, (const i64 *)d_rhs_begin, nullptr};
         BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, o->d, 0, (const i64 *)d_irhs, d_xrhs, trans, 1, want_solution ? 1 : 0, o->sm_scal, il, xl, W);
         o->launches++;
         CK(cudaGetLastError());
         if ((st = dev_sum_reset(o)) != BLU_OK || (st = dev_finish(o, n, 0, d_run, o->sm_scal, 2, d_status, want_solution ? d_nzlhs : nullptr)) != BLU_OK ||
             (st = dev_sum_read(o)) != BLU_OK) return st;
-        if (!o->h_sum[DEV_SUM_REALLOC]) break;
-        /* blu.rs:268-291: grow and run those bases again; what still says Reallocate is reported as out of memory */
-        if (grow_batch_stores(o) != BLU_OK) break;
-    }
+        *asks = o->h_sum[DEV_SUM_REALLOC] != 0;
+        return BLU_OK;
+    });
+    if (st != BLU_OK && st != BLU_REALLOCATE) return st;      /* Reallocate left over: a store could not grow */
     o->info_dirty = 1;
     return dev_sum_first(o);
 }
@@ -2411,17 +2408,18 @@ extern "C" int blu_batch_update_dev(blu_batch_t *o, const int *d_run, const doub
     int st = ensure_batch_sparse(o, 0);
     if (st == BLU_OK) st = dev_sum_ensure(o);
     if (st != BLU_OK) return st;
-    MvCall c(o);
+    MaskedCall c(o);
     o->d.run = d_run;
-    for (int attempt = 0; attempt < 40; attempt++) {
-        BLU_LAUNCH(k_update, n, 32, 0, s, o->d, 0.0, o->sm_scal, d_xtbl, attempt > 0 ? 1 : 0);
+    st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
+        BLU_LAUNCH(k_update, n, 32, 0, s, o->d, 0.0, o->sm_scal, d_xtbl, rerun ? 1 : 0);
         o->launches++;
         CK(cudaGetLastError());
         if ((st = dev_sum_reset(o)) != BLU_OK || (st = dev_finish(o, n, 0, d_run, o->sm_scal, 1, d_status, nullptr)) != BLU_OK ||
             (st = dev_sum_read(o)) != BLU_OK) return st;
-        if (!o->h_sum[DEV_SUM_REALLOC]) break;
-        if (grow_batch_stores(o) != BLU_OK) break;      /* blu.rs:319-334 */
-    }
+        *asks = o->h_sum[DEV_SUM_REALLOC] != 0;
+        return BLU_OK;
+    });
+    if (st != BLU_OK && st != BLU_REALLOCATE) return st;      /* Reallocate left over: a store could not grow */
     o->info_dirty = 1;
     return dev_sum_first(o);
 }
@@ -2551,7 +2549,7 @@ static int copy_run(blu_b200 *o, int64_t ncopy, const int64_t *dst, const int64_
         if (e.u_idx) bytes += rnd((size_t)(e.u_mem + PADDING) * 4) + rnd((size_t)(e.u_mem + PADDING) * 8);
         if (e.w_idx) bytes += rnd((size_t)(2 * e.w_mem + PADDING) * 4) + rnd((size_t)(2 * e.w_mem + PADDING) * 8);
     }
-    MvCall c(o);
+    MaskedCall c(o);
     int *dpairs = nullptr;
     int st = c.alloc(&dpairs, 2 * (size_t)ncopy);
     if (st != BLU_OK) return st;
@@ -2640,7 +2638,7 @@ static int save_check(blu_b200 *o, int64_t n, const int64_t *idx, void *const *b
 }
 
 /* the headers of the images of bases idx (on the device, checksum 0) and their sizes (bytes, on the host) */
-static int save_extents(blu_b200 *o, MvCall &c, int64_t n, const int64_t *idx, int **didx, BluImage **dhdr, int64_t *bytes) {
+static int save_extents(blu_b200 *o, MaskedCall &c, int64_t n, const int64_t *idx, int **didx, BluImage **dhdr, int64_t *bytes) {
     const cudaStream_t s = o->stream;
     blu_i64 *dbytes = nullptr;
     int st = c.alloc(didx, (size_t)n);
@@ -2659,7 +2657,7 @@ static int save_extents(blu_b200 *o, MvCall &c, int64_t n, const int64_t *idx, i
 }
 
 /* the images of bases didx into the device buffers dimg (n pointers, on the device), checksums included */
-static int save_write(blu_b200 *o, MvCall &c, int64_t n, const int *didx, const BluImage *dhdr, unsigned char *const *dimg) {
+static int save_write(blu_b200 *o, MaskedCall &c, int64_t n, const int *didx, const BluImage *dhdr, unsigned char *const *dimg) {
     const cudaStream_t s = o->stream;
     blu_u64 *part = nullptr;
     int st = c.alloc(&part, (size_t)n * SAVE_PARTS);
@@ -2679,7 +2677,7 @@ extern "C" int blu_batch_save_dev(blu_batch_t *o, int64_t n, const int64_t *idx,
     int st = save_check(o, n, idx, d_buf, cap, bytes);
     if (st != BLU_OK || n == 0) return st;
     CK(cudaSetDevice(o->device));
-    MvCall c(o);
+    MaskedCall c(o);
     int *didx = nullptr; BluImage *dhdr = nullptr;
     if ((st = save_extents(o, c, n, idx, &didx, &dhdr, bytes)) != BLU_OK || !d_buf) return st;
     for (int64_t r = 0; r < n; r++) if (cap[r] < bytes[r]) return BLU_ERROR_INVALID_ARGUMENT;
@@ -2707,7 +2705,7 @@ extern "C" int blu_batch_save(blu_batch_t *o, int64_t n, const int64_t *idx, voi
     if (st != BLU_OK || n == 0) return st;
     CK(cudaSetDevice(o->device));
     const cudaStream_t s = o->stream;
-    MvCall c(o);
+    MaskedCall c(o);
     int *didx = nullptr; BluImage *dhdr = nullptr;
     if ((st = save_extents(o, c, n, idx, &didx, &dhdr, bytes)) != BLU_OK || !buf) return st;
     for (int64_t r = 0; r < n; r++) if (cap[r] < bytes[r]) return BLU_ERROR_INVALID_ARGUMENT;
@@ -2753,7 +2751,7 @@ static bool img_header_ok(const BluImage &h, int m, int64_t cap) {
 
 /* The images at the device pointers dimg (host array): their headers come up and are checked, then (verify) their
  * checksums on the device; nothing has changed when either fails.  commit: basis dst[r] becomes the basis of image r. */
-static int restore_images(blu_b200 *o, MvCall &c, int64_t n, const int64_t *dst, const unsigned char *const *dimg_h, const int64_t *cap,
+static int restore_images(blu_b200 *o, MaskedCall &c, int64_t n, const int64_t *dst, const unsigned char *const *dimg_h, const int64_t *cap,
                           bool verify, bool commit) {
     BluDev &d = o->d;
     const cudaStream_t s = o->stream;
@@ -2839,7 +2837,7 @@ extern "C" int blu_batch_restore_dev(blu_batch_t *o, int64_t n, const int64_t *d
     const int st = restore_check(o, n, dst, d_buf, cap);
     if (st != BLU_OK || n == 0) return st;
     CK(cudaSetDevice(o->device));
-    MvCall c(o);
+    MaskedCall c(o);
     return restore_images(o, c, n, dst, (const unsigned char *const *)d_buf, cap, true, true);
 }
 
@@ -2857,7 +2855,7 @@ extern "C" int blu_batch_restore(blu_batch_t *o, int64_t n, const int64_t *dst, 
     }
     CK(cudaSetDevice(o->device));
     const cudaStream_t s = o->stream;
-    MvCall c(o);
+    MaskedCall c(o);
     const size_t scratch = img_scratch(sz);
     unsigned char *scr = nullptr;
     if ((st = c.alloc(&scr, scratch)) != BLU_OK) return st;
