@@ -75,6 +75,11 @@ def load_library(path=None):
     L.blu_solve_sparse.argtypes = [vp, ctypes.c_int64, i64p, f64p, i64p, i64p, f64p, ctypes.c_char]
     L.blu_solve_for_update.argtypes = [vp, ctypes.c_int64, i64p, f64p, i64p, i64p, f64p, ctypes.c_char]
     L.blu_update.argtypes = [vp, ctypes.c_double]
+    L.blu_clone.argtypes = [ctypes.POINTER(vp), vp]
+    for f in ("blu_save", "blu_save_dev"):
+        getattr(L, f).argtypes = [vp, vp, ctypes.c_int64, i64p]
+    for f in ("blu_restore", "blu_restore_dev"):
+        getattr(L, f).argtypes = [vp, vp, ctypes.c_int64]
     L.blu_batch_create.argtypes = [ctypes.POINTER(vp), ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, ctypes.c_int]
     L.blu_batch_destroy.argtypes = [vp]
     L.blu_batch_factorize.argtypes = [vp, i64p, i64p, i64p, f64p, ctypes.c_int64, i32p]
@@ -163,6 +168,49 @@ class _Base:
         else:
             object.__setattr__(self, name, value)
 
+    # Device memory as torch tensors (the _dev calls of BLUBatch, BLU.save_dev / restore_dev).
+
+    def _torch_device(self):
+        import torch
+        if b"emulation" in self._L.blu_version():      # the SIMT emulation build: its "device" memory is host memory
+            return torch.device("cpu")
+        if getattr(self, "_cuda_index", None) is None:
+            object.__setattr__(self, "_cuda_index", self._device if self._device >= 0 else torch.cuda.current_device())
+        return torch.device("cuda", self._cuda_index)
+
+    def _tensor(self, t, dtype, numel, name, dev):
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{name}: a torch.Tensor is expected")
+        if t.dtype != dtype:
+            raise TypeError(f"{name}: dtype {t.dtype}, expected {dtype}")
+        if t.device != dev:
+            raise ValueError(f"{name}: tensor on {t.device}, the {'batch' if isinstance(self, BLUBatch) else 'object'} is on {dev}")
+        if not t.is_contiguous():
+            raise ValueError(f"{name}: not contiguous")
+        if numel is not None and t.numel() != numel:
+            raise ValueError(f"{name}: {t.numel()} elements, expected {numel}")
+        return t
+
+    @staticmethod
+    def _ptr(t):
+        return ctypes.c_void_p(t.data_ptr()) if t is not None and t.numel() > 0 else None
+
+    def _on_stream(self, dev, fn):
+        """run fn (one library call) after everything torch has queued on its current stream of dev"""
+        import torch
+        if dev.type == "cuda":
+            s = torch.cuda.ExternalStream(self._L.blu_batch_stream(self._h), device=dev)
+            s.wait_stream(torch.cuda.current_stream(dev))
+        return fn()
+
+    @staticmethod
+    def _aligned_host(nbytes):
+        """a numpy.uint8 array of nbytes whose data starts 16-byte aligned"""
+        raw = np.zeros(int(nbytes) + 16, np.uint8)
+        k = (-raw.ctypes.data) % 16
+        return raw[k:k + int(nbytes)]
+
 
 class BLU(_Base):
     """struct BLU, blu.rs:9-20: `lu` state on the device, `lhs/ilhs/nzlhs` on the host."""
@@ -178,6 +226,7 @@ class BLU(_Base):
         self.lhs = np.zeros(self.m)
         self.ilhs = np.zeros(self.m, dtype=np.int64)
         self.nzlhs = 0
+        self._device = int(device)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -295,6 +344,74 @@ class BLU(_Base):
     # blu.rs:319
     def update(self, xtbl):
         return self._L.blu_update(self._h, float(xtbl))
+
+    def clone(self):
+        """BLU: Clone (blu_clone): a new object on this one's device with its factors, update history, pending
+        solve_for_update, getters, parameters, capacities, resident B and lhs / ilhs / nzlhs.  From then on it behaves
+        bit for bit as this one would.  Raises on a failed call."""
+        h = ctypes.c_void_p()
+        st = self._L.blu_clone(ctypes.byref(h), self._h)
+        if st != 0:
+            raise RuntimeError(f"blu_clone: status {st}")
+        c = BLU.__new__(BLU)
+        c._L, c._h, c.m, c._device = self._L, h, self.m, self._device
+        c.lhs, c.ilhs, c.nzlhs = self.lhs.copy(), self.ilhs.copy(), self.nzlhs
+        return c
+
+    def __copy__(self):
+        return self.clone()
+
+    def __deepcopy__(self, memo):
+        return self.clone()
+
+    # Images (blu_save / blu_restore): the format of BLUBatch.save / restore, so that an image moves a basis between
+    # objects and batch slots of the same m.
+
+    def save(self):
+        """The object's image as a numpy.uint8 array.  Raises on a failed call."""
+        n = ctypes.c_int64(0)
+        st = self._L.blu_save(self._h, None, 0, ctypes.byref(n))
+        if st != 0:
+            raise ValueError(f"blu_save: status {st}")
+        a = self._aligned_host(n.value)
+        st = self._L.blu_save(self._h, ctypes.c_void_p(a.ctypes.data), a.size, ctypes.byref(n))
+        if st != 0:
+            raise ValueError(f"blu_save: status {st}")
+        return a
+
+    def restore(self, img):
+        """The object becomes the basis saved in img (a buffer of bytes: a numpy.uint8 array, bytes, ...).  Returns
+        the status."""
+        a = np.frombuffer(img, np.uint8) if not isinstance(img, np.ndarray) else np.ascontiguousarray(img).view(np.uint8).reshape(-1)
+        if a.ctypes.data % 16:
+            b = self._aligned_host(a.size)
+            b[:] = a
+            a = b
+        return self._L.blu_restore(self._h, ctypes.c_void_p(a.ctypes.data), a.size)
+
+    def save_dev(self):
+        """The object's image as a 1-D torch.uint8 tensor on its device, 256-byte aligned.  Ordered after torch's
+        current stream.  Raises on a failed call."""
+        import torch
+        dev = self._torch_device()
+        n = ctypes.c_int64(0)
+        st = self._on_stream(dev, lambda: self._L.blu_save_dev(self._h, None, 0, ctypes.byref(n)))
+        if st != 0:
+            raise ValueError(f"blu_save_dev: status {st}")
+        block = torch.empty(n.value + 256, dtype=torch.uint8, device=dev)
+        at = (-block.data_ptr()) % 256
+        out = block[at:at + n.value]
+        st = self._on_stream(dev, lambda: self._L.blu_save_dev(self._h, ctypes.c_void_p(out.data_ptr()), out.numel(), ctypes.byref(n)))
+        if st != 0:
+            raise ValueError(f"blu_save_dev: status {st}")
+        return out
+
+    def restore_dev(self, img):
+        """restore from a contiguous torch.uint8 tensor on the object's device.  Returns the status."""
+        import torch
+        dev = self._torch_device()
+        t = self._tensor(img, torch.uint8, None, "img", dev)
+        return self._on_stream(dev, lambda: self._L.blu_restore_dev(self._h, ctypes.c_void_p(t.data_ptr()), t.numel()))
 
 
 class BLUBatch(_Base):
@@ -493,28 +610,6 @@ class BLUBatch(_Base):
     # Outputs come back as tensors; out tensors passed in are written in place, and the entries of bases or units that
     # do not run keep what they held (zeros when the call allocates them).
 
-    def _torch_device(self):
-        import torch
-        if b"emulation" in self._L.blu_version():      # the SIMT emulation build: its "device" memory is host memory
-            return torch.device("cpu")
-        if getattr(self, "_cuda_index", None) is None:
-            object.__setattr__(self, "_cuda_index", self._device if self._device >= 0 else torch.cuda.current_device())
-        return torch.device("cuda", self._cuda_index)
-
-    def _tensor(self, t, dtype, numel, name, dev):
-        import torch
-        if not isinstance(t, torch.Tensor):
-            raise TypeError(f"{name}: a torch.Tensor is expected")
-        if t.dtype != dtype:
-            raise TypeError(f"{name}: dtype {t.dtype}, expected {dtype}")
-        if t.device != dev:
-            raise ValueError(f"{name}: tensor on {t.device}, the batch is on {dev}")
-        if not t.is_contiguous():
-            raise ValueError(f"{name}: not contiguous")
-        if numel is not None and t.numel() != numel:
-            raise ValueError(f"{name}: {t.numel()} elements, expected {numel}")
-        return t
-
     def _out(self, t, dtype, numel, name, dev, shape):
         import torch
         if t is None:
@@ -529,18 +624,6 @@ class BLUBatch(_Base):
             self._tensor(run, torch.bool, self.nmat, "run", dev)
             return run.to(torch.int32)
         return self._tensor(run, torch.int32, self.nmat, "run", dev)
-
-    @staticmethod
-    def _ptr(t):
-        return ctypes.c_void_p(t.data_ptr()) if t is not None and t.numel() > 0 else None
-
-    def _on_stream(self, dev, fn):
-        """run fn (one library call) after everything torch has queued on its current stream of dev"""
-        import torch
-        if dev.type == "cuda":
-            s = torch.cuda.ExternalStream(self._L.blu_batch_stream(self._h), device=dev)
-            s.wait_stream(torch.cuda.current_stream(dev))
-        return fn()
 
     def factorize_subset_dev(self, b_begin, b_end, b_i, b_x, run=None, status=None):
         """Refactorize the bases whose run flag is set (every basis for run=None) from B in device memory: column j of
@@ -661,13 +744,6 @@ class BLUBatch(_Base):
         ptrs = (ctypes.c_void_p * max(n, 1))(*[b[0] for b in bufs])
         cap = _i64([b[1] for b in bufs])
         return fn(self._h, n, _pi(s), ptrs, _pi(cap), _pi(nbytes)), nbytes
-
-    @staticmethod
-    def _aligned_host(nbytes):
-        """a numpy.uint8 array of nbytes whose data starts 16-byte aligned"""
-        raw = np.zeros(int(nbytes) + 16, np.uint8)
-        k = (-raw.ctypes.data) % 16
-        return raw[k:k + int(nbytes)]
 
     def save(self, idx):
         """The images of bases idx (repeats allowed) as a list of numpy.uint8 arrays.  Raises on a failed call."""

@@ -211,7 +211,8 @@ static int alloc_dense(blu_b200 *o, int want, int want_big) {
     return st;
 }
 
-static int create_common(blu_b200 **out, int64_t nmat, int64_t m, int64_t bnz_cap, int device, int single) {
+/* like (blu_clone): the new object takes like's L/U/W capacities and dense-tail sizes instead of the defaults */
+static int create_common(blu_b200 **out, int64_t nmat, int64_t m, int64_t bnz_cap, int device, int single, const blu_b200 *like = nullptr) {
     if (!out || m < 1 || nmat < 1 || bnz_cap < 0 || m > 0x7fffff /* line counts live in 23 bits of the search keys, blu_dev_common.cuh:mkckey */) return BLU_ERROR_INVALID_ARGUMENT;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
@@ -254,6 +255,7 @@ static int create_common(blu_b200 **out, int64_t nmat, int64_t m, int64_t bnz_ca
      * device build starts larger because a Reallocate costs a full re-run here. */
     d.l_mem = d.u_mem = 8 * d.bnz_cap + 4 * m;
     d.w_mem = 24 * d.bnz_cap + 16 * m;     /* room for the fill of the sparse head without garbage collection (measured on configs[1]: 8*nnz + 8*m collects 1.4 times per basis and costs 10 %) */
+    if (like) { d.l_mem = like->d.l_mem; d.u_mem = like->d.u_mem; d.w_mem = like->d.w_mem; }
     d.prm.droptol = 1e-20; d.prm.abstol = 1e-14; d.prm.reltol = 0.1;
     d.prm.nzbias = 1; d.prm.maxsearch = 3; d.prm.pad = 4; d.prm.stretch = 0.3;
     d.prm.compress_thres = 0.5; d.prm.sparse_thres = 0.05; d.prm.search_rows = 0;
@@ -292,6 +294,7 @@ static int create_common(blu_b200 **out, int64_t nmat, int64_t m, int64_t bnz_ca
         int kd = o->kd_smem_max, kb = single ? 0 : 256;
         if (const char *e = getenv("BLU_B200_DENSE_K")) kd = atoi(e);      /* tuning knob, same as BLU_P_DENSE_K */
         if (const char *e = getenv("BLU_B200_DENSE_K_BIG")) kb = atoi(e);  /* tuning knob, same as BLU_P_DENSE_K_BIG */
+        if (like) { kd = like->d.dense_k; kb = like->want_kbig; }
         o->want_kbig = kb;
         st = alloc_dense(o, kd, kb);
     }
@@ -1105,6 +1108,7 @@ extern "C" int blu_solve_dense(blu_t *o, const double *rhs, double *lhs, char tr
     if (o->hinfo[0].nupdate < 0) return BLU_ERROR_INVALID_CALL;   /* solve_dense.rs:25 */
     int status = BLU_OK;
     int st = blu_batch_solve_dense(o, rhs, lhs, trans, &status);
+    o->info_dirty = 1;      /* the solve compacts the pivot sequence (pivotlen), as blu_solve_dense_multi's does */
     o->time_solve += 1e-3 * o->last_ms[1];
     return st != BLU_OK ? st : status;
 }
@@ -2673,11 +2677,11 @@ static int save_write(blu_b200 *o, MaskedCall &c, int64_t n, const int *didx, co
     return BLU_OK;
 }
 
-extern "C" int blu_batch_save_dev(blu_batch_t *o, int64_t n, const int64_t *idx, void *const *d_buf, const int64_t *cap, int64_t *bytes) {
-    int st = save_check(o, n, idx, d_buf, cap, bytes);
-    if (st != BLU_OK || n == 0) return st;
+/* the save calls after their argument checks (n > 0; batch and object alike) */
+static int save_device(blu_b200 *o, int64_t n, const int64_t *idx, void *const *d_buf, const int64_t *cap, int64_t *bytes) {
     CK(cudaSetDevice(o->device));
     MaskedCall c(o);
+    int st;
     int *didx = nullptr; BluImage *dhdr = nullptr;
     if ((st = save_extents(o, c, n, idx, &didx, &dhdr, bytes)) != BLU_OK || !d_buf) return st;
     for (int64_t r = 0; r < n; r++) if (cap[r] < bytes[r]) return BLU_ERROR_INVALID_ARGUMENT;
@@ -2700,12 +2704,11 @@ static size_t img_scratch(const std::vector<size_t> &sz) {
     return std::min(tot, std::max(IMG_SCRATCH, big));
 }
 
-extern "C" int blu_batch_save(blu_batch_t *o, int64_t n, const int64_t *idx, void *const *buf, const int64_t *cap, int64_t *bytes) {
-    int st = save_check(o, n, idx, buf, cap, bytes);
-    if (st != BLU_OK || n == 0) return st;
+static int save_host(blu_b200 *o, int64_t n, const int64_t *idx, void *const *buf, const int64_t *cap, int64_t *bytes) {
     CK(cudaSetDevice(o->device));
     const cudaStream_t s = o->stream;
     MaskedCall c(o);
+    int st;
     int *didx = nullptr; BluImage *dhdr = nullptr;
     if ((st = save_extents(o, c, n, idx, &didx, &dhdr, bytes)) != BLU_OK || !buf) return st;
     for (int64_t r = 0; r < n; r++) if (cap[r] < bytes[r]) return BLU_ERROR_INVALID_ARGUMENT;
@@ -2724,6 +2727,15 @@ extern "C" int blu_batch_save(blu_batch_t *o, int64_t n, const int64_t *idx, voi
         CK(cudaStreamSynchronize(s));
     }
     return BLU_OK;
+}
+
+extern "C" int blu_batch_save(blu_batch_t *o, int64_t n, const int64_t *idx, void *const *buf, const int64_t *cap, int64_t *bytes) {
+    const int st = save_check(o, n, idx, buf, cap, bytes);
+    return st != BLU_OK || n == 0 ? st : save_host(o, n, idx, buf, cap, bytes);
+}
+extern "C" int blu_batch_save_dev(blu_batch_t *o, int64_t n, const int64_t *idx, void *const *d_buf, const int64_t *cap, int64_t *bytes) {
+    const int st = save_check(o, n, idx, d_buf, cap, bytes);
+    return st != BLU_OK || n == 0 ? st : save_device(o, n, idx, d_buf, cap, bytes);
 }
 
 /* the arguments of a restore: n distinct destinations in [0, nmat), every buffer 16-byte aligned and holding a header */
@@ -2750,9 +2762,11 @@ static bool img_header_ok(const BluImage &h, int m, int64_t cap) {
 }
 
 /* The images at the device pointers dimg (host array): their headers come up and are checked, then (verify) their
- * checksums on the device; nothing has changed when either fails.  commit: basis dst[r] becomes the basis of image r. */
+ * checksums on the device; nothing has changed when either fails.  commit: basis dst[r] becomes the basis of image r.
+ * An object (n == 1, dst[0] == 0) has no per-basis stores: its own are replaced by stores of the image's capacities,
+ * and its sorted row-wise U is rebuilt when the basis is fresh -- or, keep_ur, left to the caller (blu_clone). */
 static int restore_images(blu_b200 *o, MaskedCall &c, int64_t n, const int64_t *dst, const unsigned char *const *dimg_h, const int64_t *cap,
-                          bool verify, bool commit) {
+                          bool verify, bool commit, bool keep_ur = false) {
     BluDev &d = o->d;
     const cudaStream_t s = o->stream;
     const size_t N = (size_t)d.nmat, M = (size_t)d.m;
@@ -2788,9 +2802,9 @@ static int restore_images(blu_b200 *o, MaskedCall &c, int64_t n, const int64_t *
         const BluImage &e = h[(size_t)r];
         btmax = std::max<int64_t>(btmax, e.bt_n);
         base[(size_t)r] = btot; btot += e.b_nz;
-        if (e.l_mem != d.l_mem) bytes += rnd((size_t)(e.l_mem + PADDING) * 4) + rnd((size_t)(e.l_mem + PADDING) * 8);
-        if (e.u_mem != d.u_mem) bytes += rnd((size_t)(e.u_mem + PADDING) * 4) + rnd((size_t)(e.u_mem + PADDING) * 8);
-        if (e.w_mem != d.w_mem) bytes += rnd((size_t)(2 * e.w_mem + PADDING) * 4) + rnd((size_t)(2 * e.w_mem + PADDING) * 8);
+        if (!o->single && e.l_mem != d.l_mem) bytes += rnd((size_t)(e.l_mem + PADDING) * 4) + rnd((size_t)(e.l_mem + PADDING) * 8);
+        if (!o->single && e.u_mem != d.u_mem) bytes += rnd((size_t)(e.u_mem + PADDING) * 4) + rnd((size_t)(e.u_mem + PADDING) * 8);
+        if (!o->single && e.w_mem != d.w_mem) bytes += rnd((size_t)(2 * e.w_mem + PADDING) * 4) + rnd((size_t)(2 * e.w_mem + PADDING) * 8);
         pos[(size_t)dst[r]] = (int)r; hdst[(size_t)r] = (int)dst[r];
     }
     if ((st = mv_ensure_bt_cap(o, btmax)) != BLU_OK) return st;
@@ -2810,11 +2824,19 @@ static int restore_images(blu_b200 *o, MaskedCall &c, int64_t n, const int64_t *
     if (bytes && (st = dalloc(o, &blk, bytes)) != BLU_OK) return st;
     int64_t maxnz = 0;
     if ((st = rebuild_b(o, c, dpos, nullptr, nb, ne, ni, nx, &maxnz)) != BLU_OK) { dfree(o, blk); return st; }
-    /* the resident B is the new one (a captured graph is dropped); from here on the call completes */
+    /* the resident B is the new one (a captured graph is dropped) */
+    if (o->single) {
+        /* the object's L, U and W stores (and the row-wise U, sized like U) become ones of the image's capacities; a
+         * failed allocation keeps the old stores and factors */
+        const BluImage &e = h[0];
+        if ((e.l_mem != d.l_mem || e.u_mem != d.u_mem || e.w_mem != d.w_mem) && (st = swap_stores(o, e.l_mem, e.u_mem, e.w_mem)) != BLU_OK)
+            return st;
+    }
+    /* from here on the call completes */
     if (blk) o->ext_blocks.push_back(blk);
     size_t off = 0;
     auto take = [&](size_t b) { unsigned char *p = blk + off; off += rnd(b); return p; };
-    for (int64_t r = 0; r < n; r++) {
+    for (int64_t r = 0; r < n && !o->single; r++) {
         const BluImage &e = h[(size_t)r];
         BluSlotStore f; memset(&f, 0, sizeof f);
         if (e.l_mem != d.l_mem) { f.l_idx = (int *)take((size_t)(e.l_mem + PADDING) * 4); f.l_val = (double *)take((size_t)(e.l_mem + PADDING) * 8); f.l_mem = e.l_mem; }
@@ -2822,20 +2844,34 @@ static int restore_images(blu_b200 *o, MaskedCall &c, int64_t n, const int64_t *
         if (e.w_mem != d.w_mem) { f.w_idx = (int *)take((size_t)(2 * e.w_mem + PADDING) * 4); f.w_val = (double *)take((size_t)(2 * e.w_mem + PADDING) * 8); f.w_mem = e.w_mem; }
         o->hslot[(size_t)dst[r]] = f;      /* (an old private block of dst is reclaimed at the next whole-batch store change) */
     }
-    o->have_overrides = 0;
-    for (const BluSlotStore &e : o->hslot) if (e.l_idx || e.u_idx || e.w_idx) o->have_overrides = 1;
-    CK(cudaMemcpyAsync(o->d_slot, o->hslot.data(), N * sizeof(BluSlotStore), cudaMemcpyHostToDevice, s));
+    if (!o->single) {
+        o->have_overrides = 0;
+        for (const BluSlotStore &e : o->hslot) if (e.l_idx || e.u_idx || e.w_idx) o->have_overrides = 1;
+        CK(cudaMemcpyAsync(o->d_slot, o->hslot.data(), N * sizeof(BluSlotStore), cudaMemcpyHostToDevice, s));
+    }
     BLU_LAUNCH(k_restore_slots, (int)(n * SAVE_PARTS), SAVE_THREADS, 0, s, d, (const int *)ddst, (const BluImage *)dhdr, (const unsigned char *const *)dimg);
     o->launches++;
     CK(cudaGetLastError());
+    if (o->single && !keep_ur) {
+        /* have_ur as a factorization leaves it: k_build_ur sets it where the basis is fresh (nupdate 0, status OK or
+         * WarningSingularMatrix).  k_build_ur counts in tmpi, which is slot state: the image's goes back after it, so
+         * that the object holds exactly the image. */
+        CK(cudaMemsetAsync(&d.info->have_ur, 0, sizeof(int), s));
+        BLU_LAUNCH(k_build_ur, 1, 256, 0, s, d);
+        o->launches++;
+        CK(cudaGetLastError());
+        const int t = IMG_STATE + STATE_TMPI;
+        CK(cudaMemcpyAsync(d.tmpi, dimg_h[0] + img_offset(h[0], t), (size_t)img_section_bytes(h[0], t), cudaMemcpyDeviceToDevice, s));
+        o->info_dirty = 1;
+    }
+    if (o->single) o->task_pending = 0;      /* (a pending blu_factorize_c0ntinue belonged to the old basis) */
     CK(cudaStreamSynchronize(s));      /* (pageable sources above) */
     for (int64_t r = 0; r < n; r++) o->hinfo[(size_t)dst[r]] = h[(size_t)r].info;
     return BLU_OK;
 }
 
-extern "C" int blu_batch_restore_dev(blu_batch_t *o, int64_t n, const int64_t *dst, const void *const *d_buf, const int64_t *cap) {
-    const int st = restore_check(o, n, dst, d_buf, cap);
-    if (st != BLU_OK || n == 0) return st;
+/* the restore calls after their argument checks (n > 0; batch and object alike) */
+static int restore_device(blu_b200 *o, int64_t n, const int64_t *dst, const void *const *d_buf, const int64_t *cap) {
     CK(cudaSetDevice(o->device));
     MaskedCall c(o);
     return restore_images(o, c, n, dst, (const unsigned char *const *)d_buf, cap, true, true);
@@ -2843,9 +2879,8 @@ extern "C" int blu_batch_restore_dev(blu_batch_t *o, int64_t n, const int64_t *d
 
 /* Through the device scratch in chunks; with more than one chunk, every chunk is verified before the first is
  * restored, so that a rejected image still changes nothing. */
-extern "C" int blu_batch_restore(blu_batch_t *o, int64_t n, const int64_t *dst, const void *const *buf, const int64_t *cap) {
-    int st = restore_check(o, n, dst, buf, cap);
-    if (st != BLU_OK || n == 0) return st;
+static int restore_host(blu_b200 *o, int64_t n, const int64_t *dst, const void *const *buf, const int64_t *cap) {
+    int st;
     std::vector<size_t> sz((size_t)n);
     for (int64_t r = 0; r < n; r++) {
         BluImage h;
@@ -2871,6 +2906,93 @@ extern "C" int blu_batch_restore(blu_batch_t *o, int64_t n, const int64_t *dst, 
             if ((st = restore_images(o, c, r1 - r0, dst + r0, hp.data() + r0, cap + r0, one || pass == 0, pass == 1)) != BLU_OK) return st;
         }
     }
+    return BLU_OK;
+}
+
+extern "C" int blu_batch_restore(blu_batch_t *o, int64_t n, const int64_t *dst, const void *const *buf, const int64_t *cap) {
+    const int st = restore_check(o, n, dst, buf, cap);
+    return st != BLU_OK || n == 0 ? st : restore_host(o, n, dst, buf, cap);
+}
+extern "C" int blu_batch_restore_dev(blu_batch_t *o, int64_t n, const int64_t *dst, const void *const *d_buf, const int64_t *cap) {
+    const int st = restore_check(o, n, dst, d_buf, cap);
+    return st != BLU_OK || n == 0 ? st : restore_device(o, n, dst, d_buf, cap);
+}
+
+/* ------------------------------------------------------------------ */
+/* object: clone, save and restore (the batch calls' images, one basis) */
+/* ------------------------------------------------------------------ */
+
+static const int64_t OBJECT_SLOT = 0;
+
+extern "C" int blu_save(blu_t *o, void *buf, int64_t cap, int64_t *bytes) {
+    if (!o || !o->single || !bytes || (buf && !img_aligned(buf))) return BLU_ERROR_INVALID_ARGUMENT;
+    return save_host(o, 1, &OBJECT_SLOT, buf ? &buf : nullptr, &cap, bytes);
+}
+extern "C" int blu_save_dev(blu_t *o, void *d_buf, int64_t cap, int64_t *bytes) {
+    if (!o || !o->single || !bytes || (d_buf && !img_aligned(d_buf))) return BLU_ERROR_INVALID_ARGUMENT;
+    return save_device(o, 1, &OBJECT_SLOT, d_buf ? &d_buf : nullptr, &cap, bytes);
+}
+extern "C" int blu_restore(blu_t *o, const void *buf, int64_t cap) {
+    if (!o || !o->single || !img_aligned(buf) || cap < (int64_t)sizeof(BluImage)) return BLU_ERROR_INVALID_ARGUMENT;
+    return restore_host(o, 1, &OBJECT_SLOT, &buf, &cap);
+}
+extern "C" int blu_restore_dev(blu_t *o, const void *d_buf, int64_t cap) {
+    if (!o || !o->single || !img_aligned(d_buf) || cap < (int64_t)sizeof(BluImage)) return BLU_ERROR_INVALID_ARGUMENT;
+    return restore_device(o, 1, &OBJECT_SLOT, &d_buf, &cap);
+}
+
+/* c (made by create_common with like = src) becomes src: src's image goes through device scratch (its three save
+ * launches queue on src's stream and count in src's launches), is restored into c without a checksum pass, the sorted
+ * row-wise U is copied as it is (k_build_ur would leave the same rows, but tmpi differently), and the host-side
+ * parameters and getters follow. */
+static int clone_into(blu_b200 *c, blu_b200 *src) {
+    MaskedCall cs(src);
+    int *didx = nullptr; BluImage *dhdr = nullptr; unsigned char *img = nullptr, **dimg = nullptr;
+    int64_t bytes = 0;
+    int st = save_extents(src, cs, 1, &OBJECT_SLOT, &didx, &dhdr, &bytes);
+    if (st == BLU_OK) st = cs.alloc(&img, (size_t)bytes);
+    if (st == BLU_OK) st = cs.alloc(&dimg, 1);
+    if (st != BLU_OK) return st;
+    CK(cudaMemcpyAsync(dimg, &img, sizeof img, cudaMemcpyHostToDevice, src->stream));
+    if ((st = save_write(src, cs, 1, didx, dhdr, dimg)) != BLU_OK) return st;      /* (synchronizes) */
+    {
+        MaskedCall cc(c);
+        const unsigned char *im = img;
+        if ((st = restore_images(c, cc, 1, &OBJECT_SLOT, &im, &bytes, false, true, true)) != BLU_OK) return st;
+    }
+    const BluDev &s = src->d;
+    BluDev &d = c->d;
+    const cudaStream_t cst = c->stream;
+    if (c->hinfo[0].have_ur) {
+        int nur = 0;
+        CK(cudaMemcpyAsync(&nur, s.ur_ptr + s.m, sizeof nur, cudaMemcpyDeviceToHost, cst));
+        CK(cudaStreamSynchronize(cst));
+        CK(cudaMemcpyAsync(d.ur_ptr, s.ur_ptr, (size_t)(s.m + 1) * sizeof(int), cudaMemcpyDeviceToDevice, cst));
+        CK(cudaMemcpyAsync(d.dep_ur, s.dep_ur, (size_t)s.m * sizeof(int), cudaMemcpyDeviceToDevice, cst));
+        CK(cudaMemcpyAsync(d.ur_idx, s.ur_idx, (size_t)nur * sizeof(int), cudaMemcpyDeviceToDevice, cst));
+        CK(cudaMemcpyAsync(d.ur_val, s.ur_val, (size_t)nur * sizeof(double), cudaMemcpyDeviceToDevice, cst));
+        CK(cudaStreamSynchronize(cst));
+    }
+    /* parameters (blu_set_param; the capacities and dense-tail sizes came with create_common) */
+    d.prm = s.prm; d.tree_min = s.tree_min;
+    c->realloc_factor = src->realloc_factor; c->norms = src->norms; c->nthreads = src->nthreads; c->tail_threads = src->tail_threads;
+    c->split_min = src->split_min; c->cap = src->cap; c->solve_units = src->solve_units;
+    /* the host-side getters and state */
+    c->time_factorize = src->time_factorize; c->time_solve = src->time_solve; c->time_update = src->time_update;
+    c->nrealloc = src->nrealloc; c->task_pending = src->task_pending; c->have_b = src->have_b;
+    memcpy(c->last_ms, src->last_ms, sizeof c->last_ms); memcpy(c->last_part_ms, src->last_part_ms, sizeof c->last_part_ms);
+    c->parts_timed = src->parts_timed; c->last_norms_ms = src->last_norms_ms;
+    return BLU_OK;
+}
+
+extern "C" int blu_clone(blu_t **out, blu_t *src) {
+    if (!out || !src || !src->single) return BLU_ERROR_INVALID_ARGUMENT;
+    CK(cudaSetDevice(src->device));
+    blu_b200 *c = nullptr;
+    int st = create_common(&c, 1, src->d.m, src->d.bnz_cap, src->device, 1, src);
+    if (st != BLU_OK) return st;
+    if ((st = clone_into(c, src)) != BLU_OK) { destroy_common(c); return st; }
+    *out = c;
     return BLU_OK;
 }
 

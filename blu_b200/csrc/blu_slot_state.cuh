@@ -38,6 +38,7 @@
     X(34, info, BluInfo, 1)
 #define STATE_ARRAYS 35      /* entries of the table */
 #define STATE_INFO 34        /* the entry that is BluInfo */
+#define STATE_TMPI 30        /* the entry that is tmpi (k_build_ur's scratch) */
 
 /* 4-byte words of entry a of the table for dimension m */
 BLU_HD size_t state_words(int a, size_t M) {

@@ -128,6 +128,37 @@ int blu_solve_for_update(blu_t *o, int64_t nzrhs, const int64_t *irhs, const dou
 /* BLU::update, blu.rs:319-334 -> update.rs:49 */
 int blu_update(blu_t *o, double xtbl);
 
+/* BLU: Clone.  *out becomes a new object on src's device that holds what src holds: the factors and the update history,
+ * a pending solve_for_update of either direction, every getter (the host-side BLU_I_TIME_* and BLU_I_NREALLOC too),
+ * every parameter, the L/U/W capacities exactly, the resident B and a pending blu_factorize_c0ntinue Reallocate.  From
+ * then on the clone behaves bit for bit as src would under the same calls, and src does not change (its launch count
+ * grows by the three launches that write its image).  A never-factorized src gives a never-factorized clone.  The
+ * clone goes through an image of src in device scratch (blu_save_dev's bytes), so it needs that much device memory
+ * for the duration of the call.  src from blu_batch_create, or a NULL argument: BLU_ERROR_INVALID_ARGUMENT.  A clone
+ * on another device: restore an image there. */
+int blu_clone(blu_t **out, blu_t *src);
+
+/* blu_batch_save / blu_batch_restore (below) for an object: the same image format, so an image of an object restores
+ * into any batch slot of the same m and an image of a batch slot into any object of the same m.
+ * blu_save: the object's image into buf (cap bytes, 16-byte aligned), its size into *bytes; buf == NULL: a size query.
+ * Save changes nothing.  A cap smaller than the image: BLU_ERROR_INVALID_ARGUMENT after *bytes is written.
+ * blu_restore: the object becomes the basis of the image in buf (cap bytes readable), with the batch call's checks and
+ * rejections (BLU_ERROR_INVALID_ARGUMENT, nothing changes).  Then:
+ * - its L, U and W stores take the image's capacities exactly (the object's own stores are reallocated; the sorted
+ *   row-wise U with the U store); if the image's row-wise B needs more room than the object's, that room grows;
+ * - a fresh basis (nupdate 0, status OK or BLU_WARNING_SINGULAR_MATRIX) gets the sorted row-wise U a factorization
+ *   builds, so that it solves as after that factorization;
+ * - the resident B becomes the image's columns;
+ * - parameters, BLU_I_TIME_* and BLU_I_NREALLOC stay the object's own (an image carries none of them), and a pending
+ *   blu_factorize_c0ntinue Reallocate is dropped (blu_factorize_c0ntinue with c0ntinue != 0 answers
+ *   BLU_ERROR_INVALID_CALL).
+ * The _dev variants take a buffer in device memory on the object's device; their host traffic is that of the batch
+ * calls with n = 1.  An object from blu_batch_create: BLU_ERROR_INVALID_ARGUMENT. */
+int blu_save(blu_t *o, void *buf, int64_t cap, int64_t *bytes);
+int blu_restore(blu_t *o, const void *buf, int64_t cap);
+int blu_save_dev(blu_t *o, void *d_buf, int64_t cap, int64_t *bytes);
+int blu_restore_dev(blu_t *o, const void *d_buf, int64_t cap);
+
 /* ------------------------------------------------------------------ */
 /* batch API: many independent bases of one dimension on one GPU       */
 /* (what "one BLU instance per core" is on the CPU; SURVEY.md 8e)      */
