@@ -290,15 +290,17 @@ class BLU(_Base):
             self.nzlhs = 0
 
     def solve_dense_multi(self, rhs, trans="N"):
-        """rhs[nrhs, m] -> (status, x[nrhs, m]): solve_dense for every row, all in flight together."""
+        """rhs[nrhs, m] -> (status, x[nrhs, m]): solve_dense for every row, up to BLU_B200_SOLVE_UNITS rows in flight
+        together."""
         r = _f64(rhs).reshape(-1, self.m)
         x = np.zeros_like(r)
         st = self._L.blu_solve_dense_multi(self._h, r.shape[0], _pf(r), _pf(x), _ch(trans))
         return st, x
 
     def solve_sparse_multi(self, rhs_list, trans="N"):
-        """rhs_list = [(irhs, xrhs), ...] -> (status, [(ilhs, values), ...]): solve_sparse for each, all in
-        flight together; entry n of a result is lhs[ilhs[n]] = values[n], in solve_sparse's order."""
+        """rhs_list = [(irhs, xrhs), ...] -> (status, [(ilhs, values), ...]): solve_sparse for each, up to
+        BLU_B200_SOLVE_UNITS in flight together; entry n of a result is lhs[ilhs[n]] = values[n], in solve_sparse's
+        order."""
         n = len(rhs_list)
         begin = np.zeros(n + 1, dtype=np.int64)
         for r, (ii, _) in enumerate(rhs_list):

@@ -72,8 +72,10 @@ struct blu_b200 {
     /* sparse-solve staging (object API) */
     int64_t *d_irhs; double *d_xrhs; int64_t *d_ilhs; double *d_xout; int *d_scal;
     int *h_scal; int64_t *h_ilhs; double *h_xout;   /* pinned */
-    double *dm_rhs, *dm_lhs, *dm_work; int *dm_status; int64_t multi_cap;   /* blu_solve_dense_multi staging */
-    int *sm_ints, *sm_markers, *sm_scal; double *sm_dbls, *sm_xout; int64_t *sm_ilhs, *sm_begin; int64_t smulti_cap;   /* blu_solve_sparse_multi */
+    /* scratch of the batch basis-change calls (solve_for_update / update: whole batch, subset, _dev) and of maxvolume,
+     * nothing else (ensure_batch_sparse): per basis the status word pair, the solution, the right-hand side's offsets,
+     * and in sm_dbls one xtbl */
+    int *sm_scal; double *sm_dbls, *sm_xout; int64_t *sm_ilhs, *sm_begin;
     int64_t *sm_irhs; double *sm_xrhs; int64_t smulti_rhs_cap;
     int solve_units;            /* largest chunk of units of a batch multi-RHS solve (BLU_B200_SOLVE_UNITS) */
     UnitPool up;
@@ -239,8 +241,7 @@ static int create_common(blu_b200 **out, int64_t nmat, int64_t m, int64_t bnz_ca
     o->b_external = 0; o->have_graph = 0;
     o->have_b = 0; o->info_dirty = 0; o->norms = 1; o->last_norms_ms = 0.0;
     o->have_pipe = 0; o->d_chunk_end = nullptr; o->h_chunk_end = nullptr;
-    o->dm_rhs = o->dm_lhs = o->dm_work = nullptr; o->dm_status = nullptr; o->multi_cap = 0;
-    o->sm_ints = o->sm_markers = o->sm_scal = nullptr; o->sm_dbls = o->sm_xout = nullptr; o->sm_ilhs = o->sm_begin = nullptr; o->smulti_cap = 0;
+    o->sm_scal = nullptr; o->sm_dbls = o->sm_xout = nullptr; o->sm_ilhs = o->sm_begin = nullptr;
     o->sm_irhs = nullptr; o->sm_xrhs = nullptr; o->smulti_rhs_cap = 0;
     o->solve_units = 8192;      /* configs[1], 16,384 units (DESIGN.md §5): beyond this the kernels gain ~10 %, the call nothing */
     if (const char *e = getenv("BLU_B200_SOLVE_UNITS")) { long v = atol(e); if (v >= 1 && v <= (1L << 24)) o->solve_units = (int)v; }   /* tuning / test knob */
@@ -1234,7 +1235,7 @@ static int sparse_call(blu_b200 *o, int64_t nzrhs, const int64_t *irhs, const do
     int status = BLU_OK, nz = 0, grown;
     const int rs = rerun_on_realloc(o, grow_object_stores, [&](bool, bool *asks) -> int {
         BLU_LAUNCH(k_solve_sparse, 1, 32, 0, o->stream, o->d, nrhs, (const i64 *)o->d_irhs, dx, trans, for_update, want,
-                   o->d_scal, (i64 *)o->d_ilhs, o->d_xout, SpMulti{0, 0, 0, nullptr, nullptr, nullptr, nullptr});
+                   o->d_scal, (i64 *)o->d_ilhs, o->d_xout, SpMulti{});
         o->launches++;
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(o->h_scal, o->d_scal, 2 * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
@@ -1294,106 +1295,28 @@ extern "C" int blu_update(blu_t *o, double xtbl) {
     return status;
 }
 
-/* SURVEY.md 8(f) N4: many right-hand sides against one factorization -- solve_dense (solve_dense.rs:24)
- * applied to every column of rhs[nrhs][m]; one warp per right-hand side, all of them in flight together
- * (the factors are read-only).  Bit-identical to nrhs separate blu_solve_dense calls. */
+/* SURVEY.md 8(f) N4: many right-hand sides against one factorization -- the batch call on the object's one basis
+ * (its chunks of units go through the unit pool).  Bit-identical to nrhs separate blu_solve_dense calls. */
 extern "C" int blu_solve_dense_multi(blu_t *o, int64_t nrhs, const double *rhs, double *lhs, char trans) {
     if (!o || !o->single || nrhs < 0 || (nrhs > 0 && (!rhs || !lhs))) return BLU_ERROR_INVALID_ARGUMENT;
     { int st0 = ensure_info(o); if (st0 != BLU_OK) return st0; }
     if (o->hinfo[0].nupdate < 0) return BLU_ERROR_INVALID_CALL;   /* solve_dense.rs:25 */
     if (nrhs == 0) return BLU_OK;
-    CK(cudaSetDevice(o->device));
-    const double tic = wall_now();
-    const size_t m = (size_t)o->d.m, n = (size_t)nrhs;
-    if ((int64_t)n > o->multi_cap) {
-        dfree(o, o->dm_rhs); dfree(o, o->dm_lhs); dfree(o, o->dm_work); dfree(o, o->dm_status);
-        o->dm_rhs = o->dm_lhs = o->dm_work = nullptr; o->dm_status = nullptr; o->multi_cap = 0;
-        int st = dalloc(o, &o->dm_rhs, n * m);
-        if (st == BLU_OK) st = dalloc(o, &o->dm_lhs, n * m);
-        if (st == BLU_OK) st = dalloc(o, &o->dm_work, n * m);
-        if (st == BLU_OK) st = dalloc(o, &o->dm_status, n);
-        if (st != BLU_OK) return st;
-        o->multi_cap = (int64_t)n;
-    }
-    CK(cudaMemcpyAsync(o->dm_rhs, rhs, n * m * sizeof(double), cudaMemcpyHostToDevice, o->stream));
-    BLU_LAUNCH(k_garbage_perm, 1, 32, 0, o->stream, o->d);
-    timer_start(o);
-    BLU_LAUNCH(k_solve_dense, (int)std::min<size_t>(n, 1u << 20), 32, 0, o->stream, o->d, (const double *)o->dm_rhs, o->dm_lhs, trans,
-               o->dm_status, o->dm_work, (int)nrhs, (const int *)nullptr);
-    o->launches += 2;
-    CK(cudaGetLastError());
-    timer_stop(o, 1);
-    CK(cudaMemcpyAsync(lhs, o->dm_lhs, n * m * sizeof(double), cudaMemcpyDeviceToHost, o->stream));
-    CK(cudaStreamSynchronize(o->stream));
-    o->info_dirty = 1;
-    o->time_solve += wall_now() - tic;
-    return BLU_OK;
+    return blu_batch_solve_dense_multi(o, nrhs, rhs, lhs, trans, nullptr);
 }
 
-/* Many sparse right-hand sides against one factorization: solve_sparse (solve_sparse.rs:35) for each of
- * them, one warp per right-hand side, all in flight together; every unit has its own marks, stacks and
- * vectors, the factors are only read.  Right-hand side r is irhs/xrhs[rhs_begin[r] .. rhs_begin[r+1]).
- * Results: nzlhs[r] entries (-1 if that right-hand side was rejected, status[r] says why), indices in
- * ilhs[r*m ..] in the same order as blu_solve_sparse returns them, and their VALUES compacted in
- * xlhs[r*m + n] (value of entry ilhs[r*m + n]).  Bit-identical to nrhs separate blu_solve_sparse calls. */
+/* Many sparse right-hand sides against one factorization: blu_batch_solve_sparse with every unit on the object's one
+ * basis, the solutions copied out in full rows.  Bit-identical to nrhs separate blu_solve_sparse calls. */
+static int solve_sparse_units(blu_b200 *o, const int64_t *unit_begin, const int64_t *rhs_begin, const int64_t *irhs, const double *xrhs,
+                              int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans, bool rows);
 extern "C" int blu_solve_sparse_multi(blu_t *o, int64_t nrhs, const int64_t *rhs_begin, const int64_t *irhs, const double *xrhs,
                                       int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans) {
     if (!o || !o->single || nrhs < 0 || (nrhs > 0 && (!rhs_begin || !nzlhs || !ilhs || !xlhs))) return BLU_ERROR_INVALID_ARGUMENT;
     { int st0 = ensure_info(o); if (st0 != BLU_OK) return st0; }
     if (o->hinfo[0].nupdate < 0) return BLU_ERROR_INVALID_CALL;   /* solve_sparse.rs:42 */
     if (nrhs == 0) return BLU_OK;
-    CK(cudaSetDevice(o->device));
-    const double tic = wall_now();
-    const size_t m = (size_t)o->d.m, n = (size_t)nrhs;
-    const int64_t tot = rhs_begin[nrhs];
-    if (tot < 0 || (tot > 0 && (!irhs || !xrhs))) return BLU_ERROR_INVALID_ARGUMENT;
-    int st = BLU_OK;
-    if ((int64_t)n > o->smulti_cap) {
-        dfree(o, o->sm_ints); dfree(o, o->sm_dbls); dfree(o, o->sm_markers); dfree(o, o->sm_scal); dfree(o, o->sm_xout); dfree(o, o->sm_ilhs); dfree(o, o->sm_begin);
-        o->sm_ints = o->sm_markers = o->sm_scal = nullptr; o->sm_dbls = o->sm_xout = nullptr; o->sm_ilhs = o->sm_begin = nullptr; o->smulti_cap = 0;
-        st = dalloc(o, &o->sm_ints, n * 7 * m);
-        if (st == BLU_OK) st = dalloc(o, &o->sm_dbls, n * 2 * m);
-        if (st == BLU_OK) st = dalloc(o, &o->sm_markers, n);
-        if (st == BLU_OK) st = dalloc(o, &o->sm_scal, 2 * n);
-        if (st == BLU_OK) st = dalloc(o, &o->sm_xout, n * m);
-        if (st == BLU_OK) st = dalloc(o, &o->sm_ilhs, n * m);
-        if (st == BLU_OK) st = dalloc(o, &o->sm_begin, n + 1);
-        if (st != BLU_OK) return st;
-        o->smulti_cap = (int64_t)n;
-    }
-    if (tot > o->smulti_rhs_cap) {
-        dfree(o, o->sm_irhs); dfree(o, o->sm_xrhs); o->sm_irhs = nullptr; o->sm_xrhs = nullptr; o->smulti_rhs_cap = 0;
-        st = dalloc(o, &o->sm_irhs, (size_t)tot);
-        if (st == BLU_OK) st = dalloc(o, &o->sm_xrhs, (size_t)tot);
-        if (st != BLU_OK) return st;
-        o->smulti_rhs_cap = tot;
-    }
-    CK(cudaMemcpyAsync(o->sm_begin, rhs_begin, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, o->stream));
-    if (tot > 0) {
-        CK(cudaMemcpyAsync(o->sm_irhs, irhs, (size_t)tot * sizeof(int64_t), cudaMemcpyHostToDevice, o->stream));
-        CK(cudaMemcpyAsync(o->sm_xrhs, xrhs, (size_t)tot * sizeof(double), cudaMemcpyHostToDevice, o->stream));
-    }
-    BLU_LAUNCH(k_garbage_perm, 1, 32, 0, o->stream, o->d);
-    SpMulti W{(int)nrhs, 0, 0, o->sm_ints, o->sm_dbls, o->sm_markers, (const i64 *)o->sm_begin};
-    BLU_LAUNCH(k_solve_sparse, (int)nrhs, 32, 0, o->stream, o->d, 0, (const i64 *)o->sm_irhs, (const double *)o->sm_xrhs, trans, 0, 1,
-               o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
-    o->launches += 2;
-    CK(cudaGetLastError());
-    std::vector<int> hs(2 * n);
-    CK(cudaMemcpyAsync(hs.data(), o->sm_scal, 2 * n * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
-    CK(cudaMemcpyAsync(ilhs, o->sm_ilhs, n * m * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
-    CK(cudaMemcpyAsync(xlhs, o->sm_xout, n * m * sizeof(double), cudaMemcpyDeviceToHost, o->stream));
-    CK(cudaStreamSynchronize(o->stream));
-    int worst = BLU_OK;
-    for (size_t r = 0; r < n; r++) {
-        const int s = hs[2 * r];
-        if (status) status[r] = s;
-        nzlhs[r] = s == BLU_OK ? hs[2 * r + 1] : -1;
-        if (s != BLU_OK && worst == BLU_OK) worst = s;
-    }
-    o->info_dirty = 1;
-    o->time_solve += wall_now() - tic;
-    return worst;
+    const int64_t unit_begin[2] = {0, nrhs};
+    return solve_sparse_units(o, unit_begin, rhs_begin, irhs, xrhs, nzlhs, ilhs, xlhs, status, trans, true);
 }
 
 /* ------------------------------------------------------------------ */
@@ -1495,7 +1418,7 @@ extern "C" int blu_batch_solve_for_update(blu_batch_t *o, const int64_t *rhs_beg
     if (xrhs) CK(cudaMemcpyAsync(o->sm_xrhs, xrhs, (size_t)tot * sizeof(double), cudaMemcpyHostToDevice, o->stream));
     std::vector<int> hs(2 * n);
     st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
-        SpMulti W{(int)n, rerun, 1, nullptr, nullptr, nullptr, (const i64 *)o->sm_begin};
+        SpMulti W{(int)n, rerun, (const i64 *)o->sm_begin};
         BLU_LAUNCH(k_solve_sparse, (int)n, 32, 0, o->stream, o->d, 0, (const i64 *)o->sm_irhs, xrhs ? (const double *)o->sm_xrhs : (const double *)nullptr,
                    trans, 1, want_solution ? 1 : 0, o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
         o->launches++;
@@ -1596,10 +1519,10 @@ static int up_ensure_dense(blu_b200 *o, int64_t P) {
 static int up_ensure_host(blu_b200 *o, int64_t n) {
     UnitPool &U = o->up;
     if (n <= U.hcap) return BLU_OK;
+    const int64_t want = std::max<int64_t>(n, 2 * U.hcap);
     if (U.h_ilhs) cudaFreeHost(U.h_ilhs);
     if (U.h_xout) cudaFreeHost(U.h_xout);
     U.h_ilhs = nullptr; U.h_xout = nullptr; U.hcap = 0;
-    const int64_t want = std::max<int64_t>(n, 2 * U.hcap);
     if (cudaMallocHost((void **)&U.h_ilhs, (size_t)want * sizeof(int64_t)) != cudaSuccess ||
         cudaMallocHost((void **)&U.h_xout, (size_t)want * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return BLU_ERROR_OUT_OF_MEMORY; }
     U.hcap = want;
@@ -1619,11 +1542,12 @@ static int up_compact_all(blu_b200 *o, double *kms) {
 
 /* solve_sparse (solve_sparse.rs:35-73) for the units of every basis, one warp per unit.  Unit u reads the
  * factors of its basis and nothing else of its state; marks, stacks and vectors come from the unit pool, and
- * the flop counters of the basis are added to atomically.  Each chunk's solutions are packed on the device
- * (only the nz entries of each unit cross the bus) and land in the caller's arrays at the unit's own offset. */
-extern "C" int blu_batch_solve_sparse(blu_batch_t *o, const int64_t *unit_begin, const int64_t *rhs_begin,
-                                      const int64_t *irhs, const double *xrhs,
-                                      int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans) {
+ * the flop counters of the basis are added to atomically.  Without rows, each chunk's solutions are packed on the
+ * device (only the nz entries of each unit cross the bus) and land in the caller's arrays at the unit's own offset.
+ * With rows, every unit writes its row of m and the chunk's rows go to the caller's arrays in one copy: the object's
+ * blu_solve_sparse_multi, whose solutions can be dense (configs[3]: 80 % of m), where that is the faster copy. */
+static int solve_sparse_units(blu_b200 *o, const int64_t *unit_begin, const int64_t *rhs_begin, const int64_t *irhs, const double *xrhs,
+                              int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans, bool rows) {
     if (!o || !unit_begin || unit_begin[0] != 0) return BLU_ERROR_INVALID_ARGUMENT;
     const int64_t nmat = o->d.nmat;
     const size_t m = (size_t)o->d.m;
@@ -1658,7 +1582,7 @@ extern "C" int blu_batch_solve_sparse(blu_batch_t *o, const int64_t *unit_begin,
     for (int64_t c0 = 0; c0 < nunits; c0 += P) {
         const int cnt = (int)std::min<int64_t>(P, nunits - c0);
         CK(cudaMemsetAsync(U.fill, 0, sizeof(blu_u64), o->stream));
-        SpMulti W{cnt, 0, 0, U.ints, U.dbls, U.markers, (const i64 *)U.begin + c0, nullptr, U.slot + c0, U.fill, (i64 *)U.off};
+        SpMulti W{cnt, 0, (const i64 *)U.begin + c0, nullptr, U.ints, U.dbls, U.markers, U.slot + c0, U.fill, (i64 *)U.off, rows ? (int)m : 0};
         timer_start(o);
         BLU_LAUNCH(k_solve_sparse<true>, cnt, 32, 0, o->stream, o->d, 0, (const i64 *)U.irhs, (const double *)U.xrhs, trans, 0, 1,
                    U.scal, (i64 *)U.ilhs, U.xout, W);
@@ -1668,8 +1592,13 @@ extern "C" int blu_batch_solve_sparse(blu_batch_t *o, const int64_t *unit_begin,
         kms += o->last_ms[1];
         blu_u64 fill = 0;
         CK(cudaMemcpyAsync(hs.data(), U.scal, 2 * (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, o->stream));
-        CK(cudaMemcpyAsync(hoff.data(), U.off, (size_t)cnt * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
-        CK(cudaMemcpyAsync(&fill, U.fill, sizeof(blu_u64), cudaMemcpyDeviceToHost, o->stream));
+        if (rows) {
+            CK(cudaMemcpyAsync(ilhs + (size_t)c0 * m, U.ilhs, (size_t)cnt * m * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
+            CK(cudaMemcpyAsync(xlhs + (size_t)c0 * m, U.xout, (size_t)cnt * m * sizeof(double), cudaMemcpyDeviceToHost, o->stream));
+        } else {
+            CK(cudaMemcpyAsync(hoff.data(), U.off, (size_t)cnt * sizeof(int64_t), cudaMemcpyDeviceToHost, o->stream));
+            CK(cudaMemcpyAsync(&fill, U.fill, sizeof(blu_u64), cudaMemcpyDeviceToHost, o->stream));
+        }
         CK(cudaStreamSynchronize(o->stream));
         if (fill > 0) {
             if ((st = up_ensure_host(o, (int64_t)fill)) != BLU_OK) return st;
@@ -1682,7 +1611,7 @@ extern "C" int blu_batch_solve_sparse(blu_batch_t *o, const int64_t *unit_begin,
             const int s = hs[2 * b], nz = hs[2 * b + 1];
             if (status) status[u] = s;
             nzlhs[u] = s == BLU_OK ? nz : -1;
-            if (s == BLU_OK && nz > 0) {
+            if (!rows && s == BLU_OK && nz > 0) {
                 memcpy(ilhs + u * m, U.h_ilhs + hoff[b], (size_t)nz * sizeof(int64_t));
                 memcpy(xlhs + u * m, U.h_xout + hoff[b], (size_t)nz * sizeof(double));
             }
@@ -1693,6 +1622,12 @@ extern "C" int blu_batch_solve_sparse(blu_batch_t *o, const int64_t *unit_begin,
     o->info_dirty = 1;
     o->time_solve += wall_now() - tic;
     return worst;
+}
+
+extern "C" int blu_batch_solve_sparse(blu_batch_t *o, const int64_t *unit_begin, const int64_t *rhs_begin,
+                                      const int64_t *irhs, const double *xrhs,
+                                      int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans) {
+    return solve_sparse_units(o, unit_begin, rhs_begin, irhs, xrhs, nzlhs, ilhs, xlhs, status, trans, false);
 }
 
 /* solve_dense (solve_dense.rs:24) for nrhs right-hand sides on every basis, one warp per unit (basis k,
@@ -1941,7 +1876,7 @@ extern "C" int blu_batch_maxvolume(blu_batch_t *o, int64_t ncol, const int64_t *
             BLU_LAUNCH(k_mv_setup, g, 128, 0, s, V, (blu_i64)j);
             o->launches++;
             st = rerun([&](bool again, bool *asks) -> int {
-                SpMulti W{n, again, 1, nullptr, nullptr, nullptr, (const i64 *)V.rhs_begin, (const i64 *)V.rhs_end};
+                SpMulti W{n, again, (const i64 *)V.rhs_begin, (const i64 *)V.rhs_end};
                 BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, d, 0, (const i64 *)o->db_i, (const double *)o->db_x, 'N', 1, 1,
                            o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
                 o->launches++;
@@ -1953,7 +1888,7 @@ extern "C" int blu_batch_maxvolume(blu_batch_t *o, int64_t ncol, const int64_t *
             o->launches++;
             /* the leaving row, maxvolume.rs:143-150 */
             st = rerun([&](bool again, bool *asks) -> int {
-                SpMulti W{n, again, 1, nullptr, nullptr, nullptr, (const i64 *)iota, nullptr};
+                SpMulti W{n, again, (const i64 *)iota};
                 BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, d, 0, (const i64 *)V.leave, (const double *)nullptr, 'T', 1, 0,
                            o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
                 BLU_LAUNCH(k_mv_absorb, g, 128, 0, s, V, (const int *)o->sm_scal, 2);
@@ -2228,7 +2163,7 @@ extern "C" int blu_batch_solve_for_update_subset(blu_batch_t *o, int64_t nsel, c
     if ((st = subset_mask(o, c, pos)) != BLU_OK) return st;
     std::vector<int> hs(2 * n);
     st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
-        SpMulti W{(int)n, rerun, 1, nullptr, nullptr, nullptr, (const i64 *)db, (const i64 *)de};
+        SpMulti W{(int)n, rerun, (const i64 *)db, (const i64 *)de};
         BLU_LAUNCH(k_solve_sparse, (int)n, 32, 0, s, o->d, 0, (const i64 *)o->sm_irhs, xrhs ? (const double *)o->sm_xrhs : (const double *)nullptr,
                    trans, 1, want_solution ? 1 : 0, o->sm_scal, (i64 *)o->sm_ilhs, o->sm_xout, W);
         o->launches++;
@@ -2389,7 +2324,7 @@ extern "C" int blu_batch_solve_for_update_dev(blu_batch_t *o, const int *d_run, 
     i64 *il = want_solution ? (i64 *)d_ilhs : (i64 *)o->sm_ilhs;
     double *xl = want_solution ? d_xlhs : o->sm_xout;
     st = rerun_on_realloc(o, grow_batch_stores, [&](bool rerun, bool *asks) -> int {
-        SpMulti W{n, rerun, 1, nullptr, nullptr, nullptr, (const i64 *)d_rhs_begin, nullptr};
+        SpMulti W{n, rerun, (const i64 *)d_rhs_begin};
         BLU_LAUNCH(k_solve_sparse, n, 32, 0, s, o->d, 0, (const i64 *)d_irhs, d_xrhs, trans, 1, want_solution ? 1 : 0, o->sm_scal, il, xl, W);
         o->launches++;
         CK(cudaGetLastError());
@@ -2464,7 +2399,7 @@ extern "C" int blu_batch_solve_sparse_dev(blu_batch_t *o, int64_t nunits, const 
     for (int64_t c0 = 0; c0 < nunits; c0 += P) {
         const int cnt = (int)std::min<int64_t>(P, nunits - c0);
         CK(cudaMemsetAsync(U.fill, 0, sizeof(blu_u64), s));
-        SpMulti W{cnt, 0, 0, U.ints, U.dbls, U.markers, (const i64 *)d_rhs_begin + c0, nullptr, U.slot + c0, U.fill, (i64 *)U.off};
+        SpMulti W{cnt, 0, (const i64 *)d_rhs_begin + c0, nullptr, U.ints, U.dbls, U.markers, U.slot + c0, U.fill, (i64 *)U.off};
         BLU_LAUNCH(k_solve_sparse<true>, cnt, 32, 0, s, o->d, 0, (const i64 *)d_irhs, d_xrhs, trans, 0, 1, U.scal, (i64 *)U.ilhs, U.xout, W);
         BLU_LAUNCH(k_dev_unpack, cnt, 128, 0, s, (int)m, (const int *)U.scal, (const blu_i64 *)U.off, (const blu_i64 *)U.ilhs,
                    (const double *)U.xout, (blu_i64 *)d_ilhs + (size_t)c0 * m, d_xlhs + (size_t)c0 * m);

@@ -128,11 +128,10 @@ __device__ __forceinline__ void dev_dot_sweep(int m, bool asc, const int *dep, c
  * reference); the lanes share the dot product / axpy of each step and the pointer
  * loads are batched 32 pivots at a time.  Every multiply, add, subtract and divide is
  * rounded once and sums run in the reference's order, so the result is bit-identical. */
-/* Three shapes: (a) multi_work == nullptr: unit u = basis D.slot0 + u of a batch, one right-hand side each;
- * (b) multi_work != nullptr: nrhs right-hand sides against the ONE basis in slot D.slot0 (the factors are
- * only read; every unit has its own work vector multi_work + u*m; the pivot sequence must have been
- * compacted by k_garbage_perm before); (c) as (b), but unit u reads the basis in slot unit_slot[u] (many
- * right-hand sides on every basis of a batch, blu_batch_solve_dense_multi). */
+/* Two shapes: (a) multi_work == unit_slot == nullptr: unit u = basis D.slot0 + u of a batch, one right-hand
+ * side each; (b) both given: nrhs units, unit u reads the basis in slot unit_slot[u] (many right-hand sides
+ * on every basis of a batch, blu_batch_solve_dense_multi).  The factors are only read; every unit has its
+ * own work vector multi_work + u*m; the pivot sequences must have been compacted by k_garbage_perm before. */
 __global__ void __launch_bounds__(32) k_solve_dense(BluDev D, const double *rhs_all, double *lhs_all, char trans, int *status,
                                                      double *multi_work, int nrhs, const int *unit_slot) {
     __shared__ Mat M;
@@ -142,7 +141,7 @@ __global__ void __launch_bounds__(32) k_solve_dense(BluDev D, const double *rhs_
     for (int unit = blockIdx.x; unit < nunits; unit += gridDim.x) {
         const int s = multi ? unit : D.slot0 + unit;       /* index of rhs / lhs / status */
         __syncwarp();
-        if (lane == 0) mat_view(M, D, !multi ? s : unit_slot ? unit_slot[unit] : D.slot0);
+        if (lane == 0) mat_view(M, D, unit_slot ? unit_slot[unit] : s);
         __syncwarp();
         const int m = M.m;
         BluInfo *I = M.info;

@@ -451,21 +451,22 @@ __device__ __forceinline__ void sp_ctx_init(SpCtx &C, const BluDev &D, int slot 
 }
 
 /* lu/solve_sparse.rs:356-358 and the update-cost model (lu.rs:321-326) */
-/* Workspace of blu_solve_sparse_multi: every right-hand side (unit) has its own marks, stacks, patterns
- * and the two scattered vectors, so that all units run at once against the same (read-only) factors. */
+/* The units of a k_solve_sparse launch.  k_solve_sparse<false>: unit u is basis u of a batch, on that basis' own
+ * scratch.  k_solve_sparse<true>: every unit (right-hand side) has its own marks, stacks, patterns and the two
+ * scattered vectors, so that all units run at once against the same (read-only) factors. */
 struct SpMulti {
-    int nunits;               /* 0: single call */
+    int nunits;               /* 0: one right-hand side on the basis in slot 0 (the object calls) */
     int rerun;                /* 1: only the units whose previous status was Reallocate run again */
-    int per_slot;             /* 1: unit u works on basis (slot) u of a batch with that slot's own scratch; ints/dbls/markers unused */
+    const i64 *rhs_begin;     /* nunits + 1 offsets into irhs64 / xrhs */
+    const i64 *rhs_end;       /* null, or nunits end offsets: unit u's right-hand side is [rhs_begin[u], rhs_end[u]) (columns of a resident pool) */
+    /* k_solve_sparse<true> only (blu_batch_solve_sparse and its _dev variant): */
     int *ints;                /* nunits * 7m : marked | pattern_symb | pattern | pstack | ilhs | pend | irhs */
     double *dbls;             /* nunits * 2m : work | xlhs  (all-zero between calls) */
     int *markers;             /* nunits */
-    const i64 *rhs_begin;     /* nunits + 1 offsets into irhs64 / xrhs */
-    const i64 *rhs_end;       /* null, or nunits end offsets: unit u's right-hand side is [rhs_begin[u], rhs_end[u]) (columns of a resident pool) */
-    /* k_solve_sparse<true> only (blu_batch_solve_sparse): */
     const int *unit_slot;     /* unit u reads the factors of slot unit_slot[u] */
     blu_u64 *pack_fill;       /* unit u reserves nz entries of ilhs_out / xout at *pack_fill (the chunk's solutions back to back, */
     i64 *pack_off;            /* for one short copy) and records where they start in pack_off[u] */
+    int row_stride;           /* 0: packed as above; m: unit u writes at ilhs_out / xout + u*m instead (rows of a full copy) */
 };
 __device__ __forceinline__ void sp_ctx_init_unit(SpCtx &C, const BluDev &D, const SpMulti &W, int u, int slot) {
     mat_view(C.M, D, slot);
@@ -494,10 +495,11 @@ __device__ __forceinline__ void sp_solve_done(SpCtx &C) {
 /* solve_sparse (solve_sparse.rs:35-73 + lu/solve_sparse.rs:11-360) and solve_for_update
  * (solve_for_update.rs:72-119 + lu/solve_for_update.rs:12-455).
  * scal[0] = status, scal[1] = nzlhs.  The solution leaves compacted: ilhs_out[n], xout[n].
- * Unit shapes (W.nunits > 0): per_slot -- unit u is basis u of a batch, on that basis' own scratch; otherwise
- * units on scratch of their own that only read the factors: of slot 0 (blu_solve_sparse_multi), or with
- * SLOT_UNITS of slot W.unit_slot[u], the solutions packed (blu_batch_solve_sparse).  SLOT_UNITS is a template
- * argument so that the other shapes compile as they did without it. */
+ * Without SLOT_UNITS: W.nunits == 0, one right-hand side on slot 0; otherwise unit u is basis u of a batch, on that
+ * basis' own scratch.  SLOT_UNITS: plain solves, unit u on scratch of its own that only reads the factors of slot
+ * W.unit_slot[u], the solutions packed (blu_batch_solve_sparse) or, with W.row_stride, in rows of m (the object's
+ * blu_solve_sparse_multi).  SLOT_UNITS is a template argument so that the
+ * basis-change shapes compile without the unit shape. */
 template <bool SLOT_UNITS = false>
 __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i64 *irhs64, const double *xrhs, char trans,
                                                       int for_update, int want_solution, int *scal, i64 *ilhs_out, double *xout,
@@ -505,20 +507,19 @@ __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i
     __shared__ SpCtx C;
     const int lane = threadIdx.x & 31;
     const bool units = SLOT_UNITS || W.nunits > 0;
-    const bool per_slot = !SLOT_UNITS && W.per_slot;
-    const bool multi = units && !per_slot;       /* several units share ONE basis: its state is read-only */
     if (SLOT_UNITS) for_update = 0;              /* plain solves only: the solve_for_update paths drop out of this instance */
     if (units) {
         /* unit = blockIdx.x: its slice of the right-hand sides and of the outputs */
         const int u = blockIdx.x;
-        if (per_slot && D.run && !D.run[u]) return;      /* masked out: neither its state nor its status word is touched */
+        if (!SLOT_UNITS && D.run && !D.run[u]) return;      /* masked out: neither its state nor its status word is touched */
         const i64 b = W.rhs_begin[u], e = W.rhs_end ? W.rhs_end[u] : W.rhs_begin[u + 1];
         irhs64 += b; if (xrhs) xrhs += b;
         nrhs = (e - b < 0 || e - b > 0x7fffffff) ? -1 : (int)(e - b);
         scal += 2 * u;
-        if (!SLOT_UNITS) { ilhs_out += (size_t)u * D.m; xout += (size_t)u * D.m; }
+        const size_t stride = SLOT_UNITS ? (size_t)W.row_stride : (size_t)D.m;
+        ilhs_out += (size_t)u * stride; xout += (size_t)u * stride;
         if (W.rerun && scal[0] != BLU_REALLOCATE) return;
-        if (lane == 0) { if (per_slot) sp_ctx_init(C, D, u); else sp_ctx_init_unit(C, D, W, u, SLOT_UNITS ? W.unit_slot[u] : 0); }
+        if (lane == 0) { if (SLOT_UNITS) sp_ctx_init_unit(C, D, W, u, W.unit_slot[u]); else sp_ctx_init(C, D, u); }
     } else if (lane == 0) sp_ctx_init(C, D);
     __syncwarp();
     Mat &M = C.M;
@@ -542,7 +543,7 @@ __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i
     }
     if (st != BLU_OK) { if (lane == 0) { scal[0] = st; scal[1] = 0; } return; }
     for (int n = lane; n < nrhs; n += 32) C.irhs[n] = (int)irhs64[n];
-    if (lane == 0 && !multi) I->addmem_l = I->addmem_u = I->addmem_w = 0;
+    if (lane == 0 && !SLOT_UNITS) I->addmem_l = I->addmem_u = I->addmem_w = 0;
     __syncwarp();
 
     int nz = 0;
@@ -652,7 +653,7 @@ __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i
     if (for_update && !want_solution) nz = 0;
     if (SLOT_UNITS) {
         i64 base = 0;
-        if (lane == 0) { base = (i64)atomicAdd((unsigned long long *)W.pack_fill, (unsigned long long)nz); W.pack_off[blockIdx.x] = base; }
+        if (lane == 0) { base = (i64)atomicAdd((unsigned long long *)W.pack_fill, (unsigned long long)(W.row_stride ? 0 : nz)); W.pack_off[blockIdx.x] = base; }
         base = __shfl_sync(FULLMASK, base, 0);
         ilhs_out += base; xout += base;
     }
@@ -663,7 +664,7 @@ __global__ void __launch_bounds__(32) k_solve_sparse(BluDev D, int nrhs, const i
         xout[n] = C.xlhs[j];
         C.xlhs[j] = 0.0;
     }
-    if (lane == 0) { if (multi) sp_solve_done_atomic(C); else sp_solve_done(C); scal[0] = C.status; scal[1] = nz; }
+    if (lane == 0) { if (SLOT_UNITS) sp_solve_done_atomic(C); else sp_solve_done(C); scal[0] = C.status; scal[1] = nz; }
 }
 
 /* ------------------------------------------------------------------ */

@@ -104,14 +104,21 @@ int blu_get_factors(blu_t *o, int64_t *rowperm, int64_t *colperm,
 int blu_solve_dense(blu_t *o, const double *rhs, double *lhs, char trans);
 
 /* Many right-hand sides against one factorization (SURVEY.md 8f, N4): rhs and lhs hold nrhs vectors of
- * length m back to back; the result is bit-identical to nrhs calls of blu_solve_dense. */
+ * length m back to back; the result is bit-identical to nrhs calls of blu_solve_dense.  This is
+ * blu_batch_solve_dense_multi on the object's one basis: the right-hand sides run in chunks of at most
+ * BLU_B200_SOLVE_UNITS (read from the environment when the object is created, default 8192), and the device
+ * scratch is bounded by that chunk, 24*m bytes per right-hand side, not by nrhs. */
 int blu_solve_dense_multi(blu_t *o, int64_t nrhs, const double *rhs, double *lhs, char trans);
 
 /* Many sparse right-hand sides against one factorization: right-hand side r is
  * irhs/xrhs[rhs_begin[r] .. rhs_begin[r+1]).  For every r: nzlhs[r] (or -1 and status[r], which may be NULL),
  * the pattern ilhs[r*m .. r*m+nzlhs[r]) in the order blu_solve_sparse returns it, and the VALUES of those
- * entries compacted in xlhs[r*m + n].  Bit-identical to nrhs calls of blu_solve_sparse; returns the first
- * non-OK status. */
+ * entries compacted in xlhs[r*m + n].  The rest of row r, and the rows of a rejected right-hand side, are
+ * unspecified: the rows of m come back whole, which is the faster copy for the dense solutions these calls often
+ * have.  Bit-identical to nrhs calls of blu_solve_sparse; returns the first non-OK status.  An offset of rhs_begin
+ * outside [0, rhs_begin[nrhs]]: BLU_ERROR_INVALID_ARGUMENT, nothing runs.  This is blu_batch_solve_sparse with every
+ * unit on the object's one basis: at most BLU_B200_SOLVE_UNITS right-hand sides per launch, so the device scratch is
+ * bounded by that chunk, not by nrhs. */
 int blu_solve_sparse_multi(blu_t *o, int64_t nrhs, const int64_t *rhs_begin, const int64_t *irhs, const double *xrhs,
                            int64_t *nzlhs, int64_t *ilhs, double *xlhs, int *status, char trans);
 
